@@ -2,6 +2,7 @@
 """bench.py — MPC solves/sec of the batched social-MPC solver on B200 (BASELINE.json metric).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference] [--legs all|none]
+                  [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (the whole bounded TR-LM solve of every problem) over one batch of synthetic
 scenarios. Headline workload = BASELINE.json configs[2], the configuration the north star is quoted on ("full
@@ -75,6 +76,24 @@ CPU_SAMPLE = {"obst_only_x4096": 3072, "obst_only_x65536": 3072, "soc_work_obst_
               "soc_work_obst_x65536_A3": 1536, "multistart_256x1024": 1536, "soc_work_obst_x65536_A20": 1024,
               "crowd_x16384_A50": 256, "crowd_x1M_A50": 256}
 WANT = ("u", "cmds", "cost_initial", "cost_final", "iterations", "termination", "usable", "n_evals")
+DUMP_BYTES = 60_000_000  # --dump-outputs: array data per directory, so that the files stay under 64 MB in all
+
+
+def dump_outputs(path, outputs):
+    """--dump-outputs: write every output of the timed path's last step (one row per problem) as PATH/<name>.npy in
+    float64; integer outputs widen exactly. The inputs are seeded, so two builds run with the same arguments can be
+    compared file by file. When all rows exceed DUMP_BYTES, every file holds the same fixed, seeded sample of rows, and
+    PATH/problem_index.npy lists which."""
+    n = len(next(iter(outputs.values())))
+    row_bytes = sum(8 * (v.size // n) for v in outputs.values())
+    rows = None
+    if n * row_bytes > DUMP_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(n, DUMP_BYTES // (row_bytes + 8), replace=False))
+    os.makedirs(path, exist_ok=True)
+    for name, v in outputs.items():
+        np.save(os.path.join(path, f"{name}.npy"), np.asarray(v if rows is None else v[rows], dtype=np.float64))
+    if rows is not None:
+        np.save(os.path.join(path, "problem_index.npy"), rows.astype(np.float64))
 
 
 def flops_per_solve(S, P, A_eff, m, n_full, n_light, iters):
@@ -207,8 +226,10 @@ def run_reference(args, rank, world):
     times = []
     for _ in range(args.steps):
         t0 = time.perf_counter()
-        o.solve_batch(sub, n_threads=threads, want=want)
+        out = o.solve_batch(sub, n_threads=threads, want=want)
         times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     total = sum(times)
     value = n * args.steps / total
     sample = (f"each step = first {n} problems of {args.workload} on {threads} host threads "
@@ -338,8 +359,9 @@ def time_e2e(ctx, fn, steps, warmup):
     return ts, (t_region0, time.perf_counter())
 
 
-def measure(ctx, name, steps, warmup, sampler=None, with_cpu=False, threads=1):
-    """Device-resident + end-to-end measurement of one workload on this rank. Returns a dict of raw pieces."""
+def measure(ctx, name, steps, warmup, sampler=None, with_cpu=False, threads=1, dump_dir=None):
+    """Device-resident + end-to-end measurement of one workload on this rank. Returns a dict of raw pieces. With
+    dump_dir, rank 0 writes the device-resident outputs of the last timed step there (dump_outputs)."""
     from nav2_social_mpc_controller_b200.optimizer import Optimizer
     torch = ctx.torch
     builder, desc, unique_map = WORKLOADS[name]
@@ -364,6 +386,8 @@ def measure(ctx, name, steps, warmup, sampler=None, with_cpu=False, threads=1):
     step_ms, launches, win = time_device(ctx, opt, dstruct, dev_out, steps, warmup)
     if sampler:
         sampler.mark(*win)
+    if dump_dir and ctx.rank == 0:
+        dump_outputs(dump_dir, {k: t.cpu().numpy() for k, t in dev_out.items()})
     # end to end: host-buffer C-ABI call, pinned host memory, H2D + kernels + D2H every step (the unique scenarios)
     host_np = {k: (t.numpy() if t is not None else None) for k, t in host_pinned.items()}
     hshapes = abi.result_shapes(Bu, S, nb)
@@ -727,7 +751,11 @@ def main():
     ap.add_argument("--legs", default="all", help="all | none | comma list of obst_only,multistart,scaling_sweep,scaling_sweep_omni,library_multi,fleet_tick,latency")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--latency-calls", type=int, default=300)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step of the headline workload as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -753,7 +781,7 @@ def main():
     time.sleep(0.15)
     threads = os.cpu_count() or 1
     res = measure(ctx, args.workload, args.steps, args.warmup, sampler=sampler,
-                  with_cpu=not args.no_cpu_baseline, threads=threads)
+                  with_cpu=not args.no_cpu_baseline, threads=threads, dump_dir=args.dump_outputs)
     time.sleep(0.06)
     sampler.stop()
     sampler.join(timeout=2)
