@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define SMPC_ABI_VERSION 3
+#define SMPC_ABI_VERSION 4
 #define SMPC_MAX_BLOCKS 18 /* control_horizon 18 with parameter_block_length 1: the "36x36 class" */
 
 /* Return codes of every entry point. Per-problem solver outcomes are NOT call
@@ -330,6 +330,72 @@ typedef struct smpc_fleet_io {
 int smpc_optimize_batch(smpc_handle* h, smpc_fleet_io* io);
 /* Forget the previous path / cmds (a fresh TrajectoryMemory). */
 int smpc_reset_memory(smpc_handle* h);
+
+/* ---- closed-loop episodes: N robots through their crowd scenes for T controller ticks, all on the GPU --------------
+ * One tick of SocialMPCController::computeVelocityCommands per episode and tick, then the world moves:
+ *   1. seed: the trajectorizer (smpc_trajectorize_batch_device) on the whole global path from the current pose, with
+ *      max_steps = round(max_time / dt) and dt = time_step rounded to 6 decimals (the yaml double, SURVEY Q15). The
+ *      reference's PathHandler prune and TF step are not modelled: the trajectorizer's own search picks the look-ahead
+ *      point, so a path that comes back within lookahead_dist of itself is out of scope;
+ *   2. people: constant velocity, x_k = x_0 + vx * (k * control_period) (same for y, velocities unchanged), then the
+ *      FOV filter (smpc_fov_filter_batch_device) keeps n_agents columns; skipped when n_people == 0;
+ *   3. optimize: the fleet tick's stages (as in smpc_optimize_batch) with n_poses = seed steps + 1 (0 once an episode is
+ *      done), cmds = the seed's (linear.x, angular.z) and the measured speed; each call starts with fresh warm-start
+ *      memory of its own and leaves that of smpc_optimize_batch / smpc_optimize untouched;
+ *   4. command: row 0 of the fleet tick's cmds (the seed command when optimize() returned false);
+ *   5. world step: unicycle forward Euler over control_period, yaw read back through setRPY / getYaw; the next measured
+ *      speed is the command (ideal actuator). Metrics at time (k+1) * control_period against all people of the scene;
+ *      the episode is done when the robot is within goal_tolerance of the last path pose.
+ * The people do not react to the robot and the costmap does not roll with it; omnidirectional robots are not supported.
+ * Host buffers in and out: one upload at the start, one download at the end, no host round trip per tick (the host
+ * polls a 4-byte count of active episodes every 16 ticks and stops early when it reaches 0; results do not depend on
+ * it). Returns SMPC_ERR_UNSUPPORTED for omni_solve or omnidirectional params, SMPC_ERR_ARGUMENT for invalid inputs;
+ * both before anything is launched. */
+typedef struct smpc_episode_io {
+  int n_episodes;        /* B */
+  int n_ticks;           /* T: controller ticks at most */
+  int n_path;            /* N poses per global path (>= 2) */
+  int n_people;          /* K: row stride of people (all people of a scene) */
+  int n_agents;          /* A: people columns the optimizer keeps after the FOV filter (3 = the reference), 1..63 */
+  double control_period; /* s per tick = 1 / controller_frequency (params yaml: 20 Hz -> 0.05) */
+  double goal_tolerance; /* m, position-only goal check (Nav2 SimpleGoalChecker default 0.25); >= 0.2, the distance
+                            to the path end within which the trajectorizer produces no seed (smaller: ARGUMENT) */
+  const double* global_path;    /* [B][N][2], in the costmap frame */
+  const double* pose;           /* [B][3] start pose x, y, yaw */
+  const double* speed;          /* [B][2] measured (v, w) at tick 0 */
+  const double* people;         /* [B][K][5] at t = 0: x, y, vx, vy, vz (people_msgs); may be NULL when K == 0 */
+  const int32_t* n_people_each; /* [B] <= K; may be NULL when K == 0 */
+  /* maps: same meaning as in smpc_fleet_io */
+  const uint8_t* costmaps;      /* [M][size_y][size_x] */
+  const double* costmap_origin; /* [M][2] */
+  const int32_t* costmap_index; /* [B] or NULL (episode b uses map b % M) */
+  int n_costmaps;
+  int size_x;
+  int size_y;
+  double resolution;
+  const uint32_t* od_indexes; /* [Mo][od_height * od_width] */
+  const double* od_origin;    /* [Mo][2] */
+  const int32_t* od_index;    /* [B] or NULL (episode b uses grid b % Mo) */
+  int n_od_grids;
+  uint32_t od_width;
+  uint32_t od_height;
+  float od_resolution;
+  /* out, per episode (none may be NULL) */
+  uint8_t* reached;             /* [B] 1 = within goal_tolerance of the last path pose */
+  int32_t* ticks;               /* [B] ticks run: arrival tick + 1, or T */
+  double* path_length;          /* [B] m driven */
+  double* min_person_dist;      /* [B] m, +inf for a scene without people */
+  int32_t* intimate_ticks;      /* [B] ticks with a person closer than 0.45 m */
+  int32_t* personal_ticks;      /* [B] ticks with a person closer than 1.2 m */
+  int32_t* collision_ticks;     /* [B] ticks on a costmap cell >= 253 (outside the map: 255) */
+  int32_t* not_optimized_ticks; /* [B] ticks where optimize() returned false */
+  double* cmd_variation;        /* [B] sum over k >= 1 of |v_k - v_k-1| + |w_k - w_k-1| */
+  /* optional logs (NULL = off); rows after an episode is done repeat its final pose, cmd and optimized rows are 0 */
+  double* pose_log;       /* [B][T+1][3] */
+  double* cmd_log;        /* [B][T][2] */
+  uint8_t* optimized_log; /* [B][T] */
+} smpc_episode_io;
+int smpc_run_episodes(smpc_handle* h, smpc_episode_io* io);
 
 /* ---- batched pre-solve stage on the GPU: project_people (src/optimizer.cpp:554-671 + sfm.hpp) -----------------
  * One warp per problem, lanes over agents, sequential over the horizon. Generalised from the reference's 3 people to

@@ -9,7 +9,7 @@ from __future__ import annotations
 import ctypes as C
 import numpy as np
 
-SMPC_ABI_VERSION = 3
+SMPC_ABI_VERSION = 4
 SMPC_MAX_BLOCKS = 18
 
 # enum smpc_termination
@@ -357,4 +357,48 @@ class SmpcFovArgs(C.Structure):
         ("costmap_index", C.c_void_p),
         ("people_out", C.c_void_p),
         ("n_people_out", C.c_void_p),
+    ]
+
+
+class SmpcEpisodeIo(C.Structure):
+    """struct smpc_episode_io — closed-loop episodes (smpc_run_episodes)."""
+    _fields_ = [
+        ("n_episodes", C.c_int),
+        ("n_ticks", C.c_int),
+        ("n_path", C.c_int),
+        ("n_people", C.c_int),
+        ("n_agents", C.c_int),
+        ("control_period", C.c_double),
+        ("goal_tolerance", C.c_double),
+        ("global_path", C.c_void_p),
+        ("pose", C.c_void_p),
+        ("speed", C.c_void_p),
+        ("people", C.c_void_p),
+        ("n_people_each", C.c_void_p),
+        ("costmaps", C.c_void_p),
+        ("costmap_origin", C.c_void_p),
+        ("costmap_index", C.c_void_p),
+        ("n_costmaps", C.c_int),
+        ("size_x", C.c_int),
+        ("size_y", C.c_int),
+        ("resolution", C.c_double),
+        ("od_indexes", C.c_void_p),
+        ("od_origin", C.c_void_p),
+        ("od_index", C.c_void_p),
+        ("n_od_grids", C.c_int),
+        ("od_width", C.c_uint32),
+        ("od_height", C.c_uint32),
+        ("od_resolution", C.c_float),
+        ("reached", C.c_void_p),
+        ("ticks", C.c_void_p),
+        ("path_length", C.c_void_p),
+        ("min_person_dist", C.c_void_p),
+        ("intimate_ticks", C.c_void_p),
+        ("personal_ticks", C.c_void_p),
+        ("collision_ticks", C.c_void_p),
+        ("not_optimized_ticks", C.c_void_p),
+        ("cmd_variation", C.c_void_p),
+        ("pose_log", C.c_void_p),
+        ("cmd_log", C.c_void_p),
+        ("optimized_log", C.c_void_p),
     ]

@@ -126,12 +126,14 @@ struct smpc_handle {
   smpc_memory memory;  // (unused since round 2: the level-2 memory lives on the device, smpc_fleet_state)
   smpc_fleet_state fleet;        // fleet tick (smpc_optimize_batch)
   smpc_fleet_state single;       // the one-robot fleet behind smpc_optimize
+  smpc_fleet_state episodes;     // closed-loop episodes (smpc_run_episodes)
 };
 
 const smpc_params* smpc_handle_params(smpc_handle* h) { return &h->params; }
 smpc_memory* smpc_handle_memory(smpc_handle* h) { return &h->memory; }
 smpc_fleet_state* smpc_handle_fleet(smpc_handle* h) { return &h->fleet; }
 smpc_fleet_state* smpc_handle_single(smpc_handle* h) { return &h->single; }
+smpc_fleet_state* smpc_handle_episodes(smpc_handle* h) { return &h->episodes; }
 int smpc_handle_device(smpc_handle* h) { return h->device; }
 int smpc_host_fail(int code, const std::string& msg) { return fail(code, msg); }
 cudaStream_t smpc_handle_stream(smpc_handle* h) { return h->stream; }
@@ -525,6 +527,7 @@ void smpc_destroy(smpc_handle* h) {
   h->pin_out.release();
   h->fleet.release();
   h->single.release();
+  h->episodes.release();
   if (h->queue) cudaFree(h->queue);
   if (h->arrival) cudaFree(h->arrival);
   if (h->arrival_host) cudaFreeHost(h->arrival_host);

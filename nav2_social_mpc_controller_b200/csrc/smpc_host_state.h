@@ -79,9 +79,68 @@ struct smpc_fleet_state {
   }
 };
 
+// consecutive 256-byte aligned sub-buffers of one allocation (base NULL: only count the bytes)
+struct smpc_carve {
+  char* base;
+  size_t off = 0;
+  explicit smpc_carve(void* b) : base(static_cast<char*>(b)) {}
+  template <class T>
+  T* take(size_t count) {
+    T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
+    off += (count * sizeof(T) + 255) & ~static_cast<size_t>(255);
+    return p;
+  }
+};
+
+// Device buffers of one fleet tick (all device pointers; rows of poses / cmds / robot / path have `stride` entries).
+struct smpc_fleet_dev {
+  int B, stride, A, nb;
+  float time_step, max_time;
+  // maps
+  int n_costmaps, size_x, size_y;
+  double resolution;
+  const uint8_t* maps;
+  const double* map_org;
+  const int32_t* map_index;  // may be NULL
+  int n_od_grids;
+  uint32_t od_width, od_height;
+  float od_resolution;
+  const uint32_t* od;
+  const double* od_org;
+  const int32_t* od_index;  // may be NULL
+  // per robot: poses in n_in, after the max_time cut n_each (0 = inactive) and s_each = n_each - 1 (1 when inactive)
+  const int32_t* n_in;
+  const int32_t* n_each;
+  const int32_t* s_each;
+  const double* people;  // [B][A][5]
+  const int32_t* n_people;
+  const double* speed;
+  double* poses;  // in: seed, out: result
+  double* cmds;
+  // warm-start memory (smpc_fleet_memory)
+  double* prev_poses;
+  double* prev_cmds;
+  int32_t* n_prev_poses;
+  int32_t* n_prev_cmds;
+  // stage buffers and outputs (smpc_fleet_carve_stages)
+  double *init, *robot, *pose0, *u0, *path_xy, *goal_yaw, *agents, *cmds_new, *path_new, *cost0, *cost1;
+  uint8_t *has_people, *usable, *optimized;
+  int32_t *term, *iters, *n_out, *status;
+};
+
+// Carves the stage buffers and outputs of smpc_fleet_dev (init .. path_new, then usable .. status) from c.
+void smpc_fleet_carve_stages(smpc_carve& c, smpc_fleet_dev* d);
+// Points d's memory fields at fs's per-robot warm-start memory for d->B robots of d->stride poses; (re-)creates it
+// zeroed (= no memory yet) when the shape changed or after fs->forget().
+cudaError_t smpc_fleet_memory(smpc_fleet_state* fs, smpc_fleet_dev* d, cudaStream_t st);
+// Enqueues one fleet tick on st: memory seeding, people_to_status, format_to_optimize, project_people, the solve and
+// the finish (outputs, memory update). No host synchronisation.
+int smpc_fleet_tick_enqueue(smpc_handle* h, const smpc_fleet_dev& d, cudaStream_t st);
+
 const smpc_params* smpc_handle_params(smpc_handle* h);
 smpc_fleet_state* smpc_handle_fleet(smpc_handle* h);
 smpc_fleet_state* smpc_handle_single(smpc_handle* h);
+smpc_fleet_state* smpc_handle_episodes(smpc_handle* h);
 int smpc_handle_device(smpc_handle* h);
 smpc_memory* smpc_handle_memory(smpc_handle* h);
 int smpc_host_fail(int code, const std::string& msg);
@@ -89,3 +148,9 @@ cudaStream_t smpc_handle_stream(smpc_handle* h);
 void smpc_handle_count_launch(smpc_handle* h);
 // the fleet tick on an explicit state (smpc_optimize_batch uses the handle's fleet state, smpc_optimize its own)
 int smpc_optimize_batch_on(smpc_handle* h, smpc_fleet_state* fs, smpc_fleet_io* io);
+
+#define SMPC_FLEET_CUDA(call)                                                                              \
+  do {                                                                                                     \
+    cudaError_t e__ = (call);                                                                              \
+    if (e__ != cudaSuccess) return smpc_host_fail(SMPC_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e__)); \
+  } while (0)

@@ -788,29 +788,106 @@ __global__ void fleet_finish_kernel(FleetFinish a) {
   }
 }
 
-struct Carve {
-  char* base;
-  size_t off = 0;
-  explicit Carve(void* b) : base(static_cast<char*>(b)) {}
-  template <class T>
-  T* take(size_t count) {
-    T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
-    off += (count * sizeof(T) + 255) & ~static_cast<size_t>(255);
-    return p;
-  }
-};
-
-#define FLEET_CUDA(call)                                                                                   \
-  do {                                                                                                     \
-    cudaError_t e__ = (call);                                                                              \
-    if (e__ != cudaSuccess) return smpc_host_fail(SMPC_ERR_CUDA, std::string(#call) + ": " + cudaGetErrorString(e__)); \
-  } while (0)
+using Carve = smpc_carve;
+#define FLEET_CUDA SMPC_FLEET_CUDA
 
 }  // namespace
 
-extern "C" {
+void smpc_fleet_carve_stages(smpc_carve& c, smpc_fleet_dev* d) {
+  const size_t B = d->B, BS = B * d->stride, A = d->A;
+  d->init = c.take<double>(B * A * 6);
+  d->has_people = c.take<uint8_t>(B);
+  d->robot = c.take<double>(BS * 6);
+  d->pose0 = c.take<double>(B * 3);
+  d->u0 = c.take<double>(B * d->nb * 2);
+  d->path_xy = c.take<double>(BS * 2);
+  d->goal_yaw = c.take<double>(B);
+  d->agents = c.take<double>(B * A * 6 * d->stride);
+  d->cmds_new = c.take<double>(BS * 2);
+  d->path_new = c.take<double>(BS * 3);
+  d->usable = c.take<uint8_t>(B);
+  d->term = c.take<int32_t>(B);
+  d->iters = c.take<int32_t>(B);
+  d->cost0 = c.take<double>(B);
+  d->cost1 = c.take<double>(B);
+  d->n_out = c.take<int32_t>(B);
+  d->optimized = c.take<uint8_t>(B);
+  d->status = c.take<int32_t>(B);
+}
 
-}  // extern "C"
+cudaError_t smpc_fleet_memory(smpc_fleet_state* fs, smpc_fleet_dev* d, cudaStream_t st) {
+  const int B = d->B, stride = d->stride;
+  if (fs->mem_robots != B || fs->mem_stride != stride) {
+    const size_t bytes = (size_t)B * stride * 5 * sizeof(double) + 2 * (size_t)B * sizeof(int32_t) + 1024;
+    cudaError_t e = fs->memory.reserve(bytes);
+    if (e == cudaSuccess) e = cudaMemsetAsync(fs->memory.ptr, 0, bytes, st);
+    if (e != cudaSuccess) return e;
+    fs->mem_robots = B;
+    fs->mem_stride = stride;
+  }
+  Carve cm(fs->memory.ptr);
+  d->prev_poses = cm.take<double>((size_t)B * stride * 3);
+  d->prev_cmds = cm.take<double>((size_t)B * stride * 2);
+  d->n_prev_poses = cm.take<int32_t>(B);
+  d->n_prev_cmds = cm.take<int32_t>(B);
+  return cudaSuccess;
+}
+
+int smpc_fleet_tick_enqueue(smpc_handle* h, const smpc_fleet_dev& d, cudaStream_t st) {
+  const int B = d.B, stride = d.stride, A = d.A, S = stride - 1;
+  const size_t BS = (size_t)B * stride;
+  FLEET_CUDA(cudaMemsetAsync(d.status, 0, (size_t)B * 4, st));
+
+  const unsigned g_bs = (unsigned)((BS + 255) / 256), g_b = (unsigned)((B + 255) / 256);
+  // ---- TrajectoryMemory seeding, people_to_status, format_to_optimize, project_people
+  fleet_seed_memory_kernel<<<g_bs, 256, 0, st>>>(B, stride, d.n_in, d.poses, d.cmds, d.prev_poses, d.prev_cmds,
+                                                 d.n_prev_poses);
+  fleet_seed_len_kernel<<<g_b, 256, 0, st>>>(B, d.n_in, d.n_prev_poses, d.n_prev_cmds);
+  smpc_people_status_kernel<<<(unsigned)(((size_t)B * A + 255) / 256), 256, 0, st>>>(B, A, d.people, d.n_people, d.init,
+                                                                                    d.has_people);
+  smpc_format_args fa{};
+  fa.n_problems = B; fa.n_poses = stride; fa.n_prev_poses = stride; fa.n_prev_cmds = stride; fa.n_blocks = d.nb;
+  fa.time_step = d.time_step; fa.current_path_w = smpc_handle_params(h)->current_path_w;
+  fa.current_cmds_w = smpc_handle_params(h)->current_cmds_w;
+  fa.poses = d.poses; fa.cmds = d.cmds; fa.speed = d.speed; fa.prev_poses = d.prev_poses; fa.prev_cmds = d.prev_cmds;
+  fa.robot = d.robot; fa.pose0 = d.pose0; fa.u0 = d.u0; fa.path_xy = d.path_xy; fa.goal_yaw = d.goal_yaw;
+  fa.n_poses_each = d.n_each; fa.n_prev_poses_each = d.n_prev_poses; fa.n_prev_cmds_each = d.n_prev_cmds;
+  fa.cmds_stride = stride; fa.has_people = d.has_people;
+  smpc_format_kernel<<<g_bs, 256, 0, st>>>(fa);
+  smpc_project_args pa{};
+  pa.n_problems = B; pa.n_steps = S; pa.n_agents = A; pa.n_grids = d.n_od_grids;
+  pa.od_width = d.od_width; pa.od_height = d.od_height; pa.od_resolution = d.od_resolution;
+  pa.max_time = d.max_time; pa.time_step = d.time_step;
+  pa.od_origin = d.od_org; pa.od_indexes = d.od; pa.od_index = d.od_index;
+  pa.robot = d.robot; pa.people_init = d.init; pa.agents = d.agents; pa.status = d.status; pa.n_steps_each = d.s_each;
+  {
+    const int ctas = (B + kWarps - 1) / kWarps;
+    smpc_project_kernel<<<ctas < 148 * 8 ? ctas : 148 * 8, kWarps * 32, 0, st>>>(pa);
+  }
+  FLEET_CUDA(cudaGetLastError());
+  for (int k = 0; k < 5; ++k) smpc_handle_count_launch(h);
+
+  // ---- the solve (level-1 path, per-robot horizons) with its post-solve expansion
+  smpc_batch bt{};
+  bt.n_problems = B; bt.n_steps = S; bt.n_agents = A; bt.n_costmaps = d.n_costmaps;
+  bt.size_x = d.size_x; bt.size_y = d.size_y; bt.resolution = d.resolution; bt.dt = (double)d.time_step;
+  bt.pose0 = d.pose0; bt.u0 = d.u0; bt.path_xy = d.path_xy; bt.goal_yaw = d.goal_yaw; bt.agents = d.agents;
+  bt.has_people = d.has_people; bt.costmaps = d.maps; bt.costmap_origin = d.map_org;
+  bt.costmap_index = d.map_index; bt.n_steps_each = d.s_each;
+  smpc_result rs{};
+  rs.cmds = d.cmds_new; rs.path = d.path_new; rs.usable = d.usable; rs.termination = d.term; rs.iterations = d.iters;
+  rs.cost_initial = d.cost0; rs.cost_final = d.cost1;
+  const int rc = smpc_solve_batch_device(h, &bt, &rs, st);
+  if (rc != SMPC_OK) return rc;
+
+  // ---- post-solve: outputs, memory update
+  FleetFinish ff{B, stride, d.n_in, d.n_each, d.usable, d.status, d.robot, d.path_new, d.cmds_new, d.poses, d.cmds,
+                 d.prev_poses, d.prev_cmds, d.n_prev_poses, d.n_prev_cmds, d.n_out, d.optimized};
+  fleet_finish_kernel<<<g_bs, 256, 0, st>>>(ff);
+  FLEET_CUDA(cudaGetLastError());
+  smpc_handle_count_launch(h);
+  return SMPC_OK;
+}
 
 int smpc_optimize_batch_on(smpc_handle* h, smpc_fleet_state* fs, smpc_fleet_io* io) {
   if (!h || !io || !fs) return smpc_host_fail(SMPC_ERR_ARGUMENT, "NULL argument");
@@ -856,19 +933,11 @@ int smpc_optimize_batch_on(smpc_handle* h, smpc_fleet_state* fs, smpc_fleet_io* 
   int rc = smpc_problem_dims(prm, S, nullptr, nullptr, &nb, nullptr);
   if (rc != SMPC_OK) return rc;
 
+  smpc_fleet_dev d{};
+  d.B = B; d.stride = stride; d.A = A; d.nb = nb; d.time_step = timestep; d.max_time = maxtime;
+
   // ---- persistent per-robot memory (TrajectoryMemory per robot): re-created only when the fleet shape changes
-  if (fs->mem_robots != B || fs->mem_stride != stride) {
-    const size_t bytes = (size_t)B * stride * 5 * sizeof(double) + 2 * (size_t)B * sizeof(int32_t) + 1024;
-    FLEET_CUDA(fs->memory.reserve(bytes));
-    FLEET_CUDA(cudaMemsetAsync(fs->memory.ptr, 0, bytes, st));
-    fs->mem_robots = B;
-    fs->mem_stride = stride;
-  }
-  Carve cm(fs->memory.ptr);
-  double* prev_poses = cm.take<double>((size_t)B * stride * 3);
-  double* prev_cmds = cm.take<double>((size_t)B * stride * 2);
-  int32_t* n_prev_poses = cm.take<int32_t>(B);
-  int32_t* n_prev_cmds = cm.take<int32_t>(B);
+  FLEET_CUDA(smpc_fleet_memory(fs, &d, st));
 
   // ---- costmaps and obstacle-distance grids stay on the device between ticks: re-sent only when maps_version changes
   const size_t map_bytes = (size_t)io->n_costmaps * io->size_x * io->size_y;
@@ -905,68 +974,56 @@ int smpc_optimize_batch_on(smpc_handle* h, smpc_fleet_state* fs, smpc_fleet_io* 
     fs->maps_version = io->maps_version;
     fs->maps_bytes = maps_total;
   }
+  d.n_costmaps = io->n_costmaps; d.size_x = io->size_x; d.size_y = io->size_y; d.resolution = io->resolution;
+  d.maps = d_maps; d.map_org = d_map_org;
+  d.n_od_grids = io->n_od_grids; d.od_width = io->od_width; d.od_height = io->od_height;
+  d.od_resolution = io->od_resolution; d.od = d_od; d.od_org = d_od_org;
 
-  // ---- per-tick scratch (one allocation that only ever grows)
+  // ---- per-tick scratch (one allocation that only ever grows): the ten input arrays, then the stage buffers and
+  // outputs of the tick
   const size_t BS = (size_t)B * stride;
+  auto carve_inputs = [&](Carve& c) {
+    d.poses = c.take<double>(BS * 3);
+    d.cmds = c.take<double>(BS * 2);
+    d.people = c.take<double>((size_t)B * A * 5);
+    d.n_people = c.take<int32_t>(B);
+    d.speed = c.take<double>((size_t)B * 2);
+    d.n_in = c.take<int32_t>(B);
+    d.n_each = c.take<int32_t>(B);
+    d.s_each = c.take<int32_t>(B);
+    d.map_index = c.take<int32_t>(B);
+    d.od_index = c.take<int32_t>(B);
+    smpc_fleet_carve_stages(c, &d);
+  };
   size_t need = 0;
   {
     Carve probe(nullptr);
-    probe.take<double>(BS * 3); probe.take<double>(BS * 2); probe.take<double>((size_t)B * A * 5); probe.take<int32_t>(B);
-    probe.take<double>((size_t)B * 2); probe.take<int32_t>(B); probe.take<int32_t>(B); probe.take<int32_t>(B);
-    probe.take<int32_t>(B); probe.take<int32_t>(B);
-    probe.take<double>((size_t)B * A * 6); probe.take<uint8_t>(B); probe.take<double>(BS * 6); probe.take<double>((size_t)B * 3);
-    probe.take<double>((size_t)B * nb * 2); probe.take<double>(BS * 2); probe.take<double>(B);
-    probe.take<double>((size_t)B * A * 6 * stride);
-    probe.take<double>(BS * 2); probe.take<double>(BS * 3); probe.take<uint8_t>(B); probe.take<int32_t>(B);
-    probe.take<int32_t>(B); probe.take<double>(B); probe.take<double>(B); probe.take<int32_t>(B); probe.take<uint8_t>(B);
-    probe.take<int32_t>(B);
+    carve_inputs(probe);
     need = probe.off;
   }
   FLEET_CUDA(fs->scratch.reserve(need));
   Carve cs(fs->scratch.ptr);
-  double* d_poses = cs.take<double>(BS * 3);
-  double* d_cmds = cs.take<double>(BS * 2);
-  double* d_people = cs.take<double>((size_t)B * A * 5);
-  int32_t* d_n_people = cs.take<int32_t>(B);
-  double* d_speed = cs.take<double>((size_t)B * 2);
-  int32_t* d_n_in = cs.take<int32_t>(B);
-  int32_t* d_n_each = cs.take<int32_t>(B);
-  int32_t* d_s_each = cs.take<int32_t>(B);
-  int32_t* d_map_index = cs.take<int32_t>(B);
-  int32_t* d_od_index = cs.take<int32_t>(B);
-  double* d_init = cs.take<double>((size_t)B * A * 6);
-  uint8_t* d_has_people = cs.take<uint8_t>(B);
-  double* d_robot = cs.take<double>(BS * 6);
-  double* d_pose0 = cs.take<double>((size_t)B * 3);
-  double* d_u0 = cs.take<double>((size_t)B * nb * 2);
-  double* d_path_xy = cs.take<double>(BS * 2);
-  double* d_goal_yaw = cs.take<double>(B);
-  double* d_agents = cs.take<double>((size_t)B * A * 6 * stride);
-  double* d_cmds_new = cs.take<double>(BS * 2);
-  double* d_path_new = cs.take<double>(BS * 3);
-  uint8_t* d_usable = cs.take<uint8_t>(B);
-  int32_t* d_term = cs.take<int32_t>(B);
-  int32_t* d_iters = cs.take<int32_t>(B);
-  double* d_cost0 = cs.take<double>(B);
-  double* d_cost1 = cs.take<double>(B);
-  int32_t* d_n_out = cs.take<int32_t>(B);
-  uint8_t* d_optimized = cs.take<uint8_t>(B);
-  int32_t* d_status = cs.take<int32_t>(B);
+  carve_inputs(cs);
+  double* d_poses = d.poses;
+  double* d_cmds = d.cmds;
+  double* d_people = const_cast<double*>(d.people);
+  int32_t* d_map_index = const_cast<int32_t*>(d.map_index);
+  int32_t* d_od_index = const_cast<int32_t*>(d.od_index);
   // the scratch starts with the ten input arrays (d_poses .. d_od_index) and ends with the result scalars
-  // (d_usable .. d_status): each group is one contiguous span
+  // (usable .. status): each group is one contiguous span
   const char* scratch0 = static_cast<const char*>(fs->scratch.ptr);
-  const size_t in_span = reinterpret_cast<const char*>(d_init) - scratch0;
-  const size_t tail_off = reinterpret_cast<const char*>(d_usable) - scratch0, tail_span = need - tail_off;
+  const size_t in_span = reinterpret_cast<const char*>(d.init) - scratch0;
+  const size_t tail_off = reinterpret_cast<const char*>(d.usable) - scratch0, tail_span = need - tail_off;
   const size_t io_span = reinterpret_cast<const char*>(d_people) - scratch0;  // d_poses + d_cmds: in/out
   const bool packed = in_span <= kPackedTick && tail_span + io_span <= kPackedTick;
 
   // ---- inputs up
-  struct Src { void* dev; const void* host; size_t bytes; };
+  struct Src { const void* dev; const void* host; size_t bytes; };
   const Src srcs[] = {
       {d_poses, io->poses, BS * 3 * 8},          {d_cmds, io->cmds, BS * 2 * 8},
-      {d_people, io->people, (size_t)B * A * 5 * 8}, {d_n_people, io->n_people, (size_t)B * 4},
-      {d_speed, io->speed, (size_t)B * 16},      {d_n_in, io->n_poses, (size_t)B * 4},
-      {d_n_each, n_each.data(), (size_t)B * 4},  {d_s_each, s_each.data(), (size_t)B * 4},
+      {d_people, io->people, (size_t)B * A * 5 * 8}, {d.n_people, io->n_people, (size_t)B * 4},
+      {d.speed, io->speed, (size_t)B * 16},      {d.n_in, io->n_poses, (size_t)B * 4},
+      {d.n_each, n_each.data(), (size_t)B * 4},  {d.s_each, s_each.data(), (size_t)B * 4},
       {d_map_index, io->costmap_index, (size_t)B * 4}, {d_od_index, io->od_index, (size_t)B * 4},
   };
   if (packed) {
@@ -977,68 +1034,25 @@ int smpc_optimize_batch_on(smpc_handle* h, smpc_fleet_state* fs, smpc_fleet_io* 
     FLEET_CUDA(cudaMemcpyAsync(fs->scratch.ptr, stage, in_span, cudaMemcpyHostToDevice, st));
   } else {
     for (const Src& c : srcs)
-      if (c.host) FLEET_CUDA(cudaMemcpyAsync(c.dev, c.host, c.bytes, cudaMemcpyHostToDevice, st));
+      if (c.host) FLEET_CUDA(cudaMemcpyAsync(const_cast<void*>(c.dev), c.host, c.bytes, cudaMemcpyHostToDevice, st));
   }
-  FLEET_CUDA(cudaMemsetAsync(d_status, 0, (size_t)B * 4, st));
+  if (!io->costmap_index) d.map_index = nullptr;
+  if (!io->od_index) d.od_index = nullptr;
 
-  const unsigned g_bs = (unsigned)((BS + 255) / 256), g_b = (unsigned)((B + 255) / 256);
-  // ---- TrajectoryMemory seeding, people_to_status, format_to_optimize, project_people
-  fleet_seed_memory_kernel<<<g_bs, 256, 0, st>>>(B, stride, d_n_in, d_poses, d_cmds, prev_poses, prev_cmds, n_prev_poses);
-  fleet_seed_len_kernel<<<g_b, 256, 0, st>>>(B, d_n_in, n_prev_poses, n_prev_cmds);
-  smpc_people_status_kernel<<<(unsigned)(((size_t)B * A + 255) / 256), 256, 0, st>>>(B, A, d_people, d_n_people, d_init,
-                                                                                    d_has_people);
-  smpc_format_args fa{};
-  fa.n_problems = B; fa.n_poses = stride; fa.n_prev_poses = stride; fa.n_prev_cmds = stride; fa.n_blocks = nb;
-  fa.time_step = timestep; fa.current_path_w = prm->current_path_w; fa.current_cmds_w = prm->current_cmds_w;
-  fa.poses = d_poses; fa.cmds = d_cmds; fa.speed = d_speed; fa.prev_poses = prev_poses; fa.prev_cmds = prev_cmds;
-  fa.robot = d_robot; fa.pose0 = d_pose0; fa.u0 = d_u0; fa.path_xy = d_path_xy; fa.goal_yaw = d_goal_yaw;
-  fa.n_poses_each = d_n_each; fa.n_prev_poses_each = n_prev_poses; fa.n_prev_cmds_each = n_prev_cmds;
-  fa.cmds_stride = stride; fa.has_people = d_has_people;
-  smpc_format_kernel<<<g_bs, 256, 0, st>>>(fa);
-  smpc_project_args pa{};
-  pa.n_problems = B; pa.n_steps = S; pa.n_agents = A; pa.n_grids = io->n_od_grids;
-  pa.od_width = io->od_width; pa.od_height = io->od_height; pa.od_resolution = io->od_resolution;
-  pa.max_time = maxtime; pa.time_step = timestep;
-  pa.od_origin = d_od_org; pa.od_indexes = d_od; pa.od_index = io->od_index ? d_od_index : nullptr;
-  pa.robot = d_robot; pa.people_init = d_init; pa.agents = d_agents; pa.status = d_status; pa.n_steps_each = d_s_each;
-  {
-    const int ctas = (B + kWarps - 1) / kWarps;
-    smpc_project_kernel<<<ctas < 148 * 8 ? ctas : 148 * 8, kWarps * 32, 0, st>>>(pa);
-  }
-  FLEET_CUDA(cudaGetLastError());
-  for (int k = 0; k < 5; ++k) smpc_handle_count_launch(h);
-
-  // ---- the solve (level-1 path, per-robot horizons) with its post-solve expansion
-  smpc_batch bt{};
-  bt.n_problems = B; bt.n_steps = S; bt.n_agents = A; bt.n_costmaps = io->n_costmaps;
-  bt.size_x = io->size_x; bt.size_y = io->size_y; bt.resolution = io->resolution; bt.dt = (double)timestep;
-  bt.pose0 = d_pose0; bt.u0 = d_u0; bt.path_xy = d_path_xy; bt.goal_yaw = d_goal_yaw; bt.agents = d_agents;
-  bt.has_people = d_has_people; bt.costmaps = d_maps; bt.costmap_origin = d_map_org;
-  bt.costmap_index = io->costmap_index ? d_map_index : nullptr; bt.n_steps_each = d_s_each;
-  smpc_result rs{};
-  rs.cmds = d_cmds_new; rs.path = d_path_new; rs.usable = d_usable; rs.termination = d_term; rs.iterations = d_iters;
-  rs.cost_initial = d_cost0; rs.cost_final = d_cost1;
-  rc = smpc_solve_batch_device(h, &bt, &rs, st);
+  rc = smpc_fleet_tick_enqueue(h, d, st);
   if (rc != SMPC_OK) return rc;
-
-  // ---- post-solve: outputs, memory update
-  FleetFinish ff{B, stride, d_n_in, d_n_each, d_usable, d_status, d_robot, d_path_new, d_cmds_new, d_poses, d_cmds,
-                 prev_poses, prev_cmds, n_prev_poses, n_prev_cmds, d_n_out, d_optimized};
-  fleet_finish_kernel<<<g_bs, 256, 0, st>>>(ff);
-  FLEET_CUDA(cudaGetLastError());
-  smpc_handle_count_launch(h);
 
   // ---- results down
   struct Dst { void* host; const void* dev; size_t bytes; };
   const Dst dsts[] = {
       {io->poses, d_poses, BS * 3 * 8},           {io->cmds, d_cmds, BS * 2 * 8},
-      {io->n_out, d_n_out, (size_t)B * 4},        {io->optimized, d_optimized, (size_t)B},
-      {io->termination, d_term, (size_t)B * 4},   {io->iterations, d_iters, (size_t)B * 4},
-      {io->cost_initial, d_cost0, (size_t)B * 8}, {io->cost_final, d_cost1, (size_t)B * 8},
-      {io->project_status, d_status, (size_t)B * 4},
+      {io->n_out, d.n_out, (size_t)B * 4},        {io->optimized, d.optimized, (size_t)B},
+      {io->termination, d.term, (size_t)B * 4},   {io->iterations, d.iters, (size_t)B * 4},
+      {io->cost_initial, d.cost0, (size_t)B * 8}, {io->cost_final, d.cost1, (size_t)B * 8},
+      {io->project_status, d.status, (size_t)B * 4},
   };
   if (io->people_proj)
-    FLEET_CUDA(cudaMemcpyAsync(io->people_proj, d_agents, (size_t)B * A * 6 * stride * 8, cudaMemcpyDeviceToHost, st));
+    FLEET_CUDA(cudaMemcpyAsync(io->people_proj, d.agents, (size_t)B * A * 6 * stride * 8, cudaMemcpyDeviceToHost, st));
   if (packed) {  // [d_poses, d_cmds] and [d_usable .. d_status] into one staging block, then scattered on the host
     FLEET_CUDA(fs->pin_out.reserve(io_span + tail_span));
     char* stage = static_cast<char*>(fs->pin_out.ptr);

@@ -159,3 +159,68 @@ class FleetOptimizer:
         res["optimized"] = out["optimized"].astype(bool)
         res["path"], res["cmds"], res["people_proj"] = pose_rows, cmd_rows, proj
         return res
+
+    EPISODE_METRICS = (("reached", np.uint8), ("ticks", np.int32), ("path_length", np.float64),
+                       ("min_person_dist", np.float64), ("intimate_ticks", np.int32), ("personal_ticks", np.int32),
+                       ("collision_ticks", np.int32), ("not_optimized_ticks", np.int32), ("cmd_variation", np.float64))
+
+    def run_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
+                     od: dict, ticks: int, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
+                     want_logs=False) -> dict:
+        """Closed-loop episodes on the GPU (smpc_run_episodes): each of the B robots runs its crowd scene for up to
+        `ticks` controller ticks — trajectorizer seed, constant-velocity people, FOV filter, the fleet tick, a unicycle
+        world step — with one upload and one download for the whole run. global_path [B][N][2], pose [B][3],
+        speed [B][2], people [B][K][5] at t = 0 (x, y, vx, vy, vz), n_people [B] <= K, maps as in optimize_batch.
+        Returns host numpy per episode: reached (bool), ticks, path_length, min_person_dist (inf without people),
+        intimate_ticks, personal_ticks, collision_ticks, not_optimized_ticks, cmd_variation; with want_logs also
+        pose_log [B][T+1][3], cmd_log [B][T][2], optimized_log [B][T] (bool)."""
+        io, out, logs, keep = self.episode_io(global_path, pose, speed, people, n_people, costmaps, costmap_origin,
+                                              costmap_resolution, od, ticks, control_period, goal_tolerance,
+                                              costmap_index, od_index, want_logs)
+        _lib.check(_lib.lib().smpc_run_episodes(self.opt._h, C.byref(io)))
+        res = dict(out, **logs)
+        res["reached"] = out["reached"].astype(bool)
+        if want_logs:
+            res["optimized_log"] = logs["optimized_log"].astype(bool)
+        return res
+
+    def episode_io(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
+                   od: dict, ticks: int, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
+                   want_logs=False):
+        """The smpc_episode_io of run_episodes with its output arrays: (io, metrics, logs, inputs kept alive)."""
+        B, T = self.B, int(ticks)
+        gp = np.ascontiguousarray(global_path, dtype=np.float64)
+        assert gp.ndim == 3 and gp.shape[0] == B and gp.shape[2] == 2
+        pose = np.ascontiguousarray(pose, dtype=np.float64).reshape(B, 3)
+        speed = np.ascontiguousarray(speed, dtype=np.float64).reshape(B, 2)
+        people = np.ascontiguousarray(people, dtype=np.float64)
+        K = people.shape[1] if people.ndim == 3 else 0
+        people = people.reshape(B, K, 5)
+        n_people = np.ascontiguousarray(n_people, dtype=np.int32).reshape(B)
+        costmaps = np.ascontiguousarray(costmaps, dtype=np.uint8)
+        morg = np.ascontiguousarray(costmap_origin, dtype=np.float64).reshape(-1, 2)
+        oorg = np.ascontiguousarray(od["origins"], dtype=np.float64).reshape(-1, 2)
+        oidx = np.ascontiguousarray(od["indexes"], dtype=np.uint32).reshape(oorg.shape[0], -1)
+        midx = None if costmap_index is None else np.ascontiguousarray(costmap_index, dtype=np.int32)
+        osel = None if od_index is None else np.ascontiguousarray(od_index, dtype=np.int32)
+        out = {k: np.zeros(B, dt) for k, dt in self.EPISODE_METRICS}
+        logs = dict(pose_log=np.zeros((B, T + 1, 3)), cmd_log=np.zeros((B, T, 2)),
+                    optimized_log=np.zeros((B, T), np.uint8)) if want_logs else {}
+        io = abi.SmpcEpisodeIo()
+        io.n_episodes, io.n_ticks, io.n_path, io.n_people, io.n_agents = B, T, gp.shape[1], K, self.A
+        io.control_period, io.goal_tolerance = float(control_period), float(goal_tolerance)
+        io.global_path, io.pose, io.speed = gp.ctypes.data, pose.ctypes.data, speed.ctypes.data
+        io.people = people.ctypes.data if K > 0 else None
+        io.n_people_each = n_people.ctypes.data
+        io.costmaps, io.costmap_origin = costmaps.ctypes.data, morg.ctypes.data
+        io.costmap_index = None if midx is None else midx.ctypes.data
+        io.n_costmaps, io.size_x, io.size_y = costmaps.shape[0], costmaps.shape[2], costmaps.shape[1]
+        io.resolution = float(costmap_resolution)
+        io.od_indexes, io.od_origin = oidx.ctypes.data, oorg.ctypes.data
+        io.od_index = None if osel is None else osel.ctypes.data
+        io.n_od_grids, io.od_width, io.od_height = oorg.shape[0], int(od["width"]), int(od["height"])
+        io.od_resolution = float(od["resolution"])
+        for k, v in list(out.items()) + list(logs.items()):
+            setattr(io, k, v.ctypes.data)
+        keep = (gp, pose, speed, people, n_people, costmaps, morg, oorg, oidx, midx, osel)
+        return io, out, logs, keep

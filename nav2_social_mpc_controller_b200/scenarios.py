@@ -395,6 +395,91 @@ def crowd(B: int = 65536, A: int = 20, param_set: str = "soc_work_obst", config_
     return _finish(p, seed, S, agents, np.ones(B), cms, np.zeros((M, 2)), idx, res)
 
 
+EPISODE_MARGIN = 0.8  # m between a person's constant-velocity track and the edge of the obstacle grid
+
+
+def episodes(B: int, K: int, param_set: str = "soc_work_obst", seed: int = 6, ticks: int = 200,
+             control_period: float = 0.05, n_maps: int = 16, path_length: float = 10.0, **overrides) -> dict:
+    """Closed-loop scenes for FleetOptimizer.run_episodes: a 12 m x 4 m corridor at 0.05 m (walls at y = 0.3 / 3.7,
+    lethal beyond them, one lethal box near a wall per costmap, `n_maps` costmaps shared round-robin), an
+    obstacle-distance grid to the walls over the whole corridor, a straight global path of `path_length` m along
+    y = 2 from x = 1, start poses near its first pose. K people per scene, half oncoming, half crossing diagonally, at
+    0.3-1.2 m/s. Their constant-velocity tracks stay EPISODE_MARGIN inside the obstacle grid for the whole run plus one
+    projection horizon (ticks * control_period + max_time): a person who leaves the grid makes the reference's
+    computeObstacle throw (project_status), and the crowd projection may move a person up to 0.75 m off its track.
+    Speeds are drawn up to what fits the corridor for the run. Returns the keyword arguments of
+    run_episodes plus `params`."""
+    p = make_params(param_set, **overrides)
+    rng = _rng(500 + seed)
+    res, W, H = 0.05, 240, 80
+    wall_lo, wall_hi = 0.3, 3.7
+    horizon = ticks * control_period + f32(p.max_time)
+    M = max(1, min(n_maps, B))
+    ys = np.arange(H)[:, None] * res
+    xs = np.arange(W)[None, :] * res
+    cms = np.empty((M, H, W), dtype=np.uint8)
+    for m in range(M):
+        side = 1.0 if m % 2 else -1.0
+        bx, by = rng.uniform(3.0, 9.0), 2.0 + side * rng.uniform(0.9, 1.2)
+        cm = wall_costmap(W, H, res, walls_y=(wall_lo, wall_hi), boxes=((bx, by, 0.15, 0.15),))
+        lethal = (ys <= wall_lo) | (ys >= wall_hi) | ((np.abs(xs - bx) <= 0.15) & (np.abs(ys - by) <= 0.15))
+        cm[np.broadcast_to(lethal, cm.shape)] = 254
+        cms[m] = cm
+    rows = np.arange(H)[:, None] * np.ones((1, W), dtype=int)
+    cols = np.ones((H, 1), dtype=int) * np.arange(W)[None, :]
+    r_lo, r_hi = int(round(wall_lo / res)), int(round(wall_hi / res))
+    near = np.where(np.abs(rows - r_lo) <= np.abs(rows - r_hi), r_lo, r_hi)
+    od = dict(width=W, height=H, resolution=res, origins=np.zeros((1, 2)),
+              indexes=(near * W + cols).astype(np.uint32).ravel())
+
+    pose = np.stack([np.full(B, 1.0), 2.0 + rng.uniform(-0.2, 0.2, B), rng.uniform(-0.3, 0.3, B)], axis=1)
+    gpath = _straight_path(B, np.full(B, 1.0), np.full(B, 2.0), length=path_length)
+    speed = np.stack([rng.uniform(0.0, 0.4, B), np.zeros(B)], axis=1)
+
+    lo = np.array([EPISODE_MARGIN, EPISODE_MARGIN])
+    hi = np.array([W * res - EPISODE_MARGIN, H * res - EPISODE_MARGIN])
+    people = np.zeros((B, K, 5))
+    if K > 0:
+        oncoming = (np.arange(K) % 2 == 0)[None, :].repeat(B, axis=0)
+        heading = np.empty((B, K))
+        v = np.empty((B, K))
+        todo = np.ones((B, K), dtype=bool)
+        for _ in range(64):  # draw headings until the slowest allowed speed fits the corridor
+            n = int(todo.sum())
+            if n == 0:
+                break
+            onc = oncoming[todo]
+            off = np.where(onc, rng.uniform(-0.15, 0.15, n), rng.choice([-1.0, 1.0], n) * rng.uniform(0.25, 0.6, n))
+            base = np.where(onc, math.pi, rng.choice([0.0, math.pi], n))
+            h = base + off
+            vmax = np.minimum((hi[0] - lo[0]) / (horizon * np.maximum(np.abs(np.cos(h)), 1e-9)),
+                              (hi[1] - lo[1]) / (horizon * np.maximum(np.abs(np.sin(h)), 1e-9)))
+            ok = vmax >= 0.3
+            vv = 0.3 + (np.minimum(vmax, 1.2) - 0.3) * rng.uniform(0.0, 1.0, n)
+            idx = np.argwhere(todo)[ok]
+            heading[idx[:, 0], idx[:, 1]] = h[ok]
+            v[idx[:, 0], idx[:, 1]] = vv[ok]
+            todo[idx[:, 0], idx[:, 1]] = False
+        assert not todo.any(), "corridor too short for the requested number of ticks"
+        vel = np.stack([v * np.cos(heading), v * np.sin(heading)], axis=-1)
+        ext = vel * horizon  # displacement over the run
+        start_lo = lo - np.minimum(ext, 0.0)
+        start_hi = hi - np.maximum(ext, 0.0)
+        pos = start_lo + (start_hi - start_lo) * rng.uniform(0.0, 1.0, (B, K, 2))
+        for _ in range(16):  # nobody starts within 0.6 m of the robot
+            close = np.hypot(pos[..., 0] - pose[:, None, 0], pos[..., 1] - pose[:, None, 1]) < 0.6
+            if not close.any():
+                break
+            u = rng.uniform(0.0, 1.0, (int(close.sum()), 2))
+            pos[close] = start_lo[close] + (start_hi[close] - start_lo[close]) * u
+        people[:, :, 0:2] = pos
+        people[:, :, 2:4] = vel
+    return dict(params=p, global_path=gpath, pose=pose, speed=speed, people=people,
+                n_people=np.full(B, K, dtype=np.int32), costmaps=cms, costmap_origin=np.zeros((M, 2)),
+                costmap_resolution=res, od=od, costmap_index=(np.arange(B) % M).astype(np.int32), ticks=ticks,
+                control_period=control_period)
+
+
 def with_horizons(batch: Batch, n_steps_each) -> Batch:
     """The same batch with per-problem horizons S_b <= n_steps (include/smpc.h n_steps_each): robots near their goal get
     a shorter seed from the trajectorizer (reference src/path_trajectorizer.cpp:152) and with it fewer steps, a shorter
