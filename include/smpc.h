@@ -346,7 +346,8 @@ int smpc_reset_memory(smpc_handle* h);
  *   5. world step: unicycle forward Euler over control_period, yaw read back through setRPY / getYaw; the next measured
  *      speed is the command (ideal actuator). Metrics at time (k+1) * control_period against all people of the scene;
  *      the episode is done when the robot is within goal_tolerance of the last path pose.
- * The people do not react to the robot and the costmap does not roll with it; omnidirectional robots are not supported.
+ * The people do not react to the robot here (smpc_run_crowd_episodes below moves them under the social force model)
+ * and the costmap does not roll with it; omnidirectional robots are not supported.
  * Host buffers in and out: one upload at the start, one download at the end, no host round trip per tick (the host
  * polls a 4-byte count of active episodes every 16 ticks and stops early when it reaches 0; results do not depend on
  * it). Returns SMPC_ERR_UNSUPPORTED for omni_solve or omnidirectional params, SMPC_ERR_ARGUMENT for invalid inputs;
@@ -396,6 +397,33 @@ typedef struct smpc_episode_io {
   uint8_t* optimized_log; /* [B][T] */
 } smpc_episode_io;
 int smpc_run_episodes(smpc_handle* h, smpc_episode_io* io);
+
+/* ---- closed-loop episodes with a reactive crowd ----------------------------------------------------------------------
+ * smpc_run_episodes with people who walk to their own goals under the lightsfm social force model (sfm.hpp, with the
+ * constants the controller's people projection uses) and react to the robot. io keeps its meaning; io->people holds
+ * the state at t = 0, its velocity columns the initial velocities. Per tick k and episode still running, after the
+ * fleet tick and before the world step, the crowd takes `substeps` synchronous updates of dt_s = control_period /
+ * substeps. Agents: the people 0 .. n_people_each[b]-1 of the scene (all of them, not only those the FOV filter kept)
+ * and the robot, which exerts force but is not moved by the model: at substep s it is at
+ * x_k + (s dt_s) v_k (cos th_k, sin th_k) with velocity v_k (cos th_k, sin th_k), (v_k, w_k) = the command of tick k.
+ * Forces on a person: toward its goal at its desired speed (braking -v / 0.5 once the goal is cleared), the nearest
+ * obstacle cell of the episode's obstacle-distance grid at its current position (radius 0.5; none outside the grid),
+ * and the pair force of every other person and of the robot. updatePosition (sfm.hpp:512-545): velocity capped at the
+ * desired speed; the goal is cleared for good the first time an updated position is within 0.25 m of it; vz becomes
+ * lightsfm's angular velocity. The FOV filter and the world step's metrics read the crowd's state (the controller at
+ * tick k sees the people after k crowd ticks). Once an episode is done its people stand still.
+ * Returns what smpc_run_episodes returns, plus SMPC_ERR_ARGUMENT for crowd == NULL, goals / desired_speed NULL while
+ * n_people > 0, n_people > 63, substeps outside 1..64, a non-finite goal or a desired speed that is not finite and
+ * > 0 for a person < n_people_each[b], or people_disturbance == NULL; all before anything is launched. */
+typedef struct smpc_crowd_io {
+  const double* goals;         /* [B][K][2] each person's goal, in the costmap frame */
+  const double* desired_speed; /* [B][K] lightsfm desiredVelocity, m/s, > 0 */
+  int substeps;                /* social-force updates per control period, 1..64 (dt_s = control_period / substeps) */
+  double* people_disturbance;  /* [B] out: sum over ticks run, substeps and people of |F(robot -> person)| * dt_s */
+  double* people_log;          /* [B][T+1][K][5] or NULL: x, y, vx, vy, vz at every tick (row 0 = the input); rows
+                                  after an episode is done repeat its final row */
+} smpc_crowd_io;
+int smpc_run_crowd_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd);
 
 /* ---- batched pre-solve stage on the GPU: project_people (src/optimizer.cpp:554-671 + sfm.hpp) -----------------
  * One warp per problem, lanes over agents, sequential over the horizon. Generalised from the reference's 3 people to

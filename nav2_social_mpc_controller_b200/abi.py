@@ -402,3 +402,14 @@ class SmpcEpisodeIo(C.Structure):
         ("cmd_log", C.c_void_p),
         ("optimized_log", C.c_void_p),
     ]
+
+
+class SmpcCrowdIo(C.Structure):
+    """struct smpc_crowd_io — the reactive crowd of smpc_run_crowd_episodes."""
+    _fields_ = [
+        ("goals", C.c_void_p),
+        ("desired_speed", C.c_void_p),
+        ("substeps", C.c_int),
+        ("people_disturbance", C.c_void_p),
+        ("people_log", C.c_void_p),
+    ]

@@ -1,9 +1,12 @@
-// smpc_episode.cu — closed-loop episodes (smpc_run_episodes): B robots through their crowd scenes for up to T controller
-// ticks, every tick enqueued on the handle's stream without a host round trip. One tick per episode is
-//   trajectorizer (seed) -> tick prep (people at k * dt_c, seed repack, max_time cut) -> FOV filter -> fleet tick
-//   (smpc_fleet_tick_enqueue) -> world step (robot Euler step, metrics, goal check, logs).
-// The fleet tick runs on the handle's third fleet state, so episodes never touch the warm-start memory of
-// smpc_optimize_batch or smpc_optimize.
+// smpc_episode.cu — closed-loop episodes (smpc_run_episodes, smpc_run_crowd_episodes): B robots through their crowd
+// scenes for up to T controller ticks, every tick enqueued on the handle's stream without a host round trip. One tick
+// per episode is
+//   trajectorizer (seed) -> tick prep (constant-velocity people at k * dt_c, seed repack, max_time cut) -> FOV filter
+//   -> fleet tick (smpc_fleet_tick_enqueue) -> [reactive crowd step, smpc_crowd.cu] -> world step (robot Euler step,
+//   metrics, goal check, logs).
+// Both entries share one loop: with a crowd the prep leaves the people alone, the FOV filter and the world step read
+// the crowd's state, and the crowd step moves it from tick k to k + 1. The fleet tick runs on the handle's third fleet
+// state, so episodes never touch the warm-start memory of smpc_optimize_batch or smpc_optimize.
 #include <cuda_runtime.h>
 
 #include <cmath>
@@ -18,6 +21,7 @@
 namespace {
 
 constexpr int kPollTicks = 16;  // ticks between two reads of the device count of active episodes
+constexpr int kCrowdMaxPeople = 63;  // people + robot in the 64 agent slots of smpc_crowd_step_kernel
 // The trajectorizer produces no step within this distance of the path end (smpc_trajectorize_kernel,
 // src/path_trajectorizer.cpp:152). A robot that close has no seed, so the fleet tick leaves it inactive and its
 // command is zero: a goal tolerance below this distance could leave it standing short of the goal until T.
@@ -84,6 +88,7 @@ struct EpisodeStep {
   const double* cmds;          // [B][stride][2] fleet tick output: row 0 is the command
   const uint8_t* optimized;    // [B]
   const double* people0;       // [B][K][5]
+  const double* people_now;    // [B][K][5] people at (k+1) * dt_c (reactive crowd), or NULL: people0 at constant velocity
   const int32_t* n_people;     // [B] or NULL (K == 0)
   const double* global_path;   // [B][N][2]
   const uint8_t* maps;
@@ -135,8 +140,15 @@ __global__ void __launch_bounds__(128) smpc_episode_step_kernel(EpisodeStep a) {
   const int np = a.K > 0 ? a.n_people[b] : 0;
   double dmin = INFINITY;
   for (int j = lane; j < np; j += 32) {
-    const double* p = a.people0 + ((size_t)b * a.K + j) * 5;
-    const double px = __dadd_rn(p[0], __dmul_rn(p[2], t1)), py = __dadd_rn(p[1], __dmul_rn(p[3], t1));
+    double px, py;
+    if (a.people_now) {
+      px = a.people_now[((size_t)b * a.K + j) * 5];
+      py = a.people_now[((size_t)b * a.K + j) * 5 + 1];
+    } else {
+      const double* p = a.people0 + ((size_t)b * a.K + j) * 5;
+      px = __dadd_rn(p[0], __dmul_rn(p[2], t1));
+      py = __dadd_rn(p[1], __dmul_rn(p[3], t1));
+    }
     dmin = fmin(dmin, hypot_rn(__dsub_rn(px, x1), __dsub_rn(py, y1)));
   }
   for (int off = 16; off > 0; off >>= 1) dmin = fmin(dmin, __shfl_xor_sync(0xffffffffu, dmin, off));
@@ -199,17 +211,18 @@ __global__ void __launch_bounds__(128) smpc_episode_step_kernel(EpisodeStep a) {
   }
 }
 
-int fail_arg(const char* msg) { return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string("run_episodes: ") + msg); }
-
-}  // namespace
-
-extern "C" int smpc_run_episodes(smpc_handle* h, smpc_episode_io* io) {
+// The loop of both entries; crowd == NULL: constant-velocity people (smpc_run_episodes).
+int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd, const char* name) {
+  auto fail_arg = [name](const char* msg) {
+    return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string(name) + ": " + msg);
+  };
   if (!h || !io) return smpc_host_fail(SMPC_ERR_ARGUMENT, "NULL argument");
   const smpc_params* prm = smpc_handle_params(h);
   if (prm->omni_solve)
-    return smpc_host_fail(SMPC_ERR_UNSUPPORTED, "run_episodes: the fleet tick has no omnidirectional solve");
+    return smpc_host_fail(SMPC_ERR_UNSUPPORTED, std::string(name) + ": the fleet tick has no omnidirectional solve");
   if (prm->omnidirectional)
-    return smpc_host_fail(SMPC_ERR_UNSUPPORTED, "run_episodes: the world step moves a unicycle, not an omnidirectional robot");
+    return smpc_host_fail(SMPC_ERR_UNSUPPORTED,
+                          std::string(name) + ": the world step moves a unicycle, not an omnidirectional robot");
   const int B = io->n_episodes, T = io->n_ticks, N = io->n_path, K = io->n_people, A = io->n_agents;
   if (B < 0) return fail_arg("n_episodes < 0");
   if (N < 2) return fail_arg("n_path < 2");
@@ -236,6 +249,20 @@ extern "C" int smpc_run_episodes(smpc_handle* h, smpc_episode_io* io) {
       return fail_arg("costmap_index[b] outside 0..n_costmaps-1");
     if (io->od_index && (io->od_index[b] < 0 || io->od_index[b] >= io->n_od_grids))
       return fail_arg("od_index[b] outside 0..n_od_grids-1");
+  }
+  const bool reactive = crowd != nullptr;
+  if (reactive) {
+    if (K > kCrowdMaxPeople) return fail_arg("n_people above 63 (people + robot share one warp's 64 slots)");
+    if (crowd->substeps < 1 || crowd->substeps > 64) return fail_arg("substeps outside 1..64");
+    if (K > 0 && (!crowd->goals || !crowd->desired_speed)) return fail_arg("missing goals or desired speeds");
+    if (!crowd->people_disturbance) return fail_arg("missing output");
+    for (int b = 0; b < B && K > 0; ++b)
+      for (int i = 0; i < io->n_people_each[b]; ++i) {
+        const double* g = crowd->goals + ((size_t)b * K + i) * 2;
+        const double vd = crowd->desired_speed[(size_t)b * K + i];
+        if (!std::isfinite(g[0]) || !std::isfinite(g[1])) return fail_arg("non-finite goal");
+        if (!std::isfinite(vd) || !(vd > 0.0)) return fail_arg("desired_speed not finite and > 0");
+      }
   }
   // the trajectorizer integrates with the yaml DOUBLE time_step (SURVEY Q15), as FleetOptimizer.trajectorize_batch
   const double traj_dt = std::round((double)prm->time_step * 1e6) / 1e6;
@@ -265,6 +292,9 @@ extern "C" int smpc_run_episodes(smpc_handle* h, smpc_episode_io* io) {
   const size_t od_bytes = (size_t)io->n_od_grids * io->od_width * io->od_height * sizeof(uint32_t);
   const size_t Bz = B, Kz = K, BS = Bz * stride;
   const bool logs_pose = io->pose_log != nullptr, logs_cmd = io->cmd_log != nullptr, logs_opt = io->optimized_log != nullptr;
+  const bool logs_people = reactive && crowd->people_log != nullptr;
+  double *goals = nullptr, *vdes = nullptr, *disturbance = nullptr, *people_log = nullptr;
+  uint8_t* has_goal = nullptr;
   int32_t* n_people_dev = nullptr;
   double *gp, *pose, *people0, *people, *seed_cmds, *pose_log, *cmd_log, *path_length, *min_dist, *cmd_var;
   int32_t *map_index, *od_index, *n_steps, *fov_n, *ticks, *intimate, *personal, *collision, *not_opt;
@@ -309,6 +339,13 @@ extern "C" int smpc_run_episodes(smpc_handle* h, smpc_episode_io* io) {
     pose_log = c.take<double>(logs_pose ? Bz * (T + 1) * 3 : 0);
     cmd_log = c.take<double>(logs_cmd ? Bz * T * 2 : 0);
     opt_log = c.take<uint8_t>(logs_opt ? Bz * T : 0);
+    if (reactive) {  // people holds the crowd's state of the current tick
+      goals = c.take<double>(Bz * Kz * 2);
+      vdes = c.take<double>(Bz * Kz);
+      has_goal = c.take<uint8_t>(Bz * Kz);
+      disturbance = c.take<double>(Bz);
+      people_log = c.take<double>(logs_people ? Bz * (T + 1) * Kz * 5 : 0);
+    }
   };
   size_t need = 0;
   {
@@ -331,6 +368,15 @@ extern "C" int smpc_run_episodes(smpc_handle* h, smpc_episode_io* io) {
   };
   for (const Up& u : ups)
     if (u.host && u.bytes) SMPC_FLEET_CUDA(cudaMemcpyAsync(u.dev, u.host, u.bytes, cudaMemcpyHostToDevice, st));
+  if (reactive) {
+    if (K > 0) {
+      SMPC_FLEET_CUDA(cudaMemcpyAsync(people, io->people, Bz * Kz * 40, cudaMemcpyHostToDevice, st));
+      SMPC_FLEET_CUDA(cudaMemcpyAsync(goals, crowd->goals, Bz * Kz * 16, cudaMemcpyHostToDevice, st));
+      SMPC_FLEET_CUDA(cudaMemcpyAsync(vdes, crowd->desired_speed, Bz * Kz * 8, cudaMemcpyHostToDevice, st));
+      SMPC_FLEET_CUDA(cudaMemsetAsync(has_goal, 1, Bz * Kz, st));
+    }
+    SMPC_FLEET_CUDA(cudaMemsetAsync(disturbance, 0, Bz * 8, st));
+  }
   SMPC_FLEET_CUDA(cudaMemsetAsync(active, 1, Bz, st));
   SMPC_FLEET_CUDA(cudaMemsetAsync(fov_people, 0, Bz * A * 40, st));
   SMPC_FLEET_CUDA(cudaMemsetAsync(fov_n, 0, Bz * 4, st));  // K == 0: nobody to filter, n_people stays 0
@@ -357,7 +403,8 @@ extern "C" int smpc_run_episodes(smpc_handle* h, smpc_episode_io* io) {
   fa.people_in = people; fa.n_people_in = n_people_dev; fa.pose = pose; fa.costmap_origin = map_org;
   fa.costmap_index = d.map_index; fa.people_out = fov_people; fa.n_people_out = fov_n;
 
-  EpisodePrep pp{B, K, stride, max_steps, maxsize, 0.0, n_steps, seed_cmds, active, people0, people, d.poses, d.cmds,
+  // with a crowd the prep moves nobody (K = 0 there): the crowd step does
+  EpisodePrep pp{B, reactive ? 0 : K, stride, max_steps, maxsize, 0.0, n_steps, seed_cmds, active, people0, people, d.poses, d.cmds,
                  const_cast<int32_t*>(d.n_in), const_cast<int32_t*>(d.n_each), const_cast<int32_t*>(d.s_each)};
   EpisodeStep es{};
   es.B = B; es.K = K; es.T = T; es.stride = stride; es.n_path = N;
@@ -369,11 +416,22 @@ extern "C" int smpc_run_episodes(smpc_handle* h, smpc_episode_io* io) {
   es.reached = reached; es.ticks = ticks; es.path_length = path_length; es.min_dist = min_dist;
   es.intimate = intimate; es.personal = personal; es.collision = collision; es.not_optimized = not_opt;
   es.cmd_variation = cmd_var;
+  es.people_now = reactive ? people : nullptr;
   es.pose_log = logs_pose ? pose_log : nullptr;
   es.cmd_log = logs_cmd ? cmd_log : nullptr;
   es.optimized_log = logs_opt ? opt_log : nullptr;
 
-  const int prep_rows = stride > K ? stride : K;
+  smpc_crowd_step_args ca{};
+  if (reactive) {
+    ca.B = B; ca.K = K; ca.T = T; ca.stride = stride; ca.substeps = crowd->substeps; ca.dt_c = io->control_period;
+    ca.active = active; ca.n_people = n_people_dev; ca.pose = pose; ca.cmds = d.cmds; ca.goals = goals; ca.vdes = vdes;
+    ca.has_goal = has_goal; ca.people = people; ca.disturbance = disturbance;
+    ca.people_log = logs_people ? people_log : nullptr;
+    ca.n_od_grids = io->n_od_grids; ca.od_width = io->od_width; ca.od_height = io->od_height;
+    ca.od_resolution = io->od_resolution; ca.od = od; ca.od_org = od_org; ca.od_index = d.od_index;
+  }
+
+  const int prep_rows = stride > pp.K ? stride : pp.K;
   const unsigned g_prep = (unsigned)((Bz * prep_rows + 255) / 256), g_step = (unsigned)((Bz + 3) / 4);
   for (int k = 0; k < T; ++k) {
     rc = smpc_trajectorize_batch_device(h, &ta, st);
@@ -388,6 +446,11 @@ extern "C" int smpc_run_episodes(smpc_handle* h, smpc_episode_io* io) {
     }
     rc = smpc_fleet_tick_enqueue(h, d, st);
     if (rc != SMPC_OK) return rc;
+    if (reactive) {
+      ca.k = k;
+      rc = smpc_crowd_step_enqueue(h, ca, st);
+      if (rc != SMPC_OK) return rc;
+    }
     es.k = k;
     smpc_episode_step_kernel<<<g_step, 128, 0, st>>>(es);
     SMPC_FLEET_CUDA(cudaGetLastError());
@@ -409,6 +472,8 @@ extern "C" int smpc_run_episodes(smpc_handle* h, smpc_episode_io* io) {
       {logs_pose ? io->pose_log : nullptr, pose_log, Bz * (T + 1) * 24},
       {logs_cmd ? io->cmd_log : nullptr, cmd_log, Bz * T * 16},
       {logs_opt ? io->optimized_log : nullptr, opt_log, Bz * T},
+      {reactive ? crowd->people_disturbance : nullptr, disturbance, Bz * 8},
+      {logs_people ? crowd->people_log : nullptr, people_log, Bz * (T + 1) * Kz * 40},
   };
   for (const Down& c : downs)
     if (c.host) SMPC_FLEET_CUDA(cudaMemcpyAsync(c.host, c.dev, c.bytes, cudaMemcpyDeviceToHost, st));
@@ -422,6 +487,21 @@ extern "C" int smpc_run_episodes(smpc_handle* h, smpc_episode_io* io) {
         std::memcpy(io->pose_log + ((size_t)b * (T + 1) + k) * 3, io->pose_log + ((size_t)b * (T + 1) + tb) * 3, 24);
     if (logs_cmd) std::memset(io->cmd_log + ((size_t)b * T + tb) * 2, 0, (size_t)(T - tb) * 16);
     if (logs_opt) std::memset(io->optimized_log + (size_t)b * T + tb, 0, (size_t)(T - tb));
+    if (logs_people)  // the people of a finished episode stand where they were at its last tick
+      for (int k = tb + 1; k <= T; ++k)
+        std::memcpy(crowd->people_log + ((size_t)b * (T + 1) + k) * Kz * 5,
+                    crowd->people_log + ((size_t)b * (T + 1) + tb) * Kz * 5, Kz * 40);
   }
   return SMPC_OK;
+}
+
+}  // namespace
+
+extern "C" int smpc_run_episodes(smpc_handle* h, smpc_episode_io* io) {
+  return run_episodes(h, io, nullptr, "run_episodes");
+}
+
+extern "C" int smpc_run_crowd_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd) {
+  if (!crowd) return smpc_host_fail(SMPC_ERR_ARGUMENT, "run_crowd_episodes: NULL crowd");
+  return run_episodes(h, io, crowd, "run_crowd_episodes");
 }

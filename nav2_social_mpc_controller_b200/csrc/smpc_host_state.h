@@ -137,6 +137,30 @@ cudaError_t smpc_fleet_memory(smpc_fleet_state* fs, smpc_fleet_dev* d, cudaStrea
 // the finish (outputs, memory update). No host synchronisation.
 int smpc_fleet_tick_enqueue(smpc_handle* h, const smpc_fleet_dev& d, cudaStream_t st);
 
+// One controller tick of the reactive crowd of smpc_run_crowd_episodes (smpc_crowd.cu), all device pointers.
+struct smpc_crowd_step_args {
+  int B, K, T, k, stride, substeps;
+  double dt_c;
+  const uint8_t* active;       // [B] episodes still running; the others keep their people
+  const int32_t* n_people;     // [B] people of each scene (<= K)
+  const double* pose;          // [B][3] robot pose of tick k
+  const double* cmds;          // [B][stride][2] fleet tick output: row 0 is the command of tick k
+  const double* goals;         // [B][K][2]
+  const double* vdes;          // [B][K]
+  uint8_t* has_goal;           // [B][K] lightsfm goal flags
+  double* people;              // [B][K][5] in: tick k, out: tick k + 1
+  double* disturbance;         // [B] accumulated
+  double* people_log;          // [B][T+1][K][5] or NULL
+  int n_od_grids;
+  uint32_t od_width, od_height;
+  float od_resolution;
+  const uint32_t* od;
+  const double* od_org;
+  const int32_t* od_index;     // may be NULL (grid b % n_od_grids)
+};
+// Enqueues smpc_crowd_step_kernel on st (one launch).
+int smpc_crowd_step_enqueue(smpc_handle* h, const smpc_crowd_step_args& a, cudaStream_t st);
+
 const smpc_params* smpc_handle_params(smpc_handle* h);
 smpc_fleet_state* smpc_handle_fleet(smpc_handle* h);
 smpc_fleet_state* smpc_handle_single(smpc_handle* h);

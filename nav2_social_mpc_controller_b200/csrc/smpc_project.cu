@@ -13,6 +13,7 @@
 #include "../../include/smpc.h"
 #include "smpc_host_state.h"
 #include "smpc_math.cuh"
+#include "smpc_sfm.cuh"
 
 namespace {
 
@@ -24,55 +25,9 @@ struct AgentSmem {  // structure of arrays, one slot per agent of the current st
   double nx[kMaxAgents], ny[kMaxAgents], nvx[kMaxAgents], nvy[kMaxAgents];  // next-step staging
 };
 
-__device__ __forceinline__ double wrap_pi(double a) {
-  while (a <= -M_PI) a += 2 * M_PI;
-  while (a > M_PI) a -= 2 * M_PI;
-  return a;
-}
-
-// lightsfm social force of one agent pair exactly as the reference writes it (sfm.hpp:239-281): d = other - me,
-// w = my velocity - other's. Out of line: the projection kernel only comes here for degenerate geometry (coincident
-// agents, zero interaction vector, |sin theta| < 1e-9 — e.g. two people standing still, where theta == 0 switches the
-// lateral term off), where the two-atan2 form and its exact-zero tests decide the result.
-__device__ __noinline__ void sfm_pair_reference(double dx, double dy, double wx, double wy, double* fx, double* fy) {
-  const double kSocial = 2.1, kLambda = 2.0, kGamma = 0.35, kN = 2.0, kNPrime = 3.0;
-  const double z = dx * dx + dy * dy;
-  const double dn = sqrt(z);
-  double ex = dx, ey = dy;
-  if (z > 0.0) {
-    ex = dx / dn;
-    ey = dy / dn;
-  }
-  const double Ix = kLambda * wx + ex, Iy = kLambda * wy + ey;
-  const double il = sqrt(Ix * Ix + Iy * Iy);
-  const double ix = Ix / il, iy = Iy / il;
-  const double a1 = wrap_pi(atan2(iy, ix));
-  const double a2 = wrap_pi(atan2(ey, ex));
-  const double th = wrap_pi(a2 - a1);
-  const double B = kGamma * il;
-  const double fv = -exp(-dn / B - (kNPrime * B * th) * (kNPrime * B * th));
-  double sgn = -1.0;
-  if (th == 0) sgn = 0; else if (th > 0) sgn = 1;
-  const double fa = -sgn * exp(-dn / B - (kN * B * th) * (kN * B * th));
-  *fx = kSocial * (fv * ix + fa * (-iy));
-  *fy = kSocial * (fv * iy + fa * ix);
-}
-
-// computeObstacle: the vector the reference stores in obstacles1 (agent - nearest obstacle cell, SURVEY Q10)
-__device__ __forceinline__ bool nearest_obstacle(const smpc_project_args& a, const uint32_t* idx, double ox, double oy,
-                                                 double x, double y, double* out_x, double* out_y) {
-  const unsigned int xc = (unsigned int)floor((x - ox) / a.od_resolution);
-  const unsigned int yc = (unsigned int)floor((y - oy) / a.od_resolution);
-  if (xc >= a.od_width || yc >= a.od_height) return false;
-  const unsigned int ob = idx[xc + yc * a.od_width];
-  if (ob >= a.od_width * a.od_height) return false;
-  const unsigned int cy = ob / a.od_width, cx = ob % a.od_width;
-  const float fx = cx * a.od_resolution + ox;  // float-rounded like the reference (:719-720)
-  const float fy = cy * a.od_resolution + oy;
-  *out_x = x - (double)fx;
-  *out_y = y - (double)fy;
-  return true;
-}
+using smpc::nearest_obstacle;
+using smpc::sfm_pair;
+using smpc::wrap_pi;
 
 __global__ void __launch_bounds__(kWarps * 32) smpc_project_kernel(smpc_project_args a) {
   __shared__ AgentSmem sm[kWarps];
@@ -82,8 +37,7 @@ __global__ void __launch_bounds__(kWarps * 32) smpc_project_kernel(smpc_project_
   const int n_warps = (gridDim.x * blockDim.x) >> 5;
   const int A = a.n_agents, stride = a.n_steps + 1;
   const double dt = (double)a.time_step;
-  const double kDesired = 2.0, kObstacle = 20.0, kSigma = 0.2, kSocial = 2.1, kLambda = 2.0, kGamma = 0.35, kN = 2.0,
-               kNPrime = 3.0, kRelax = 0.5;
+  const double kDesired = 2.0, kObstacle = 20.0, kSigma = 0.2, kRelax = 0.5;  // pair-force constants: smpc_sfm.cuh
 
   for (int b = warp; b < a.n_problems; b += n_warps) {
     // this problem's own horizon (rows keep the stride of the batch's longest one)
@@ -150,7 +104,8 @@ __global__ void __launch_bounds__(kWarps * 32) smpc_project_kernel(smpc_project_
         gx[q] = s.px[slot] + (double)a.max_time * s.vx[slot];
         gy[q] = s.py[slot] + (double)a.max_time * s.vy[slot];
         has_goal[q] = true;
-        if (!nearest_obstacle(a, idx, ox, oy, s.px[slot], s.py[slot], &obx[q], &oby[q])) err = 1;
+        if (!nearest_obstacle(a.od_width, a.od_height, a.od_resolution, idx, ox, oy, s.px[slot], s.py[slot], &obx[q], &oby[q]))
+          err = 1;
       }
       __syncwarp();
     }
@@ -221,32 +176,9 @@ __global__ void __launch_bounds__(kWarps * 32) smpc_project_kernel(smpc_project_
         double sfx = 0.0, sfy = 0.0;
         for (int k = 0; k <= n; ++k) {
           if (k == slot) continue;
-          const double dx = s.px[k] - px, dy = s.py[k] - py;
-          const double wx = vx - s.vx[k], wy = vy - s.vy[k];
-          // Generic geometry: unit vectors by reciprocal square roots, ONE atan2 of (cross, dot) for the angle from the
-          // interaction direction i to e, the kernel's own exp (smpc_math.cuh; each within ~1 ulp of the libm call it
-          // replaces — the projected trajectories move by ~1e-15). Degenerate geometry: the reference's formulation.
-          const double z = dx * dx + dy * dy;
-          const double inv_dn = smpc::rsqrt_pos(z);  // NaN for z == 0: caught by the test on `cross` below
-          const double dn = z * inv_dn, ex = dx * inv_dn, ey = dy * inv_dn;
-          const double Ix = kLambda * wx + ex, Iy = kLambda * wy + ey;
-          const double L2 = Ix * Ix + Iy * Iy;
-          const double inv_il = smpc::rsqrt_pos(L2);
-          const double il = L2 * inv_il, ix = Ix * inv_il, iy = Iy * inv_il;
-          const double cross = ey * ix - ex * iy, dot = ex * ix + ey * iy;
-          if (fabs(cross) > 1e-9) {  // false for NaN
-            const double th = smpc::atan2_unit(cross, dot);
-            const double Bth = kGamma * il * th, base = -dn * inv_il * (1.0 / kGamma);
-            const double fv = -smpc::exp_nonpos(base - (kNPrime * Bth) * (kNPrime * Bth));
-            const double fa = -copysign(smpc::exp_nonpos(base - (kN * Bth) * (kN * Bth)), th);
-            sfx += kSocial * (fv * ix - fa * iy);
-            sfy += kSocial * (fv * iy + fa * ix);
-          } else {
-            double rx, ry;
-            sfm_pair_reference(dx, dy, wx, wy, &rx, &ry);
-            sfx += rx;
-            sfy += ry;
-          }
+          const double2 f = sfm_pair(s.px[k] - px, s.py[k] - py, vx - s.vx[k], vy - s.vy[k], sfx, sfy);
+          sfx = f.x;
+          sfy = f.y;
         }
         fx += sfx;
         fy += sfy;
@@ -285,7 +217,8 @@ __global__ void __launch_bounds__(kWarps * 32) smpc_project_kernel(smpc_project_
         s.py[slot] = s.ny[slot];
         s.vx[slot] = s.nvx[slot];
         s.vy[slot] = s.nvy[slot];
-        if (!nearest_obstacle(a, idx, ox, oy, s.px[slot], s.py[slot], &obx[q], &oby[q])) err = 1;
+        if (!nearest_obstacle(a.od_width, a.od_height, a.od_resolution, idx, ox, oy, s.px[slot], s.py[slot], &obx[q], &oby[q]))
+          err = 1;
         double* o = out + (size_t)slot * 6 * stride + (i + 1);
         o[0] = s.px[slot];
         o[stride] = s.py[slot];

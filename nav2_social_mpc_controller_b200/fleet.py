@@ -184,6 +184,38 @@ class FleetOptimizer:
             res["optimized_log"] = logs["optimized_log"].astype(bool)
         return res
 
+    def run_crowd_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
+                           costmap_resolution, od: dict, ticks: int, goals, desired_speed, substeps=1,
+                           control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
+                           want_logs=False) -> dict:
+        """Closed-loop episodes with a reactive crowd (smpc_run_crowd_episodes): run_episodes, but the people walk to
+        their goals [B][K][2] at their desired speeds [B][K] under the lightsfm social force model, `substeps` updates
+        per control period, and give way to the robot; people [B][K][5] is their state at t = 0. Returns the dict of
+        run_episodes plus people_disturbance [B] (sum of |F(robot -> person)| * dt_s over ticks, substeps and people);
+        with want_logs also people_log [B][T+1][K][5] (x, y, vx, vy, vz at every tick, row 0 = the input)."""
+        io, out, logs, keep = self.episode_io(global_path, pose, speed, people, n_people, costmaps, costmap_origin,
+                                              costmap_resolution, od, ticks, control_period, goal_tolerance,
+                                              costmap_index, od_index, want_logs)
+        B, T, K = self.B, int(ticks), io.n_people
+        goals = np.ascontiguousarray(goals, dtype=np.float64).reshape(B, K, 2)
+        vdes = np.ascontiguousarray(desired_speed, dtype=np.float64).reshape(B, K)
+        crowd = abi.SmpcCrowdIo()
+        crowd.goals = goals.ctypes.data if K > 0 else None
+        crowd.desired_speed = vdes.ctypes.data if K > 0 else None
+        crowd.substeps = int(substeps)
+        disturbance = np.zeros(B)
+        crowd.people_disturbance = disturbance.ctypes.data
+        people_log = np.zeros((B, T + 1, K, 5)) if want_logs else None
+        crowd.people_log = None if people_log is None else people_log.ctypes.data
+        _lib.check(_lib.lib().smpc_run_crowd_episodes(self.opt._h, C.byref(io), C.byref(crowd)))
+        res = dict(out, **logs)
+        res["reached"] = out["reached"].astype(bool)
+        res["people_disturbance"] = disturbance
+        if want_logs:
+            res["optimized_log"] = logs["optimized_log"].astype(bool)
+            res["people_log"] = people_log
+        return res
+
     def episode_io(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
                    od: dict, ticks: int, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
                    want_logs=False):

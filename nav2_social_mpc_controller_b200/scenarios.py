@@ -480,6 +480,101 @@ def episodes(B: int, K: int, param_set: str = "soc_work_obst", seed: int = 6, ti
                 control_period=control_period)
 
 
+CROWD_SPACING = 0.7    # m between two people's starts
+CROWD_CLEARANCE = 0.6  # m between a start and the robot, and between a start and any lethal cell
+GOAL_BAND = 3.0  # m of corridor at each end that holds the goals of the walkers along it (denser crowds push each other
+                 # past their goals and out of the corridor's open ends)
+
+
+def _lethal_clearance_ok(costmaps, res: float, clearance: float) -> np.ndarray:
+    """[M][H][W] bool: no lethal cell centre lies within `clearance` m of any point of this cell."""
+    M, H, W = costmaps.shape
+    lethal = costmaps >= 253
+    r = clearance + res * math.sqrt(0.5)  # the farthest point of a cell is half a diagonal from its centre
+    n = int(math.ceil(r / res))
+    near = np.zeros_like(lethal)
+    pad = np.pad(lethal, ((0, 0), (n, n), (n, n)))
+    for dy in range(-n, n + 1):
+        for dx in range(-n, n + 1):
+            if dx * dx + dy * dy <= (r / res) ** 2:
+                near |= pad[:, n + dy: n + dy + H, n + dx: n + dx + W]
+    return ~near
+
+
+def crowd_episodes(B: int, K: int, seed: int = 6, ticks: int = 200, substeps: int = 1,
+                   param_set: str = "soc_work_obst", **kw) -> dict:
+    """Closed-loop scenes with a reactive crowd for FleetOptimizer.run_crowd_episodes: the corridors, costmaps, paths
+    and start poses of episodes(B, 0, ...) and K people per scene who walk to goals of their own. People i % 3 == 0
+    walk toward the robot (goals near the robot's start end), i % 3 == 1 walk the robot's way (goals at the far end),
+    i % 3 == 2 cross the corridor (goals on the other side, 0.8-1.0 m from its centre line). Desired speeds are
+    0.3-1.2 m/s and every person starts at its desired speed toward its goal. Starts keep CROWD_CLEARANCE from the
+    robot's start and from every lethal cell and CROWD_SPACING from each other. Goals keep EPISODE_MARGIN + 0.5 m/s *
+    max_time from the ends of the obstacle-distance grid: 0.5 m/s caps the controller's projection of a person, so a
+    projected person never leaves the grid. Returns the keyword arguments of run_crowd_episodes plus `params` and
+    `ticks`."""
+    s = episodes(B, 0, param_set=param_set, seed=seed, ticks=ticks, **kw)
+    p = s["params"]
+    rng = _rng(900 + seed)
+    od, res = s["od"], s["costmap_resolution"]
+    W, H = int(od["width"]), int(od["height"])
+    x_lo = EPISODE_MARGIN + 0.5 * f32(p.max_time)
+    x_hi = W * od["resolution"] - x_lo
+    y_mid = 2.0
+    kind = np.arange(K) % 3
+    onc, same, cross = kind == 0, kind == 1, kind == 2
+    clear_ok = _lethal_clearance_ok(s["costmaps"], res, CROWD_CLEARANCE)
+    cidx = s["costmap_index"]
+    pose = s["pose"]
+
+    def draw(n):
+        """starts [n][K][2] and goals [n][K][2] of n scenes"""
+        start = np.empty((n, K, 2))
+        goal = np.empty((n, K, 2))
+        u = lambda lo, hi: rng.uniform(lo, hi, (n, K))  # noqa: E731
+        start[..., 0] = np.where(onc, u(x_lo + GOAL_BAND + 1.0, x_hi), np.where(same, u(x_lo, x_hi - GOAL_BAND - 1.0),
+                                                                                 u(2.5, x_hi - 0.5)))
+        side = rng.choice([-1.0, 1.0], (n, K))
+        start[..., 1] = np.where(cross, y_mid + side * u(0.8, 1.0), u(y_mid - 1.0, y_mid + 1.0))
+        goal[..., 0] = np.where(onc, u(x_lo, x_lo + GOAL_BAND), np.where(same, u(x_hi - GOAL_BAND, x_hi),
+                                                                            np.clip(start[..., 0] + u(-1.0, 1.0), x_lo,
+                                                                                    x_hi)))
+        goal[..., 1] = np.where(cross, y_mid - side * u(0.8, 1.0), u(y_mid - 1.0, y_mid + 1.0))
+        return start, goal
+
+    start, goal = draw(B)
+    todo = np.arange(B) if K > 0 else np.arange(0)
+    for it in range(400):  # redraw the people who break a rule; only scenes with such people are looked at again
+        st = start[todo]
+        mx = np.clip((st[..., 0] / res).astype(np.int64), 0, W - 1)
+        my = np.clip((st[..., 1] / res).astype(np.int64), 0, H - 1)
+        bad = ~clear_ok[cidx[todo][:, None], my, mx]
+        bad |= np.hypot(st[..., 0] - pose[todo, None, 0], st[..., 1] - pose[todo, None, 1]) < CROWD_CLEARANCE
+        d = np.hypot(st[:, :, None, 0] - st[:, None, :, 0], st[:, :, None, 1] - st[:, None, :, 1])
+        d[:, np.tril_indices(K)[0], np.tril_indices(K)[1]] = np.inf  # each pair once: the later person moves
+        bad |= (d < CROWD_SPACING).any(axis=1)
+        keep = bad.any(axis=1)
+        todo, bad = todo[keep], bad[keep]
+        if todo.size == 0:
+            break
+        if it % 50 == 49:  # a scene still stuck after 50 rounds: draw all of its people again
+            bad[:] = True
+        s2, g2 = draw(todo.size)
+        st, gl = start[todo], goal[todo]
+        st[bad], gl[bad] = s2[bad], g2[bad]
+        start[todo], goal[todo] = st, gl
+    else:
+        raise AssertionError("could not place the crowd: fewer people or a longer corridor")
+    vdes = rng.uniform(0.3, 1.2, (B, K))
+    dg = goal - start
+    heading = dg / np.linalg.norm(dg, axis=-1, keepdims=True) if K > 0 else dg
+    people = np.zeros((B, K, 5))
+    people[..., 0:2] = start
+    people[..., 2:4] = heading * vdes[..., None]
+    s.update(people=people, n_people=np.full(B, K, dtype=np.int32), goals=goal, desired_speed=vdes,
+             substeps=substeps)
+    return s
+
+
 def with_horizons(batch: Batch, n_steps_each) -> Batch:
     """The same batch with per-problem horizons S_b <= n_steps (include/smpc.h n_steps_each): robots near their goal get
     a shorter seed from the trajectorizer (reference src/path_trajectorizer.cpp:152) and with it fewer steps, a shorter
