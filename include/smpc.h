@@ -425,6 +425,40 @@ typedef struct smpc_crowd_io {
 } smpc_crowd_io;
 int smpc_run_crowd_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd);
 
+/* ---- closed-loop episodes in shared scenes: several robots in one crowd -----------------------------------------------
+ * smpc_run_crowd_episodes with the B robots grouped into S = B / R scenes of R = robots_per_scene consecutive robots
+ * (robot r of scene s is episode s * R + r). The robots of a scene share one reactive crowd, one costmap and one
+ * obstacle-distance grid, and each robot's controller sees the other robots of its scene as people.
+ * Layout: io and crowd keep their fields. Per robot, B rows: global_path, pose, speed, every metric, pose_log, cmd_log,
+ * optimized_log and people_disturbance. Per scene, S rows (a scene is stored once): io->people [S][K][5],
+ * io->n_people_each [S], crowd->goals [S][K][2], crowd->desired_speed [S][K] and crowd->people_log [S][T+1][K][5].
+ * costmap_index and od_index stay per robot and must be equal within a scene (with a NULL index array, robot b uses
+ * map b % M, which must then be equal within a scene too).
+ * What robot b sees at tick k: the FOV filter's input list holds the other R-1 robots of its scene first, in index
+ * order, then the scene's people after k crowd steps. A robot enters as the person (x, y, v cos th, v sin th, w) with
+ * its pose of tick k and its measured speed (v, w) of tick k (speed at k = 0, the previous command after that); a
+ * robot whose episode is done stands at its final pose with zero velocity and stays visible. Robots go first because
+ * the FOV filter keeps the first n_agents survivors: behind three people in view the robot most likely to be on a
+ * collision course would drop out.
+ * Crowd: one update per scene and substep with the K people and the R robots as agents (K + R <= 64). Each person feels
+ * the pair force of every other person, then of robots 0 .. R-1 in order (R = 1: smpc_run_crowd_episodes exactly).
+ * Robot r at substep s is at x_k + (s dt_s) v_k (cos th_k, sin th_k) for its own command; a finished robot stands
+ * still. people_disturbance[b] sums |F(robot b -> person)| * dt_s while robot b runs. A scene's people move while any
+ * robot of the scene runs; after that they stand still and their people_log rows repeat the final row.
+ * World: robots do not push each other (no contact model); the person metrics stay against people only. Per robot
+ * (scene->robot_min_dist, robot_intimate_ticks): the nearest other robot of the scene at (k+1) * control_period over
+ * the ticks robot b ran (+inf for R = 1) and the ticks with another robot closer than 0.45 m.
+ * Returns what smpc_run_crowd_episodes returns, plus SMPC_ERR_ARGUMENT for scene == NULL, robots_per_scene outside
+ * 1..8, n_episodes not a multiple of it, n_people + robots_per_scene > 64, costmap_index or od_index differing within a
+ * scene, or robot_min_dist / robot_intimate_ticks NULL; all before anything is launched. */
+typedef struct smpc_scene_io {
+  int robots_per_scene;          /* R, 1..8 */
+  double* robot_min_dist;        /* [B] out: m, nearest other robot of the scene; +inf for R = 1 */
+  int32_t* robot_intimate_ticks; /* [B] out: ticks with another robot of the scene closer than 0.45 m */
+} smpc_scene_io;
+int smpc_run_shared_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd,
+                             const smpc_scene_io* scene);
+
 /* ---- batched pre-solve stage on the GPU: project_people (src/optimizer.cpp:554-671 + sfm.hpp) -----------------
  * One warp per problem, lanes over agents, sequential over the horizon. Generalised from the reference's 3 people to
  * A columns. Inputs (device pointers): robot [B][S+1][6] = the robot AgentTrajectory of format_to_optimize

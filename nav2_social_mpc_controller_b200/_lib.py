@@ -68,6 +68,8 @@ def lib():
     L.smpc_run_episodes.restype = C.c_int
     L.smpc_run_crowd_episodes.argtypes = [C.c_void_p, P(abi.SmpcEpisodeIo), P(abi.SmpcCrowdIo)]
     L.smpc_run_crowd_episodes.restype = C.c_int
+    L.smpc_run_shared_episodes.argtypes = [C.c_void_p, P(abi.SmpcEpisodeIo), P(abi.SmpcCrowdIo), P(abi.SmpcSceneIo)]
+    L.smpc_run_shared_episodes.restype = C.c_int
     L.smpc_reset_memory.argtypes = [C.c_void_p]
     L.smpc_reset_memory.restype = C.c_int
     L.smpc_project_people_batch.argtypes = [C.c_void_p, P(abi.SmpcProjectArgs)]
@@ -119,6 +121,7 @@ EXPORTED_SYMBOLS = (
     "smpc_eval_batch", "smpc_multistart_argmin_device", "smpc_last_kernel_ms", "smpc_launch_count",
     "smpc_measure_fp64_peak", "smpc_debug_polymin", "smpc_debug_math", "smpc_debug_plan_chunks", "smpc_set_group",
     "smpc_optimize", "smpc_optimize_batch", "smpc_run_episodes", "smpc_run_crowd_episodes",
+    "smpc_run_shared_episodes",
     "smpc_reset_memory", "smpc_project_people_batch", "smpc_project_people_batch_device",
     "smpc_format_batch_device", "smpc_people_to_status_device", "smpc_memory_update_device",
     "smpc_trajectorize_batch_device", "smpc_fov_filter_batch_device", "smpc_multi_create", "smpc_multi_destroy",

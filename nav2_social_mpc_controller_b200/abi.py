@@ -413,3 +413,12 @@ class SmpcCrowdIo(C.Structure):
         ("people_disturbance", C.c_void_p),
         ("people_log", C.c_void_p),
     ]
+
+
+class SmpcSceneIo(C.Structure):
+    """struct smpc_scene_io — the shared scenes of smpc_run_shared_episodes."""
+    _fields_ = [
+        ("robots_per_scene", C.c_int),
+        ("robot_min_dist", C.c_void_p),
+        ("robot_intimate_ticks", C.c_void_p),
+    ]

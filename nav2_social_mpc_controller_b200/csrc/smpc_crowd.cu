@@ -1,9 +1,10 @@
-// smpc_crowd.cu — the reactive crowd of the closed-loop episodes (smpc_run_crowd_episodes): the people of every scene
-// walk to their own goals under the lightsfm social force model (reference include/nav2_social_mpc_controller/sfm.hpp,
-// the same model and constants the controller's people projection uses, smpc_sfm.cuh), avoid the walls of the
-// scene's obstacle-distance grid and each other, and give way to the robot, which exerts force as an extra agent but
-// is moved by the world step, not by the model. One warp per episode, lanes over people (two slots per lane), the
-// agent states of the current substep in shared memory, laid out like smpc_project_kernel.
+// smpc_crowd.cu — the reactive crowd of the closed-loop episodes (smpc_run_crowd_episodes, smpc_run_shared_episodes):
+// the people of every scene walk to their own goals under the lightsfm social force model (reference
+// include/nav2_social_mpc_controller/sfm.hpp, the same model and constants the controller's people projection uses,
+// smpc_sfm.cuh), avoid the walls of the scene's obstacle-distance grid and each other, and give way to the scene's
+// robots, which exert force as extra agents but are moved by the world step, not by the model. One warp per scene,
+// lanes over people (two slots per lane), the agent states of the current substep in shared memory, laid out like
+// smpc_project_kernel: the people in slots 0 .. n-1, the R robots in slots n .. n+R-1.
 #include <cuda_runtime.h>
 
 #include <cmath>
@@ -15,43 +16,59 @@
 
 namespace {
 
-constexpr int kMaxAgents = 64;  // people + robot
+constexpr int kMaxAgents = 64;  // people + robots
+constexpr int kMaxRobots = 8;   // robots per scene
 constexpr int kWarps = 4;
 
 struct CrowdSmem {  // structure of arrays, one slot per agent of the current substep
   double px[kMaxAgents], py[kMaxAgents], vx[kMaxAgents], vy[kMaxAgents];
   double nx[kMaxAgents], ny[kMaxAgents], nvx[kMaxAgents], nvy[kMaxAgents];  // next-substep staging
+  double dist[kMaxRobots][32];  // per robot and lane: sum of |F(robot -> person)| dt_s over this lane's people
 };
 
-// One controller tick k of the crowd: `substeps` synchronous lightsfm updates of dt_s = dt_c / substeps, every force
-// from the state at the start of its substep. The robot is at x_k + (s dt_s) v_k (cos th_k, sin th_k) at substep s.
+// One controller tick k of the crowd of scene b: `substeps` synchronous lightsfm updates of dt_s = dt_c / substeps,
+// every force from the state at the start of its substep. Robot r is at x_k + (s dt_s) v_k (cos th_k, sin th_k) at
+// substep s for its own pose and command of tick k; a robot whose episode is done stands still (v = 0).
 // Forces on person i (sfm.hpp:188-281): desired force to its goal at its own desired speed (braking -v / 0.5 once the
 // goal is cleared), the obstacle force of the nearest obstacle cell of the grid at the person's current position
 // (radius 0.5; none outside the grid), and the pair force of every other person and of the robot. Unlike the
 // reference's projection (SURVEY Q10) the obstacle enters as a position, so people are pushed away from the walls.
+// The pair forces come from the people first, then from robots 0 .. R-1 in order (R = 1: the arithmetic of one robot).
 // updatePosition (sfm.hpp:512-545): velocity capped at the desired speed, the goal cleared for good the first time the
-// updated position is within 0.25 m of it; vz carries lightsfm's angular velocity. The robot's pair term,
-// |F(robot -> i)| dt_s, accumulates into disturbance[b].
+// updated position is within 0.25 m of it; vz carries lightsfm's angular velocity. Robot r's pair term,
+// |F(robot -> i)| dt_s, accumulates into disturbance[b * R + r] while that robot runs. The people move while any robot
+// of the scene runs.
 __global__ void __launch_bounds__(kWarps * 32) smpc_crowd_step_kernel(smpc_crowd_step_args a) {
   __shared__ CrowdSmem sm[kWarps];
   CrowdSmem& s = sm[threadIdx.x >> 5];
   const int lane = threadIdx.x & 31;
-  const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  if (b >= a.B || !a.active[b]) return;  // warp-uniform
+  const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;  // scene
+  if (b >= a.B) return;  // warp-uniform
+  const int R = a.R, r0 = b * R;
+  bool running = false;
+  for (int r = 0; r < R; ++r) running |= a.active[r0 + r] != 0;
+  if (!running) return;  // warp-uniform
   const double kDesired = 2.0, kObstacle = 20.0, kSigma = 0.2, kRelax = 0.5, kRadius = 0.5, kGoalRadius = 0.25;
   const int K = a.K, n = K > 0 ? a.n_people[b] : 0;
   const double dts = a.dt_c / (double)a.substeps;
   double* P = a.people + (size_t)b * K * 5;
-  const int gi = a.od_index ? a.od_index[b] : (b % a.n_od_grids);
+  const int gi = a.od_index ? a.od_index[r0] : (r0 % a.n_od_grids);
   const uint32_t* idx = a.od + (size_t)gi * a.od_width * a.od_height;
   const double ox = a.od_org[2 * gi], oy = a.od_org[2 * gi + 1];
 
-  // robot: pose and command of tick k (the world step applies the same command)
-  const double v = a.cmds[(size_t)b * a.stride * 2];
-  const double rx = a.pose[3 * b], ry = a.pose[3 * b + 1];
-  double rs, rc;
-  sincos(a.pose[3 * b + 2], &rs, &rc);
-  const double rvx = __dmul_rn(v, rc), rvy = __dmul_rn(v, rs);
+  // lane r < R: robot r's pose and command of tick k (the world step applies the same command)
+  double rx = 0.0, ry = 0.0, rvx = 0.0, rvy = 0.0;
+  if (lane < R) {
+    const int rb = r0 + lane;
+    const double v = a.active[rb] ? a.cmds[(size_t)rb * a.stride * 2] : 0.0;
+    rx = a.pose[3 * rb];
+    ry = a.pose[3 * rb + 1];
+    double rs, rc;
+    sincos(a.pose[3 * rb + 2], &rs, &rc);
+    rvx = __dmul_rn(v, rc);
+    rvy = __dmul_rn(v, rs);
+  }
+  for (int r = 0; r < R; ++r) s.dist[r][lane] = 0.0;
 
   double yaw[2], vz[2], gx[2], gy[2], vdes[2];
   bool goal[2], mine[2];
@@ -77,14 +94,13 @@ __global__ void __launch_bounds__(kWarps * 32) smpc_crowd_step_kernel(smpc_crowd
   if (a.people_log && a.k == 0)  // row 0 = the input state
     for (int e = lane; e < K * 5; e += 32) a.people_log[(size_t)b * (a.T + 1) * K * 5 + e] = P[e];
 
-  double dist = 0.0;
   for (int sub = 0; sub < a.substeps; ++sub) {
-    if (lane == 0) {  // the robot as agent n
+    if (lane < R) {  // robot r as agent n + r
       const double ts = __dmul_rn((double)sub, dts);
-      s.px[n] = __dadd_rn(rx, __dmul_rn(ts, rvx));
-      s.py[n] = __dadd_rn(ry, __dmul_rn(ts, rvy));
-      s.vx[n] = rvx;
-      s.vy[n] = rvy;
+      s.px[n + lane] = __dadd_rn(rx, __dmul_rn(ts, rvx));
+      s.py[n + lane] = __dadd_rn(ry, __dmul_rn(ts, rvy));
+      s.vx[n + lane] = rvx;
+      s.vy[n + lane] = rvy;
     }
     __syncwarp();
     for (int q = 0; q < 2; ++q) {
@@ -111,16 +127,19 @@ __global__ void __launch_bounds__(kWarps * 32) smpc_crowd_step_kernel(smpc_crowd
           fy = -vy / kRelax;
         }
       }
-      // social force from every other person, then from the robot (sfm.hpp:239-281)
+      // social force from every other person, then from the robots (sfm.hpp:239-281)
       double2 f = make_double2(0.0, 0.0);
       for (int k = 0; k < n; ++k) {
         if (k == slot) continue;
         f = smpc::sfm_pair(s.px[k] - px, s.py[k] - py, vx - s.vx[k], vy - s.vy[k], f.x, f.y);
       }
-      const double2 fr = smpc::sfm_pair(s.px[n] - px, s.py[n] - py, vx - s.vx[n], vy - s.vy[n], 0.0, 0.0);
-      f.x += fr.x;
-      f.y += fr.y;
-      dist += sqrt(fr.x * fr.x + fr.y * fr.y) * dts;
+      for (int r = 0; r < R; ++r) {
+        const int j = n + r;
+        const double2 fr = smpc::sfm_pair(s.px[j] - px, s.py[j] - py, vx - s.vx[j], vy - s.vy[j], 0.0, 0.0);
+        f.x += fr.x;
+        f.y += fr.y;
+        s.dist[r][lane] += sqrt(fr.x * fr.x + fr.y * fr.y) * dts;
+      }
       fx += f.x;
       fy += f.y;
       // obstacle force (sfm.hpp:206-221) of the nearest obstacle cell at the current position; none outside the grid
@@ -179,8 +198,11 @@ __global__ void __launch_bounds__(kWarps * 32) smpc_crowd_step_kernel(smpc_crowd
     __syncwarp();
   }
 
-  for (int off = 16; off > 0; off >>= 1) dist += __shfl_xor_sync(0xffffffffu, dist, off);
-  if (lane == 0) a.disturbance[b] += dist;
+  for (int r = 0; r < R; ++r) {
+    double dist = s.dist[r][lane];
+    for (int off = 16; off > 0; off >>= 1) dist += __shfl_xor_sync(0xffffffffu, dist, off);
+    if (lane == 0 && a.active[r0 + r]) a.disturbance[r0 + r] += dist;
+  }
   double* log = a.people_log ? a.people_log + ((size_t)b * (a.T + 1) + a.k + 1) * K * 5 : nullptr;
   for (int q = 0; q < 2; ++q) {
     const int slot = lane + 32 * q;

@@ -1,14 +1,17 @@
-// smpc_episode.cu — closed-loop episodes (smpc_run_episodes, smpc_run_crowd_episodes): B robots through their crowd
-// scenes for up to T controller ticks, every tick enqueued on the handle's stream without a host round trip. One tick
-// per episode is
-//   trajectorizer (seed) -> tick prep (constant-velocity people at k * dt_c, seed repack, max_time cut) -> FOV filter
-//   -> fleet tick (smpc_fleet_tick_enqueue) -> [reactive crowd step, smpc_crowd.cu] -> world step (robot Euler step,
-//   metrics, goal check, logs).
-// Both entries share one loop: with a crowd the prep leaves the people alone, the FOV filter and the world step read
-// the crowd's state, and the crowd step moves it from tick k to k + 1. The fleet tick runs on the handle's third fleet
-// state, so episodes never touch the warm-start memory of smpc_optimize_batch or smpc_optimize.
+// smpc_episode.cu — closed-loop episodes (smpc_run_episodes, smpc_run_crowd_episodes, smpc_run_shared_episodes): B
+// robots through their crowd scenes for up to T controller ticks, every tick enqueued on the handle's stream without a
+// host round trip. One tick per episode is
+//   trajectorizer (seed) -> tick prep (constant-velocity people at k * dt_c, seed repack, max_time cut) -> [scene view]
+//   -> FOV filter -> fleet tick (smpc_fleet_tick_enqueue) -> [reactive crowd step, smpc_crowd.cu] -> world step (robot
+//   Euler step, metrics, goal check, logs) -> [robot-robot metrics].
+// All entries share one loop: with a crowd the prep leaves the people alone, the FOV filter and the world step read
+// the crowd's state, and the crowd step moves it from tick k to k + 1. Shared scenes (R robots per scene, one crowd per
+// scene) add the scene view, which puts the other robots of the scene in front of the people the FOV filter sees, and
+// the robot-robot metrics. The fleet tick runs on the handle's third fleet state, so episodes never touch the
+// warm-start memory of smpc_optimize_batch or smpc_optimize.
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <mutex>
@@ -21,7 +24,9 @@
 namespace {
 
 constexpr int kPollTicks = 16;  // ticks between two reads of the device count of active episodes
-constexpr int kCrowdMaxPeople = 63;  // people + robot in the 64 agent slots of smpc_crowd_step_kernel
+constexpr int kCrowdMaxAgents = 64;  // people + robots in the agent slots of smpc_crowd_step_kernel
+constexpr int kMaxRobotsPerScene = 8;
+constexpr double kIntimate = 0.45;  // m, the intimate zone of the person metrics
 // The trajectorizer produces no step within this distance of the path end (smpc_trajectorize_kernel,
 // src/path_trajectorizer.cpp:152). A robot that close has no seed, so the fleet tick leaves it inactive and its
 // command is zero: a goal tolerance below this distance could leave it standing short of the goal until T.
@@ -83,13 +88,14 @@ __global__ void smpc_episode_prep_kernel(EpisodePrep a) {
 }
 
 struct EpisodeStep {
-  int B, K, T, k, stride, n_path;
+  int B, R, K, T, k, stride, n_path;  // R robots per scene: robot b sees the people of scene b / R
   double dt_c, goal_tol;
   const double* cmds;          // [B][stride][2] fleet tick output: row 0 is the command
   const uint8_t* optimized;    // [B]
-  const double* people0;       // [B][K][5]
-  const double* people_now;    // [B][K][5] people at (k+1) * dt_c (reactive crowd), or NULL: people0 at constant velocity
-  const int32_t* n_people;     // [B] or NULL (K == 0)
+  const double* people0;       // [B/R][K][5]
+  const double* people_now;    // [B/R][K][5] people at (k+1) * dt_c (reactive crowd), or NULL: people0 at constant
+                               // velocity
+  const int32_t* n_people;     // [B/R] or NULL (K == 0)
   const double* global_path;   // [B][N][2]
   const uint8_t* maps;
   const double* map_org;
@@ -119,7 +125,7 @@ __device__ __forceinline__ double hypot_rn(double dx, double dy) {  // no FMA co
 }
 
 // One warp per episode, lanes over people. Robot: unicycle forward Euler over dt_c, yaw through setRPY / getYaw.
-// Metrics at time (k+1) * dt_c against all people of the scene (not only those the FOV filter kept).
+// Metrics at time (k+1) * dt_c against all people of the scene (not only those the FOV filter kept; no robots).
 __global__ void __launch_bounds__(128) smpc_episode_step_kernel(EpisodeStep a) {
   const int b = (blockIdx.x * blockDim.x + threadIdx.x) >> 5, lane = threadIdx.x & 31;
   if (b >= a.B || !a.active[b]) return;  // warp-uniform
@@ -137,15 +143,16 @@ __global__ void __launch_bounds__(128) smpc_episode_step_kernel(EpisodeStep a) {
 
   // nearest person at (k+1) * dt_c
   const double t1 = __dmul_rn((double)(a.k + 1), a.dt_c);
-  const int np = a.K > 0 ? a.n_people[b] : 0;
+  const int sc = b / a.R;
+  const int np = a.K > 0 ? a.n_people[sc] : 0;
   double dmin = INFINITY;
   for (int j = lane; j < np; j += 32) {
     double px, py;
     if (a.people_now) {
-      px = a.people_now[((size_t)b * a.K + j) * 5];
-      py = a.people_now[((size_t)b * a.K + j) * 5 + 1];
+      px = a.people_now[((size_t)sc * a.K + j) * 5];
+      py = a.people_now[((size_t)sc * a.K + j) * 5 + 1];
     } else {
-      const double* p = a.people0 + ((size_t)b * a.K + j) * 5;
+      const double* p = a.people0 + ((size_t)sc * a.K + j) * 5;
       px = __dadd_rn(p[0], __dmul_rn(p[2], t1));
       py = __dadd_rn(p[1], __dmul_rn(p[3], t1));
     }
@@ -170,7 +177,7 @@ __global__ void __launch_bounds__(128) smpc_episode_step_kernel(EpisodeStep a) {
   if (a.k == 0) {
     a.path_length[b] = step;
     a.min_dist[b] = dmin;
-    a.intimate[b] = dmin < 0.45;
+    a.intimate[b] = dmin < kIntimate;
     a.personal[b] = dmin < 1.2;
     a.collision[b] = cost >= 253;
     a.not_optimized[b] = !opt;
@@ -182,7 +189,7 @@ __global__ void __launch_bounds__(128) smpc_episode_step_kernel(EpisodeStep a) {
   } else {
     a.path_length[b] = __dadd_rn(a.path_length[b], step);
     a.min_dist[b] = fmin(a.min_dist[b], dmin);
-    a.intimate[b] += dmin < 0.45;
+    a.intimate[b] += dmin < kIntimate;
     a.personal[b] += dmin < 1.2;
     a.collision[b] += cost >= 253;
     a.not_optimized[b] += !opt;
@@ -211,8 +218,75 @@ __global__ void __launch_bounds__(128) smpc_episode_step_kernel(EpisodeStep a) {
   }
 }
 
-// The loop of both entries; crowd == NULL: constant-velocity people (smpc_run_episodes).
-int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd, const char* name) {
+struct SceneView {
+  int B, R, K, n_view;  // n_view = R - 1 + K rows per robot
+  const uint8_t* active;    // [B]
+  const double* pose;       // [B][3] x_k
+  const double* speed;      // [B][2] measured speed of tick k
+  const double* people;     // [B/R][K][5] the crowd after k steps
+  const int32_t* n_people;  // [B/R] or NULL (K == 0)
+  double* view;             // [B][n_view][5] the FOV filter's input
+  int32_t* n_view_each;     // [B]
+};
+
+// One thread per (robot, row): rows 0 .. R-2 hold the other robots of the scene in index order as people
+// (x, y, v cos th, v sin th, w) with the measured speed of tick k (zero once a robot is done), then the scene's people.
+// Robots go first because the FOV filter keeps the first n_agents survivors.
+__global__ void smpc_scene_view_kernel(SceneView a) {
+  const long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= (long long)a.B * a.n_view) return;
+  const int b = (int)(t / a.n_view), i = (int)(t % a.n_view);
+  const int sc = b / a.R, me = b % a.R;
+  double* o = a.view + ((size_t)b * a.n_view + i) * 5;
+  if (i < a.R - 1) {
+    const int ob = sc * a.R + (i < me ? i : i + 1);
+    const bool on = a.active[ob] != 0;
+    const double v = on ? a.speed[2 * ob] : 0.0, w = on ? a.speed[2 * ob + 1] : 0.0;
+    double st, ct;
+    sincos(a.pose[3 * ob + 2], &st, &ct);
+    o[0] = a.pose[3 * ob];
+    o[1] = a.pose[3 * ob + 1];
+    o[2] = __dmul_rn(v, ct);
+    o[3] = __dmul_rn(v, st);
+    o[4] = w;
+  } else {
+    const double* p = a.people + ((size_t)sc * a.K + (i - (a.R - 1))) * 5;
+    for (int q = 0; q < 5; ++q) o[q] = p[q];
+  }
+  if (i == 0) a.n_view_each[b] = a.R - 1 + (a.K > 0 ? a.n_people[sc] : 0);
+}
+
+struct RobotMetrics {
+  int B, R, k;
+  const double* pose;    // [B][3] x_k+1 (after the world step)
+  const int32_t* ticks;  // [B] == k + 1 for the robots that ran tick k
+  double* min_dist;      // [B]
+  int32_t* intimate;     // [B]
+};
+
+// One thread per robot that ran tick k: the nearest other robot of its scene at (k+1) * dt_c (finished robots stand
+// at their final pose). +inf with one robot per scene.
+__global__ void smpc_robot_metrics_kernel(RobotMetrics a) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= a.B || a.ticks[b] != a.k + 1) return;
+  const int r0 = b - b % a.R;
+  const double x = a.pose[3 * b], y = a.pose[3 * b + 1];
+  double dmin = INFINITY;
+  for (int o = r0; o < r0 + a.R; ++o)
+    if (o != b) dmin = fmin(dmin, hypot_rn(__dsub_rn(a.pose[3 * o], x), __dsub_rn(a.pose[3 * o + 1], y)));
+  if (a.k == 0) {
+    a.min_dist[b] = dmin;
+    a.intimate[b] = dmin < kIntimate;
+  } else {
+    a.min_dist[b] = fmin(a.min_dist[b], dmin);
+    a.intimate[b] += dmin < kIntimate;
+  }
+}
+
+// The loop of all entries; crowd == NULL: constant-velocity people (smpc_run_episodes); scene == NULL: one robot per
+// scene (smpc_run_episodes, smpc_run_crowd_episodes).
+int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd, const smpc_scene_io* scene,
+                 const char* name) {
   auto fail_arg = [name](const char* msg) {
     return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string(name) + ": " + msg);
   };
@@ -243,20 +317,31 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
   if (!io->reached || !io->ticks || !io->path_length || !io->min_person_dist || !io->intimate_ticks ||
       !io->personal_ticks || !io->collision_ticks || !io->not_optimized_ticks || !io->cmd_variation)
     return fail_arg("missing output");
+  const int R = scene ? scene->robots_per_scene : 1;
+  if (R < 1 || R > kMaxRobotsPerScene) return fail_arg("robots_per_scene outside 1..8");
+  if (B % R != 0) return fail_arg("n_episodes not a multiple of robots_per_scene");
+  if (scene && (!scene->robot_min_dist || !scene->robot_intimate_ticks)) return fail_arg("missing output");
+  const int S = B / R;  // scenes: people, n_people_each, goals, desired_speed and people_log have S rows
+  for (int c = 0; c < S && K > 0; ++c)
+    if (io->n_people_each[c] < 0 || io->n_people_each[c] > K) return fail_arg("n_people_each[b] outside 0..K");
   for (int b = 0; b < B; ++b) {
-    if (K > 0 && (io->n_people_each[b] < 0 || io->n_people_each[b] > K)) return fail_arg("n_people_each[b] outside 0..K");
     if (io->costmap_index && (io->costmap_index[b] < 0 || io->costmap_index[b] >= io->n_costmaps))
       return fail_arg("costmap_index[b] outside 0..n_costmaps-1");
     if (io->od_index && (io->od_index[b] < 0 || io->od_index[b] >= io->n_od_grids))
       return fail_arg("od_index[b] outside 0..n_od_grids-1");
+    const int r0 = b - b % R;  // the robots of a scene share its costmap and obstacle grid
+    if ((io->costmap_index ? io->costmap_index[b] != io->costmap_index[r0] : b % io->n_costmaps != r0 % io->n_costmaps) ||
+        (io->od_index ? io->od_index[b] != io->od_index[r0] : b % io->n_od_grids != r0 % io->n_od_grids))
+      return fail_arg("costmap_index or od_index differs within a scene");
   }
   const bool reactive = crowd != nullptr;
   if (reactive) {
-    if (K > kCrowdMaxPeople) return fail_arg("n_people above 63 (people + robot share one warp's 64 slots)");
+    if (K + R > kCrowdMaxAgents)
+      return fail_arg("n_people + robots_per_scene above 64 (people and robots share one warp's 64 slots)");
     if (crowd->substeps < 1 || crowd->substeps > 64) return fail_arg("substeps outside 1..64");
     if (K > 0 && (!crowd->goals || !crowd->desired_speed)) return fail_arg("missing goals or desired speeds");
     if (!crowd->people_disturbance) return fail_arg("missing output");
-    for (int b = 0; b < B && K > 0; ++b)
+    for (int b = 0; b < S && K > 0; ++b)
       for (int i = 0; i < io->n_people_each[b]; ++i) {
         const double* g = crowd->goals + ((size_t)b * K + i) * 2;
         const double vd = crowd->desired_speed[(size_t)b * K + i];
@@ -290,10 +375,14 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
   // ---- maps, uploaded once per call
   const size_t map_bytes = (size_t)io->n_costmaps * io->size_x * io->size_y;
   const size_t od_bytes = (size_t)io->n_od_grids * io->od_width * io->od_height * sizeof(uint32_t);
-  const size_t Bz = B, Kz = K, BS = Bz * stride;
+  const size_t Bz = B, Sz = S, Kz = K, BS = Bz * stride;
+  const int n_view = scene ? R - 1 + K : 0;  // rows of a robot's scene view (0: the FOV filter reads the people)
+  const bool fov = scene ? n_view > 0 : K > 0;
   const bool logs_pose = io->pose_log != nullptr, logs_cmd = io->cmd_log != nullptr, logs_opt = io->optimized_log != nullptr;
   const bool logs_people = reactive && crowd->people_log != nullptr;
   double *goals = nullptr, *vdes = nullptr, *disturbance = nullptr, *people_log = nullptr;
+  double *view = nullptr, *robot_min = nullptr;
+  int32_t *view_n = nullptr, *robot_intimate = nullptr;
   uint8_t* has_goal = nullptr;
   int32_t* n_people_dev = nullptr;
   double *gp, *pose, *people0, *people, *seed_cmds, *pose_log, *cmd_log, *path_length, *min_dist, *cmd_var;
@@ -312,9 +401,9 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
     gp = c.take<double>(Bz * N * 2);
     pose = c.take<double>(Bz * 3);
     speed = c.take<double>(Bz * 2);
-    people0 = c.take<double>(Bz * Kz * 5);
-    people = c.take<double>(Bz * Kz * 5);
-    n_people_dev = c.take<int32_t>(Bz);
+    people0 = c.take<double>(Sz * Kz * 5);
+    people = c.take<double>(Sz * Kz * 5);
+    n_people_dev = c.take<int32_t>(Sz);
     seed_cmds = c.take<double>(Bz * max_steps * 3);
     n_steps = c.take<int32_t>(Bz);
     fov_people = c.take<double>(Bz * A * 5);
@@ -340,11 +429,17 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
     cmd_log = c.take<double>(logs_cmd ? Bz * T * 2 : 0);
     opt_log = c.take<uint8_t>(logs_opt ? Bz * T : 0);
     if (reactive) {  // people holds the crowd's state of the current tick
-      goals = c.take<double>(Bz * Kz * 2);
-      vdes = c.take<double>(Bz * Kz);
-      has_goal = c.take<uint8_t>(Bz * Kz);
+      goals = c.take<double>(Sz * Kz * 2);
+      vdes = c.take<double>(Sz * Kz);
+      has_goal = c.take<uint8_t>(Sz * Kz);
       disturbance = c.take<double>(Bz);
-      people_log = c.take<double>(logs_people ? Bz * (T + 1) * Kz * 5 : 0);
+      people_log = c.take<double>(logs_people ? Sz * (T + 1) * Kz * 5 : 0);
+    }
+    if (scene) {
+      view = c.take<double>(Bz * n_view * 5);
+      view_n = c.take<int32_t>(Bz);
+      robot_min = c.take<double>(Bz);
+      robot_intimate = c.take<int32_t>(Bz);
     }
   };
   size_t need = 0;
@@ -364,16 +459,16 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       {map_org, io->costmap_origin, (size_t)io->n_costmaps * 16}, {od_org, io->od_origin, (size_t)io->n_od_grids * 16},
       {map_index, io->costmap_index, Bz * 4}, {od_index, io->od_index, Bz * 4},
       {gp, io->global_path, Bz * N * 16}, {pose, io->pose, Bz * 24}, {speed, io->speed, Bz * 16},
-      {people0, K > 0 ? io->people : nullptr, Bz * Kz * 40}, {n_people_dev, K > 0 ? io->n_people_each : nullptr, Bz * 4},
+      {people0, K > 0 ? io->people : nullptr, Sz * Kz * 40}, {n_people_dev, K > 0 ? io->n_people_each : nullptr, Sz * 4},
   };
   for (const Up& u : ups)
     if (u.host && u.bytes) SMPC_FLEET_CUDA(cudaMemcpyAsync(u.dev, u.host, u.bytes, cudaMemcpyHostToDevice, st));
   if (reactive) {
     if (K > 0) {
-      SMPC_FLEET_CUDA(cudaMemcpyAsync(people, io->people, Bz * Kz * 40, cudaMemcpyHostToDevice, st));
-      SMPC_FLEET_CUDA(cudaMemcpyAsync(goals, crowd->goals, Bz * Kz * 16, cudaMemcpyHostToDevice, st));
-      SMPC_FLEET_CUDA(cudaMemcpyAsync(vdes, crowd->desired_speed, Bz * Kz * 8, cudaMemcpyHostToDevice, st));
-      SMPC_FLEET_CUDA(cudaMemsetAsync(has_goal, 1, Bz * Kz, st));
+      SMPC_FLEET_CUDA(cudaMemcpyAsync(people, io->people, Sz * Kz * 40, cudaMemcpyHostToDevice, st));
+      SMPC_FLEET_CUDA(cudaMemcpyAsync(goals, crowd->goals, Sz * Kz * 16, cudaMemcpyHostToDevice, st));
+      SMPC_FLEET_CUDA(cudaMemcpyAsync(vdes, crowd->desired_speed, Sz * Kz * 8, cudaMemcpyHostToDevice, st));
+      SMPC_FLEET_CUDA(cudaMemsetAsync(has_goal, 1, Sz * Kz, st));
     }
     SMPC_FLEET_CUDA(cudaMemsetAsync(disturbance, 0, Bz * 8, st));
   }
@@ -398,16 +493,17 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
   ta.global_path = gp; ta.path_index = nullptr; ta.pose = pose; ta.poses = d.poses; ta.cmds = seed_cmds; ta.n_steps = n_steps;
 
   smpc_fov_args fa{};
-  fa.n_robots = B; fa.n_in_max = K; fa.n_out_max = A; fa.n_costmaps = io->n_costmaps;
+  fa.n_robots = B; fa.n_in_max = scene ? n_view : K; fa.n_out_max = A; fa.n_costmaps = io->n_costmaps;
   fa.size_x = io->size_x; fa.size_y = io->size_y; fa.resolution = io->resolution; fa.fov_angle = prm->fov_angle;
-  fa.people_in = people; fa.n_people_in = n_people_dev; fa.pose = pose; fa.costmap_origin = map_org;
+  fa.people_in = scene ? view : people; fa.n_people_in = scene ? view_n : n_people_dev; fa.pose = pose;
+  fa.costmap_origin = map_org;
   fa.costmap_index = d.map_index; fa.people_out = fov_people; fa.n_people_out = fov_n;
 
   // with a crowd the prep moves nobody (K = 0 there): the crowd step does
   EpisodePrep pp{B, reactive ? 0 : K, stride, max_steps, maxsize, 0.0, n_steps, seed_cmds, active, people0, people, d.poses, d.cmds,
                  const_cast<int32_t*>(d.n_in), const_cast<int32_t*>(d.n_each), const_cast<int32_t*>(d.s_each)};
   EpisodeStep es{};
-  es.B = B; es.K = K; es.T = T; es.stride = stride; es.n_path = N;
+  es.B = B; es.R = R; es.K = K; es.T = T; es.stride = stride; es.n_path = N;
   es.dt_c = io->control_period; es.goal_tol = io->goal_tolerance;
   es.cmds = d.cmds; es.optimized = d.optimized; es.people0 = people0; es.n_people = K > 0 ? n_people_dev : nullptr;
   es.global_path = gp; es.maps = maps; es.map_org = map_org; es.map_index = d.map_index;
@@ -423,7 +519,7 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
 
   smpc_crowd_step_args ca{};
   if (reactive) {
-    ca.B = B; ca.K = K; ca.T = T; ca.stride = stride; ca.substeps = crowd->substeps; ca.dt_c = io->control_period;
+    ca.B = S; ca.R = R; ca.K = K; ca.T = T; ca.stride = stride; ca.substeps = crowd->substeps; ca.dt_c = io->control_period;
     ca.active = active; ca.n_people = n_people_dev; ca.pose = pose; ca.cmds = d.cmds; ca.goals = goals; ca.vdes = vdes;
     ca.has_goal = has_goal; ca.people = people; ca.disturbance = disturbance;
     ca.people_log = logs_people ? people_log : nullptr;
@@ -431,8 +527,12 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
     ca.od_resolution = io->od_resolution; ca.od = od; ca.od_org = od_org; ca.od_index = d.od_index;
   }
 
+  const SceneView sv{B, R, K, n_view, active, pose, speed, people, K > 0 ? n_people_dev : nullptr, view, view_n};
+  RobotMetrics rm{B, R, 0, pose, ticks, robot_min, robot_intimate};
+
   const int prep_rows = stride > pp.K ? stride : pp.K;
   const unsigned g_prep = (unsigned)((Bz * prep_rows + 255) / 256), g_step = (unsigned)((Bz + 3) / 4);
+  const unsigned g_view = (unsigned)((Bz * n_view + 255) / 256), g_robots = (unsigned)((Bz + 255) / 256);
   for (int k = 0; k < T; ++k) {
     rc = smpc_trajectorize_batch_device(h, &ta, st);
     if (rc != SMPC_OK) return rc;
@@ -440,7 +540,12 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
     smpc_episode_prep_kernel<<<g_prep, 256, 0, st>>>(pp);
     SMPC_FLEET_CUDA(cudaGetLastError());
     smpc_handle_count_launch(h);
-    if (K > 0) {
+    if (scene && fov) {
+      smpc_scene_view_kernel<<<g_view, 256, 0, st>>>(sv);
+      SMPC_FLEET_CUDA(cudaGetLastError());
+      smpc_handle_count_launch(h);
+    }
+    if (fov) {
       rc = smpc_fov_filter_batch_device(h, &fa, st);
       if (rc != SMPC_OK) return rc;
     }
@@ -455,6 +560,12 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
     smpc_episode_step_kernel<<<g_step, 128, 0, st>>>(es);
     SMPC_FLEET_CUDA(cudaGetLastError());
     smpc_handle_count_launch(h);
+    if (scene) {  // needs every robot's pose at k + 1
+      rm.k = k;
+      smpc_robot_metrics_kernel<<<g_robots, 256, 0, st>>>(rm);
+      SMPC_FLEET_CUDA(cudaGetLastError());
+      smpc_handle_count_launch(h);
+    }
     if ((k + 1) % kPollTicks == 0 && k + 1 < T) {
       SMPC_FLEET_CUDA(cudaMemcpyAsync(host_active, n_active, sizeof(int), cudaMemcpyDeviceToHost, st));
       SMPC_FLEET_CUDA(cudaStreamSynchronize(st));
@@ -473,7 +584,9 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       {logs_cmd ? io->cmd_log : nullptr, cmd_log, Bz * T * 16},
       {logs_opt ? io->optimized_log : nullptr, opt_log, Bz * T},
       {reactive ? crowd->people_disturbance : nullptr, disturbance, Bz * 8},
-      {logs_people ? crowd->people_log : nullptr, people_log, Bz * (T + 1) * Kz * 40},
+      {logs_people ? crowd->people_log : nullptr, people_log, Sz * (T + 1) * Kz * 40},
+      {scene ? scene->robot_min_dist : nullptr, robot_min, Bz * 8},
+      {scene ? scene->robot_intimate_ticks : nullptr, robot_intimate, Bz * 4},
   };
   for (const Down& c : downs)
     if (c.host) SMPC_FLEET_CUDA(cudaMemcpyAsync(c.host, c.dev, c.bytes, cudaMemcpyDeviceToHost, st));
@@ -487,10 +600,13 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
         std::memcpy(io->pose_log + ((size_t)b * (T + 1) + k) * 3, io->pose_log + ((size_t)b * (T + 1) + tb) * 3, 24);
     if (logs_cmd) std::memset(io->cmd_log + ((size_t)b * T + tb) * 2, 0, (size_t)(T - tb) * 16);
     if (logs_opt) std::memset(io->optimized_log + (size_t)b * T + tb, 0, (size_t)(T - tb));
-    if (logs_people)  // the people of a finished episode stand where they were at its last tick
-      for (int k = tb + 1; k <= T; ++k)
-        std::memcpy(crowd->people_log + ((size_t)b * (T + 1) + k) * Kz * 5,
-                    crowd->people_log + ((size_t)b * (T + 1) + tb) * Kz * 5, Kz * 40);
+  }
+  for (int c = 0; c < S && logs_people; ++c) {  // the people of a finished scene stand where they were at its last tick
+    int tc = 0;
+    for (int r = 0; r < R; ++r) tc = std::max(tc, (int)io->ticks[c * R + r]);
+    for (int k = tc + 1; k <= T; ++k)
+      std::memcpy(crowd->people_log + ((size_t)c * (T + 1) + k) * Kz * 5,
+                  crowd->people_log + ((size_t)c * (T + 1) + tc) * Kz * 5, Kz * 40);
   }
   return SMPC_OK;
 }
@@ -498,10 +614,17 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
 }  // namespace
 
 extern "C" int smpc_run_episodes(smpc_handle* h, smpc_episode_io* io) {
-  return run_episodes(h, io, nullptr, "run_episodes");
+  return run_episodes(h, io, nullptr, nullptr, "run_episodes");
 }
 
 extern "C" int smpc_run_crowd_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd) {
   if (!crowd) return smpc_host_fail(SMPC_ERR_ARGUMENT, "run_crowd_episodes: NULL crowd");
-  return run_episodes(h, io, crowd, "run_crowd_episodes");
+  return run_episodes(h, io, crowd, nullptr, "run_crowd_episodes");
+}
+
+extern "C" int smpc_run_shared_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd,
+                                        const smpc_scene_io* scene) {
+  if (!crowd) return smpc_host_fail(SMPC_ERR_ARGUMENT, "run_shared_episodes: NULL crowd");
+  if (!scene) return smpc_host_fail(SMPC_ERR_ARGUMENT, "run_shared_episodes: NULL scene");
+  return run_episodes(h, io, crowd, scene, "run_shared_episodes");
 }

@@ -137,26 +137,27 @@ cudaError_t smpc_fleet_memory(smpc_fleet_state* fs, smpc_fleet_dev* d, cudaStrea
 // the finish (outputs, memory update). No host synchronisation.
 int smpc_fleet_tick_enqueue(smpc_handle* h, const smpc_fleet_dev& d, cudaStream_t st);
 
-// One controller tick of the reactive crowd of smpc_run_crowd_episodes (smpc_crowd.cu), all device pointers.
+// One controller tick of the reactive crowd of smpc_run_crowd_episodes / smpc_run_shared_episodes (smpc_crowd.cu), all
+// device pointers. B scenes of R robots each: robot r of scene b is robot b * R + r (R = 1: one robot per scene).
 struct smpc_crowd_step_args {
-  int B, K, T, k, stride, substeps;
+  int B, R, K, T, k, stride, substeps;
   double dt_c;
-  const uint8_t* active;       // [B] episodes still running; the others keep their people
+  const uint8_t* active;       // [B*R] robots still running; a scene none of whose robots runs keeps its people
   const int32_t* n_people;     // [B] people of each scene (<= K)
-  const double* pose;          // [B][3] robot pose of tick k
-  const double* cmds;          // [B][stride][2] fleet tick output: row 0 is the command of tick k
+  const double* pose;          // [B*R][3] robot pose of tick k
+  const double* cmds;          // [B*R][stride][2] fleet tick output: row 0 is the command of tick k
   const double* goals;         // [B][K][2]
   const double* vdes;          // [B][K]
   uint8_t* has_goal;           // [B][K] lightsfm goal flags
   double* people;              // [B][K][5] in: tick k, out: tick k + 1
-  double* disturbance;         // [B] accumulated
+  double* disturbance;         // [B*R] accumulated while the robot runs
   double* people_log;          // [B][T+1][K][5] or NULL
   int n_od_grids;
   uint32_t od_width, od_height;
   float od_resolution;
   const uint32_t* od;
   const double* od_org;
-  const int32_t* od_index;     // may be NULL (grid b % n_od_grids)
+  const int32_t* od_index;     // [B*R], equal within a scene, or NULL (grid (b * R) % n_od_grids)
 };
 // Enqueues smpc_crowd_step_kernel on st (one launch).
 int smpc_crowd_step_enqueue(smpc_handle* h, const smpc_crowd_step_args& a, cudaStream_t st);

@@ -193,22 +193,51 @@ class FleetOptimizer:
         per control period, and give way to the robot; people [B][K][5] is their state at t = 0. Returns the dict of
         run_episodes plus people_disturbance [B] (sum of |F(robot -> person)| * dt_s over ticks, substeps and people);
         with want_logs also people_log [B][T+1][K][5] (x, y, vx, vy, vz at every tick, row 0 = the input)."""
+        return self._crowd_run(None, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
+                               costmap_resolution, od, ticks, goals, desired_speed, substeps, control_period,
+                               goal_tolerance, costmap_index, od_index, want_logs)
+
+    def run_shared_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
+                            costmap_resolution, od: dict, ticks: int, goals, desired_speed, robots_per_scene,
+                            substeps=1, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
+                            want_logs=False) -> dict:
+        """Closed-loop episodes in shared scenes (smpc_run_shared_episodes): run_crowd_episodes with the B robots
+        grouped into S = B / R scenes of R = robots_per_scene consecutive robots that share one crowd, costmap and
+        obstacle grid, and that see each other as people. Per robot: global_path [B][N][2], pose [B][3],
+        speed [B][2], costmap_index / od_index [B] (equal within a scene). Per scene: people [S][K][5],
+        n_people [S], goals [S][K][2], desired_speed [S][K]. Returns the dict of run_crowd_episodes plus
+        robot_min_dist [B] (nearest other robot of the scene, inf for R = 1) and robot_intimate_ticks [B]; with
+        want_logs people_log is per scene, [S][T+1][K][5]."""
+        return self._crowd_run(int(robots_per_scene), global_path, pose, speed, people, n_people, costmaps,
+                               costmap_origin, costmap_resolution, od, ticks, goals, desired_speed, substeps,
+                               control_period, goal_tolerance, costmap_index, od_index, want_logs)
+
+    def _crowd_run(self, R, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
+                   od, ticks, goals, desired_speed, substeps, control_period, goal_tolerance, costmap_index, od_index,
+                   want_logs) -> dict:
+        """run_crowd_episodes (R None) or run_shared_episodes (R robots per scene)."""
         io, out, logs, keep = self.episode_io(global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                                               costmap_resolution, od, ticks, control_period, goal_tolerance,
-                                              costmap_index, od_index, want_logs)
+                                              costmap_index, od_index, want_logs, robots_per_scene=R or 1)
         B, T, K = self.B, int(ticks), io.n_people
-        goals = np.ascontiguousarray(goals, dtype=np.float64).reshape(B, K, 2)
-        vdes = np.ascontiguousarray(desired_speed, dtype=np.float64).reshape(B, K)
+        S = B // (R or 1)
+        goals = np.ascontiguousarray(goals, dtype=np.float64).reshape(S, K, 2)
+        vdes = np.ascontiguousarray(desired_speed, dtype=np.float64).reshape(S, K)
         crowd = abi.SmpcCrowdIo()
         crowd.goals = goals.ctypes.data if K > 0 else None
         crowd.desired_speed = vdes.ctypes.data if K > 0 else None
         crowd.substeps = int(substeps)
         disturbance = np.zeros(B)
         crowd.people_disturbance = disturbance.ctypes.data
-        people_log = np.zeros((B, T + 1, K, 5)) if want_logs else None
+        people_log = np.zeros((S, T + 1, K, 5)) if want_logs else None
         crowd.people_log = None if people_log is None else people_log.ctypes.data
-        _lib.check(_lib.lib().smpc_run_crowd_episodes(self.opt._h, C.byref(io), C.byref(crowd)))
         res = dict(out, **logs)
+        if R is None:
+            _lib.check(_lib.lib().smpc_run_crowd_episodes(self.opt._h, C.byref(io), C.byref(crowd)))
+        else:
+            res.update(robot_min_dist=np.zeros(B), robot_intimate_ticks=np.zeros(B, np.int32))
+            scene = abi.SmpcSceneIo(R, res["robot_min_dist"].ctypes.data, res["robot_intimate_ticks"].ctypes.data)
+            _lib.check(_lib.lib().smpc_run_shared_episodes(self.opt._h, C.byref(io), C.byref(crowd), C.byref(scene)))
         res["reached"] = out["reached"].astype(bool)
         res["people_disturbance"] = disturbance
         if want_logs:
@@ -218,17 +247,19 @@ class FleetOptimizer:
 
     def episode_io(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
                    od: dict, ticks: int, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                   want_logs=False):
-        """The smpc_episode_io of run_episodes with its output arrays: (io, metrics, logs, inputs kept alive)."""
+                   want_logs=False, robots_per_scene=1):
+        """The smpc_episode_io of run_episodes with its output arrays: (io, metrics, logs, inputs kept alive).
+        people and n_people have one row per scene of robots_per_scene robots."""
         B, T = self.B, int(ticks)
+        S = B // robots_per_scene
         gp = np.ascontiguousarray(global_path, dtype=np.float64)
         assert gp.ndim == 3 and gp.shape[0] == B and gp.shape[2] == 2
         pose = np.ascontiguousarray(pose, dtype=np.float64).reshape(B, 3)
         speed = np.ascontiguousarray(speed, dtype=np.float64).reshape(B, 2)
         people = np.ascontiguousarray(people, dtype=np.float64)
         K = people.shape[1] if people.ndim == 3 else 0
-        people = people.reshape(B, K, 5)
-        n_people = np.ascontiguousarray(n_people, dtype=np.int32).reshape(B)
+        people = people.reshape(S, K, 5)
+        n_people = np.ascontiguousarray(n_people, dtype=np.int32).reshape(S)
         costmaps = np.ascontiguousarray(costmaps, dtype=np.uint8)
         morg = np.ascontiguousarray(costmap_origin, dtype=np.float64).reshape(-1, 2)
         oorg = np.ascontiguousarray(od["origins"], dtype=np.float64).reshape(-1, 2)

@@ -513,6 +513,16 @@ def crowd_episodes(B: int, K: int, seed: int = 6, ticks: int = 200, substeps: in
     projected person never leaves the grid. Returns the keyword arguments of run_crowd_episodes plus `params` and
     `ticks`."""
     s = episodes(B, 0, param_set=param_set, seed=seed, ticks=ticks, **kw)
+    people, goal, vdes = _place_crowd(s, K, seed, s["pose"][:, None, :2])
+    s.update(people=people, n_people=np.full(B, K, dtype=np.int32), goals=goal, desired_speed=vdes,
+             substeps=substeps)
+    return s
+
+
+def _place_crowd(s: dict, K: int, seed: int, robots: np.ndarray):
+    """The people of crowd_episodes for the scenes of s (episodes(B, 0, ...)): starts keep CROWD_CLEARANCE from every
+    robot start robots [B][R][2] and from lethal cells. Returns people [B][K][5], goals [B][K][2], desired speeds."""
+    B = robots.shape[0]
     p = s["params"]
     rng = _rng(900 + seed)
     od, res = s["od"], s["costmap_resolution"]
@@ -524,7 +534,6 @@ def crowd_episodes(B: int, K: int, seed: int = 6, ticks: int = 200, substeps: in
     onc, same, cross = kind == 0, kind == 1, kind == 2
     clear_ok = _lethal_clearance_ok(s["costmaps"], res, CROWD_CLEARANCE)
     cidx = s["costmap_index"]
-    pose = s["pose"]
 
     def draw(n):
         """starts [n][K][2] and goals [n][K][2] of n scenes"""
@@ -543,12 +552,14 @@ def crowd_episodes(B: int, K: int, seed: int = 6, ticks: int = 200, substeps: in
 
     start, goal = draw(B)
     todo = np.arange(B) if K > 0 else np.arange(0)
-    for it in range(400):  # redraw the people who break a rule; only scenes with such people are looked at again
+    for it in range(2000):  # redraw the people who break a rule; only scenes with such people are looked at again
         st = start[todo]
         mx = np.clip((st[..., 0] / res).astype(np.int64), 0, W - 1)
         my = np.clip((st[..., 1] / res).astype(np.int64), 0, H - 1)
         bad = ~clear_ok[cidx[todo][:, None], my, mx]
-        bad |= np.hypot(st[..., 0] - pose[todo, None, 0], st[..., 1] - pose[todo, None, 1]) < CROWD_CLEARANCE
+        rs = robots[todo]
+        bad |= np.hypot(st[:, :, None, 0] - rs[:, None, :, 0], st[:, :, None, 1] - rs[:, None, :, 1]).min(
+            axis=2, initial=np.inf) < CROWD_CLEARANCE
         d = np.hypot(st[:, :, None, 0] - st[:, None, :, 0], st[:, :, None, 1] - st[:, None, :, 1])
         d[:, np.tril_indices(K)[0], np.tril_indices(K)[1]] = np.inf  # each pair once: the later person moves
         bad |= (d < CROWD_SPACING).any(axis=1)
@@ -570,8 +581,70 @@ def crowd_episodes(B: int, K: int, seed: int = 6, ticks: int = 200, substeps: in
     people = np.zeros((B, K, 5))
     people[..., 0:2] = start
     people[..., 2:4] = heading * vdes[..., None]
-    s.update(people=people, n_people=np.full(B, K, dtype=np.int32), goals=goal, desired_speed=vdes,
-             substeps=substeps)
+    return people, goal, vdes
+
+
+SHARED_STAGGER = 1.5  # m between the starts (and the goals) of two robots of a scene going the same way
+SHARED_SPACING = 1.0  # m between any two robot starts of a scene
+SHARED_LATERAL = 0.3  # m: robot lanes lie within this distance of the corridor's centre line y = 2
+
+
+def shared_episodes(S: int, R: int, K: int, seed: int = 6, ticks: int = 200, substeps: int = 1,
+                    param_set: str = "soc_work_obst", **kw) -> dict:
+    """Shared scenes for FleetOptimizer.run_shared_episodes: the corridors of crowd_episodes(S, K, ...), each with R
+    robots (robot r of scene c is robot c * R + r) and one crowd of K people. Even robots drive +x, odd robots -x, so
+    they meet head-on. Each robot follows a straight path along its own lane y = 2 + u, |u| <= SHARED_LATERAL; robots
+    going the same way start (and end) SHARED_STAGGER apart along x, any two starts are at least SHARED_SPACING apart
+    and keep CROWD_CLEARANCE from lethal cells, and every path endpoint keeps EPISODE_MARGIN + 0.5 m/s * max_time from
+    the ends of the obstacle grid: the other robots enter a robot's controller as people, and a projected person must
+    not leave the grid. The people are placed as in crowd_episodes, clear of every robot start. Returns the keyword
+    arguments of run_shared_episodes (per robot: global_path, pose, speed, costmap_index; per scene: people, n_people,
+    goals, desired_speed) plus `params` and `ticks`. Raises ValueError when R robots do not fit the corridor."""
+    s = episodes(S, 0, param_set=param_set, seed=seed, ticks=ticks, **kw)
+    p = s["params"]
+    rng = _rng(1300 + seed)
+    od, res = s["od"], s["costmap_resolution"]
+    x_lo = EPISODE_MARGIN + 0.5 * f32(p.max_time)
+    x_hi = int(od["width"]) * od["resolution"] - x_lo
+    r = np.arange(R)
+    fwd = r % 2 == 0
+    n_fwd = (R + 1) // 2
+    length = x_hi - x_lo - SHARED_STAGGER * (n_fwd - 1)
+    x0 = np.where(fwd, x_lo + SHARED_STAGGER * (r // 2), x_hi - SHARED_STAGGER * (r // 2))
+    dx = np.abs(x0[:, None] - x0[None, :]) + np.where(np.eye(R, dtype=bool), np.inf, 0.0)
+    if R > 1 and (length < 1.0 or np.any(dx * dx + (2 * SHARED_LATERAL) ** 2 < SHARED_SPACING ** 2)):
+        raise ValueError(f"{R} robots per scene do not fit the corridor")
+    clear_ok = _lethal_clearance_ok(s["costmaps"], res, CROWD_CLEARANCE)
+    H, W = s["costmaps"].shape[1:]
+    cidx = s["costmap_index"]
+    mx = np.clip((x0 / res).astype(np.int64), 0, W - 1)
+    y = np.empty((S, R))
+    todo = np.arange(S)
+    for _ in range(400):  # redraw the lanes of scenes whose starts are too close or near a lethal cell
+        y[todo] = 2.0 + rng.uniform(-SHARED_LATERAL, SHARED_LATERAL, (todo.size, R))
+        yt = y[todo]
+        my = np.clip((yt / res).astype(np.int64), 0, H - 1)
+        bad = ~clear_ok[cidx[todo][:, None], my, mx[None, :]].all(axis=1)
+        d = np.hypot(dx[None], yt[:, :, None] - yt[:, None, :])
+        bad |= (d < SHARED_SPACING).any(axis=(1, 2))
+        todo = todo[bad]
+        if todo.size == 0:
+            break
+    else:
+        raise AssertionError("could not place the robots of a scene")
+    direction = np.where(fwd, 1.0, -1.0)
+    N = int(round(length / 0.05)) + 1
+    gpath = np.empty((S, R, N, 2))
+    gpath[..., 0] = x0[None, :, None] + direction[None, :, None] * np.linspace(0.0, length, N)[None, None, :]
+    gpath[..., 1] = y[:, :, None]
+    yaw = np.where(fwd, 0.0, math.pi)[None, :] + rng.uniform(-0.2, 0.2, (S, R))
+    pose = np.stack([np.broadcast_to(x0, (S, R)), y, yaw], axis=-1)
+    speed = np.stack([rng.uniform(0.0, 0.4, (S, R)), np.zeros((S, R))], axis=-1)
+    people, goal, vdes = _place_crowd(s, K, seed, pose[..., :2])
+    s.update(global_path=gpath.reshape(S * R, N, 2), pose=pose.reshape(S * R, 3), speed=speed.reshape(S * R, 2),
+             costmap_index=np.repeat(cidx, R).astype(np.int32), people=people,
+             n_people=np.full(S, K, dtype=np.int32), goals=goal, desired_speed=vdes, substeps=substeps,
+             robots_per_scene=R)
     return s
 
 
