@@ -459,6 +459,28 @@ typedef struct smpc_scene_io {
 int smpc_run_shared_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd,
                              const smpc_scene_io* scene);
 
+/* ---- per-robot critic weights: several controller tunings in one call -------------------------------------------------
+ * A table of P rows of the nine critic weights and a per-robot row index. Robot / episode b's critics use row
+ * set_index[b] instead of the handle's weights; everything else (tolerances, horizon, block length, trajectorizer,
+ * max_time / time_step, FOV, current_*_w) stays the handle's. A robot computes exactly what it computes on a handle whose
+ * params carry its row, so comparing tunings on the same scenes, or sweeping a weight, is one call.
+ * smpc_optimize_batch_weighted is smpc_optimize_batch with the table: the same fleet state and warm-start memory (a second
+ * way into the same tick). smpc_run_weighted_episodes is smpc_run_episodes (crowd == NULL, scene == NULL),
+ * smpc_run_crowd_episodes (scene == NULL) or smpc_run_shared_episodes (both given; a scene needs a crowd) with the table;
+ * set_index has one entry per robot, also in shared scenes, and the launches per tick are those of the unweighted entry.
+ * Returns what the unweighted entry returns, plus SMPC_ERR_ARGUMENT for w == NULL, n_sets < 1, a NULL array, an index
+ * outside 0..n_sets-1 or a weight that is not finite, and SMPC_ERR_UNSUPPORTED for omni_solve; all before anything is
+ * launched. */
+typedef struct smpc_weight_sets {
+  int n_sets;               /* P >= 1 */
+  const double* weights;    /* [P][9]: distance, socialwork, velocity, angle, agent_angle, proxemics,
+                               velocity_feasibility, obstacle, goal_align (smpc_params order) */
+  const int32_t* set_index; /* [B] in 0..P-1: the row robot / episode b uses */
+} smpc_weight_sets;
+int smpc_optimize_batch_weighted(smpc_handle* h, smpc_fleet_io* io, const smpc_weight_sets* w);
+int smpc_run_weighted_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd /* NULL: constant-velocity people */,
+                               const smpc_scene_io* scene /* NULL: one robot per scene */, const smpc_weight_sets* w);
+
 /* ---- batched pre-solve stage on the GPU: project_people (src/optimizer.cpp:554-671 + sfm.hpp) -----------------
  * One warp per problem, lanes over agents, sequential over the horizon. Generalised from the reference's 3 people to
  * A columns. Inputs (device pointers): robot [B][S+1][6] = the robot AgentTrajectory of format_to_optimize

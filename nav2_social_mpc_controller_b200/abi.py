@@ -422,3 +422,22 @@ class SmpcSceneIo(C.Structure):
         ("robot_min_dist", C.c_void_p),
         ("robot_intimate_ticks", C.c_void_p),
     ]
+
+
+class SmpcWeightSets(C.Structure):
+    """struct smpc_weight_sets — per-robot critic weights (smpc_optimize_batch_weighted, smpc_run_weighted_episodes)."""
+    _fields_ = [
+        ("n_sets", C.c_int),
+        ("weights", C.c_void_p),
+        ("set_index", C.c_void_p),
+    ]
+
+
+# the nine critic weights of a row of smpc_weight_sets.weights, in smpc_params order
+WEIGHT_NAMES = ("distance_w", "socialwork_w", "velocity_w", "angle_w", "agent_angle_w", "proxemics_w",
+                "velocity_feasibility_w", "obstacle_w", "goal_align_w")
+
+
+def weight_row(params) -> np.ndarray:
+    """The nine critic weights of a params struct (SmpcParams or OptimizerParams) as one row of a weight table."""
+    return np.array([float(getattr(params, k)) for k in WEIGHT_NAMES])

@@ -70,6 +70,10 @@ struct DevBatch {
   // scenario sharing: problem b reads row scenario[b] of the per-scene arrays (NULL: row b); n_rows = rows of those arrays
   const int32_t* scenario;
   int n_rows;
+  // per-problem critic weights (the weighted solve kernel only; NULL = DevParams' w_*): problem b uses row
+  // weight_set[b] of weights [P][9], in DevParams order w_distance .. w_goal
+  const double* weights;
+  const int32_t* weight_set;
 };
 
 struct DevResult {
@@ -359,7 +363,8 @@ constexpr int kRedStride = 33;  // odd stride of the per-warp reduction scratch:
 // D = parameters per block: 2 = (v, w), the reference's unicycle (update_state.hpp:46-61); 3 = (vx, vy, w), the
 // omnidirectional extension (holonomic Euler step x += (vx cos th - vy sin th) dt, consistent with the reference's
 // trajectorizer, path_trajectorizer.hpp:106-123; the reference has no omnidirectional SOLVE).
-template <int NB, int D = 2>
+// WT = the weighted solve kernel: the group's problem carries its own critic weights in a 9-double slot (kWt).
+template <int NB, int D = 2, bool WT = false>
 struct Layout {
   static constexpr int P = D * NB;
   static constexpr int NH = P * (P + 1) / 2;
@@ -378,7 +383,8 @@ struct Layout {
   static constexpr int kYaw = kCarry + NC;  // sin, cos of yaw0
   static constexpr int kState = kYaw + 2;    // LmState (solver scalars parked here across the evaluation)
   static constexpr int kProb = kState + 22;  // Prob (group-uniform problem view)
-  static constexpr int kAa = kProb + 18;  // agent-angle steering target per step [S]
+  static constexpr int kWt = kProb + 18;  // critic weights of the problem [9] (WT only)
+  static constexpr int kAa = kWt + (WT ? 9 : 0);  // agent-angle steering target per step [S]
   __host__ __device__ static constexpr int total(int S) { return ((kAa + S) | 1); }  // odd stride: no bank conflicts
   static constexpr int kRedDoubles = NE * kRedStride;  // per-WARP scratch behind the per-group regions
   __host__ __device__ static constexpr int g(int c) { return 2 + c; }
@@ -435,11 +441,13 @@ enum StateFlags {
 // its cost and directional derivative only (Ceres evaluates exactly cost + gradient there, line_search.cc), so its
 // J^T J is not built and kNoHessian is returned. st == nullptr: always build J^T J.
 // ---------------------------------------------------------------------------------------------------
-template <int NB, int G, bool PPL, int D = 2>
+// Critic weight k of DevParams' w_* order: the kernel parameter, or (WT) the problem's row in the group's workspace.
+#define SMPC_W(field, k) (WT ? ws[L::kWt + (k)] : prm.field)
+template <int NB, int G, bool PPL, int D = 2, bool WT = false>
 __device__ __forceinline__ unsigned evaluate(const DevParams& prm, const DevBatch& bt, const Prob& pb, bool live,
                                              double* ws, double* red, const double* xs, int lane, double* out,
                                              const LmState* st) {
-  using L = Layout<NB, D>;
+  using L = Layout<NB, D, WT>;
   constexpr int P = L::P;
   const int gl = lane & (G - 1);
   const unsigned gmask = Group<G>::mask(lane);
@@ -522,8 +530,8 @@ __device__ __forceinline__ unsigned evaluate(const DevParams& prm, const DevBatc
       const double tgt = aa[j];
       if (tgt == tgt) {
         const double del = wrap_angle(Th - tgt);
-        ra = prm.w_agent_angle * (del * del);
-        caT = 2.0 * prm.w_agent_angle * del;
+        ra = SMPC_W(w_agent_angle, 4) * (del * del);
+        caT = 2.0 * SMPC_W(w_agent_angle, 4) * del;
       }
       // --- SocialWork (k=1) and Proxemics (k=2) ----------------------------------------------------
       // robot velocity uses lv = v_{b(i)} and the NEW heading (omnidirectional: the body velocity rotated into the world)
@@ -534,7 +542,7 @@ __device__ __forceinline__ unsigned evaluate(const DevParams& prm, const DevBatc
       double wp = 0.0;
       double G4[4] = {0, 0, 0, 0};  // gradient of (wr + wp) wrt (dX, dY, dvx, dvy) of the robot
       double dmin = DBL_MAX, pdx = 0.0, pdy = 0.0;
-      const bool do_social = prm.w_social != 0.0;
+      const bool do_social = SMPC_W(w_social, 1) != 0.0;
       // agent records (x, y, vx, vy) of step j+1, one 32-byte sector each; the next agent's record is fetched
       // while the current pair interaction is evaluated
       const double2* rec = reinterpret_cast<const double2*>(pb.packed) + ((size_t)(j + 1)) * 2;
@@ -610,15 +618,15 @@ __device__ __forceinline__ unsigned evaluate(const DevParams& prm, const DevBatc
       if (do_social) {
         const double wr = Frx * Frx + Fry * Fry;
         SMPC_UNROLL for (int c = 0; c < 4; ++c) G4[c] = 2.0 * fma(Fry, JFy[c], fma(Frx, JFx[c], G4[c]));
-        rs = prm.w_social * (wr + wp + 1e-6);
-        sX = prm.w_social * G4[0];
-        sY = prm.w_social * G4[1];
-        sL = prm.w_social * (G4[2] * cT + G4[3] * sT);
+        rs = SMPC_W(w_social, 1) * (wr + wp + 1e-6);
+        sX = SMPC_W(w_social, 1) * G4[0];
+        sY = SMPC_W(w_social, 1) * G4[1];
+        sL = SMPC_W(w_social, 1) * (G4[2] * cT + G4[3] * sT);
         if (D == 3) {
-          sM = prm.w_social * (-G4[2] * sT + G4[3] * cT);
-          sTh = prm.w_social * (-G4[2] * rvy + G4[3] * rvx);
+          sM = SMPC_W(w_social, 1) * (-G4[2] * sT + G4[3] * cT);
+          sTh = SMPC_W(w_social, 1) * (-G4[2] * rvy + G4[3] * rvx);
         } else {
-          sTh = prm.w_social * vj * (-G4[2] * sT + G4[3] * cT);
+          sTh = SMPC_W(w_social, 1) * vj * (-G4[2] * sT + G4[3] * cT);
         }
       }
       // Proxemics: w * 3 * exp(-dmin / 0.25), proxemics_cost_function.hpp:128-149.
@@ -627,10 +635,10 @@ __device__ __forceinline__ unsigned evaluate(const DevParams& prm, const DevBatc
       //  * Ceres 2.0.0 (ceres_compat < 210) has no numeric_limits specialisation for Jets: the primary template returns
       //    Jet() = 0, std::min keeps it, and every DIFFERENTIATED evaluation sees the constant residual 3 w with a zero
       //    Jacobian row, while cost-only evaluations (candidate cost) see the true minimum distance.
-      const double r_true = (dmin == DBL_MAX) ? 0.0 : prm.w_prox * (3.0 * exp(-dmin / (0.5 * 0.5)));
+      const double r_true = (dmin == DBL_MAX) ? 0.0 : SMPC_W(w_prox, 5) * (3.0 * exp(-dmin / (0.5 * 0.5)));
       cprox_plain = 0.5 * r_true * r_true;
       if (prm.ceres_compat < 210) {
-        rp = prm.w_prox * 3.0;
+        rp = SMPC_W(w_prox, 5) * 3.0;
       } else if (dmin == DBL_MAX) {
         flags |= kJacobianBad;
       } else {
@@ -718,14 +726,14 @@ __device__ __forceinline__ unsigned evaluate(const DevParams& prm, const DevBatc
       if (j < ch) {
         const double e = 0.6 - vj;
         if (D == 3) {  // omnidirectional extension: w ((0.6 - vx)^2 + vy^2)
-          const double r = prm.w_velocity * e * e + prm.w_velocity * vyj * vyj;
-          const double cL = -2.0 * prm.w_velocity * e, cM = 2.0 * prm.w_velocity * vyj;
+          const double r = SMPC_W(w_velocity, 2) * e * e + SMPC_W(w_velocity, 2) * vyj * vyj;
+          const double cL = -2.0 * SMPC_W(w_velocity, 2) * e, cM = 2.0 * SMPC_W(w_velocity, 2) * vyj;
           cost += 0.5 * r * r;
           mLL += cL * cL; mLM += cL * cM; mMM += cM * cM;
           qL += cL * r; qM += cM * r;
         } else {
-          const double r = prm.w_velocity * e * e;
-          const double cL = -2.0 * prm.w_velocity * e;
+          const double r = SMPC_W(w_velocity, 2) * e * e;
+          const double cL = -2.0 * SMPC_W(w_velocity, 2) * e;
           cost += 0.5 * r * r;
           mLL += cL * cL;
           qL += cL * r;
@@ -734,8 +742,8 @@ __device__ __forceinline__ unsigned evaluate(const DevParams& prm, const DevBatc
       // --- GoalAlign (k=4): w * wrap(psi - Theta)^2 -----------------------------------------------------
       {
         const double turn = wrap_angle(pb.goal_yaw - Th);
-        const double r = prm.w_goal * turn * turn;
-        const double cTh = -2.0 * prm.w_goal * turn;
+        const double r = SMPC_W(w_goal, 8) * turn * turn;
+        const double cTh = -2.0 * SMPC_W(w_goal, 8) * turn;
         cost += 0.5 * r * r;
         mTT += cTh * cTh;
         qT += cTh * r;
@@ -744,8 +752,8 @@ __device__ __forceinline__ unsigned evaluate(const DevParams& prm, const DevBatc
       {
         const double ex = X - pb.fin_x, ey = Y - pb.fin_y;
         const double q2 = ex * ex + ey * ey;
-        const double r = prm.w_distance * q2 * q2;
-        const double k = 4.0 * prm.w_distance * q2;
+        const double r = SMPC_W(w_distance, 0) * q2 * q2;
+        const double k = 4.0 * SMPC_W(w_distance, 0) * q2;
         const double cX = k * ex, cY = k * ey;
         cost += 0.5 * r * r;
         mXX += cX * cX; mXY += cX * cY; mYY += cY * cY;
@@ -754,8 +762,8 @@ __device__ __forceinline__ unsigned evaluate(const DevParams& prm, const DevBatc
       {
         const double ex = X - ld_in<PPL>(pb.px + j + 1), ey = Y - ld_in<PPL>(pb.px + stride + j + 1);
         const double q2 = ex * ex + ey * ey;
-        const double r = prm.w_angle * q2 * q2;
-        const double k = 4.0 * prm.w_angle * q2;
+        const double r = SMPC_W(w_angle, 3) * q2 * q2;
+        const double k = 4.0 * SMPC_W(w_angle, 3) * q2;
         const double cX = k * ex, cY = k * ey;
         cost += 0.5 * r * r;
         mXX += cX * cX; mXY += cX * cY; mYY += cY * cY;
@@ -767,8 +775,8 @@ __device__ __forceinline__ unsigned evaluate(const DevParams& prm, const DevBatc
         const double gx = (fxw - pb.org_x) * inv_res, gy = (fyw - pb.org_y) * inv_res;
         double f, dfdr, dfdc;
         bicubic<PPL>(pb.map, bt.size_x, bt.size_y, gy, gx, f, dfdr, dfdc);
-        const double r = prm.w_obstacle * f;
-        const double kx = prm.w_obstacle * dfdc * inv_res, ky = prm.w_obstacle * dfdr * inv_res;
+        const double r = SMPC_W(w_obstacle, 7) * f;
+        const double kx = SMPC_W(w_obstacle, 7) * dfdc * inv_res, ky = SMPC_W(w_obstacle, 7) * dfdr * inv_res;
         const double cTh = 0.25 * (-kx * sT + ky * cT);
         cost += 0.5 * r * r;
         mXX += kx * kx; mXY += kx * ky; mXT += kx * cTh;
@@ -809,12 +817,12 @@ __device__ __forceinline__ unsigned evaluate(const DevParams& prm, const DevBatc
             double dk[D], r = 0.0;
             SMPC_UNROLL for (int k = 0; k < D; ++k) {
               dk[k] = xs[D * i + k] - xs[D * (i - 1) + k];
-              r += prm.w_vf * dk[k] * dk[k];
+              r += SMPC_W(w_vf, 6) * dk[k] * dk[k];
             }
             red[0 * kRedStride + lane] += 0.5 * r * r;
             red[1 * kRedStride + lane] += 0.5 * r * r;
             SMPC_UNROLL for (int k = 0; k < D; ++k) {
-              const double jk = 2.0 * prm.w_vf * dk[k];
+              const double jk = 2.0 * SMPC_W(w_vf, 6) * dk[k];
               red[L::g(D * (i - 1) + k) * kRedStride + lane] -= jk * r;
               red[L::g(D * i + k) * kRedStride + lane] += jk * r;
             }
@@ -884,7 +892,7 @@ __device__ __forceinline__ unsigned evaluate(const DevParams& prm, const DevBatc
       SMPC_UNROLL for (int i = 1; i < NB; ++i) {
         if (i < pb.nbd) {
           double jk[D];
-          SMPC_UNROLL for (int k = 0; k < D; ++k) jk[k] = 2.0 * prm.w_vf * (xs[D * i + k] - xs[D * (i - 1) + k]);
+          SMPC_UNROLL for (int k = 0; k < D; ++k) jk[k] = 2.0 * SMPC_W(w_vf, 6) * (xs[D * i + k] - xs[D * (i - 1) + k]);
           SMPC_UNROLL for (int k = 0; k < D; ++k) {
             SMPC_UNROLL for (int l = 0; l < D; ++l) {
               const double v = jk[k] * jk[l];
@@ -921,6 +929,7 @@ __device__ __forceinline__ unsigned evaluate(const DevParams& prm, const DevBatc
   __syncwarp();
   return flags;
 }
+#undef SMPC_W
 
 // ---------------------------------------------------------------------------------------------------
 // Interpolating-polynomial minimiser of the Armijo line search (ceres polynomial.cc, SURVEY Appendix A).
@@ -1286,9 +1295,9 @@ __device__ __forceinline__ void load_problem(const DevParams& prm, const DevBatc
 }
 
 // Agent-angle steering targets of every step -> group shared memory (once per problem).
-template <int NB, int G, bool PPL, int D = 2>
+template <int NB, int G, bool PPL, int D = 2, bool WT = false>
 __device__ __forceinline__ void agent_angle_setup(const DevBatch& bt, const Prob& pb, int lane, double* ws) {
-  using L = Layout<NB, D>;
+  using L = Layout<NB, D, WT>;
   const int gl = lane & (G - 1);
   if (gl == 0) {
     double s0, c0;
@@ -1404,10 +1413,10 @@ __device__ __forceinline__ void trace_row(const DevResult& rs, int b, int row, d
   o[4] = cost_plain; o[5] = aux; o[6] = code; o[7] = radius;
 }
 
-template <int NB, int G, bool PPL, int D = 2>
+template <int NB, int G, bool PPL, int D = 2, bool WT = false>
 __device__ __forceinline__ void solve_loop(const DevParams& prm, const DevBatch& bt, const DevResult& rs, int* queue,
                                            double* ws, double* red, int lane) {
-  using L = Layout<NB, D>;
+  using L = Layout<NB, D, WT>;
   constexpr int P = L::P;
   const int gl = lane & (G - 1);
   const unsigned gmask = Group<G>::mask(lane);
@@ -1484,9 +1493,13 @@ __device__ __forceinline__ void solve_loop(const DevParams& prm, const DevBatch&
         if (gl == 0) {
           if (!PPL && bt.arrival != nullptr) wait_for_costmap(bt.arrival, nb_);
           load_problem<PPL>(prm, bt, nb_, *pbs);
+          if (WT) {  // the problem's critic weights: row weight_set[b] of the batch's table
+            const double* row = bt.weights + 9 * (size_t)ld_in<PPL>(bt.weight_set + nb_);
+            SMPC_UNROLL for (int k = 0; k < 9; ++k) ws[L::kWt + k] = ld_in<PPL>(row + k);
+          }
         }
         __syncwarp(gmask);
-        agent_angle_setup<NB, G, PPL, D>(bt, *pbs, lane, ws);
+        agent_angle_setup<NB, G, PPL, D, WT>(bt, *pbs, lane, ws);
         if (gl == 0) {
           // IterationZero: project the start point onto the box. Blocks the problem does not use (shorter horizon than
           // the batch's) stay exactly zero: no residual touches them, so their rows of J^T J and J^T r are zero, the LM
@@ -1535,7 +1548,7 @@ __device__ __forceinline__ void solve_loop(const DevParams& prm, const DevBatch&
     }
 
     const bool live = (gs->flags & kLive) != 0;
-    const unsigned fl = evaluate<NB, G, PPL, D>(prm, bt, *pbs, live, ws, red, cand, lane,
+    const unsigned fl = evaluate<NB, G, PPL, D, WT>(prm, bt, *pbs, live, ws, red, cand, lane,
                                              ws + ((gs->flags & kSwapped) ? L::kBuf0 : L::kBuf1), gs);
 
     // ---- phase logic: the group's first lane alone, on the group's shared-memory state -----------------------

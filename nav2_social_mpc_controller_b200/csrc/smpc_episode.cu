@@ -285,8 +285,9 @@ __global__ void smpc_robot_metrics_kernel(RobotMetrics a) {
 
 // The loop of all entries; crowd == NULL: constant-velocity people (smpc_run_episodes); scene == NULL: one robot per
 // scene (smpc_run_episodes, smpc_run_crowd_episodes).
+// w != NULL: per-episode critic weights (smpc_run_weighted_episodes).
 int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd, const smpc_scene_io* scene,
-                 const char* name) {
+                 const char* name, const smpc_weight_sets* w = nullptr) {
   auto fail_arg = [name](const char* msg) {
     return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string(name) + ": " + msg);
   };
@@ -321,6 +322,10 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
   if (R < 1 || R > kMaxRobotsPerScene) return fail_arg("robots_per_scene outside 1..8");
   if (B % R != 0) return fail_arg("n_episodes not a multiple of robots_per_scene");
   if (scene && (!scene->robot_min_dist || !scene->robot_intimate_ticks)) return fail_arg("missing output");
+  if (w) {
+    const int rc = smpc_check_weight_sets(w, B, name);
+    if (rc != SMPC_OK) return rc;
+  }
   const int S = B / R;  // scenes: people, n_people_each, goals, desired_speed and people_log have S rows
   for (int c = 0; c < S && K > 0; ++c)
     if (io->n_people_each[c] < 0 || io->n_people_each[c] > K) return fail_arg("n_people_each[b] outside 0..K");
@@ -391,6 +396,8 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
   double *map_org, *od_org, *fov_people, *speed;
   uint32_t* od;
   int* n_active;
+  double* weights = nullptr;
+  int32_t* weight_set = nullptr;
   auto carve = [&](smpc_carve& c) {
     maps = c.take<uint8_t>(map_bytes);
     od = c.take<uint32_t>(od_bytes / 4);
@@ -435,6 +442,10 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       disturbance = c.take<double>(Bz);
       people_log = c.take<double>(logs_people ? Sz * (T + 1) * Kz * 5 : 0);
     }
+    if (w) {
+      weights = c.take<double>((size_t)w->n_sets * 9);
+      weight_set = c.take<int32_t>(Bz);
+    }
     if (scene) {
       view = c.take<double>(Bz * n_view * 5);
       view_n = c.take<int32_t>(Bz);
@@ -460,6 +471,7 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       {map_index, io->costmap_index, Bz * 4}, {od_index, io->od_index, Bz * 4},
       {gp, io->global_path, Bz * N * 16}, {pose, io->pose, Bz * 24}, {speed, io->speed, Bz * 16},
       {people0, K > 0 ? io->people : nullptr, Sz * Kz * 40}, {n_people_dev, K > 0 ? io->n_people_each : nullptr, Sz * 4},
+      {weights, w ? w->weights : nullptr, w ? (size_t)w->n_sets * 72 : 0}, {weight_set, w ? w->set_index : nullptr, Bz * 4},
   };
   for (const Up& u : ups)
     if (u.host && u.bytes) SMPC_FLEET_CUDA(cudaMemcpyAsync(u.dev, u.host, u.bytes, cudaMemcpyHostToDevice, st));
@@ -485,6 +497,7 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
   d.n_od_grids = io->n_od_grids; d.od_width = io->od_width; d.od_height = io->od_height;
   d.od_resolution = io->od_resolution; d.od = od; d.od_org = od_org; d.od_index = io->od_index ? od_index : nullptr;
   d.people = fov_people; d.n_people = fov_n; d.speed = speed;
+  d.weights = weights; d.weight_set = weight_set;
 
   smpc_trajectorize_args ta{};
   ta.n_problems = B; ta.n_path = N; ta.max_steps = max_steps; ta.omnidirectional = 0;
@@ -627,4 +640,12 @@ extern "C" int smpc_run_shared_episodes(smpc_handle* h, smpc_episode_io* io, con
   if (!crowd) return smpc_host_fail(SMPC_ERR_ARGUMENT, "run_shared_episodes: NULL crowd");
   if (!scene) return smpc_host_fail(SMPC_ERR_ARGUMENT, "run_shared_episodes: NULL scene");
   return run_episodes(h, io, crowd, scene, "run_shared_episodes");
+}
+
+extern "C" int smpc_run_weighted_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd,
+                                          const smpc_scene_io* scene, const smpc_weight_sets* w) {
+  const int rc = smpc_check_weight_sets(w, 0, "run_weighted_episodes");  // the indices: once B is known
+  if (rc != SMPC_OK) return rc;
+  if (scene && !crowd) return smpc_host_fail(SMPC_ERR_ARGUMENT, "run_weighted_episodes: a shared scene needs a crowd");
+  return run_episodes(h, io, crowd, scene, "run_weighted_episodes", w);
 }

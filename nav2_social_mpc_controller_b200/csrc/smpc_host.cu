@@ -225,6 +225,8 @@ void to_dev_batch(const smpc_batch& in, smpc::DevBatch* d) {
   d->cta_sync = 1;
   d->scenario = in.scenario_index;
   d->n_rows = in.scenario_index ? in.n_scenarios : in.n_problems;
+  d->weights = nullptr;
+  d->weight_set = nullptr;
 }
 
 // Build the packed agent records of a batch in the handle's scratch buffer (one small kernel per batch).
@@ -541,14 +543,18 @@ void smpc_destroy(smpc_handle* h) {
 
 // One solve launch of `in` (device pointers) on `stream`. `queue` = this launch's work-queue counter; the packed agent
 // records go to slice [first, first + B) of a scratch buffer sized for `total_problems`.
+// weights / weight_set (device, NULL = the handle's weights): per-problem critic weights, see smpc_solve_batch_weighted.
 static int launch_solve_on(smpc_handle* h, const smpc_batch* in, smpc_result* out, int* queue, size_t total_problems,
-                           size_t first, bool timed, cudaStream_t stream, unsigned* arrival = nullptr) {
+                           size_t first, bool timed, cudaStream_t stream, unsigned* arrival = nullptr,
+                           const double* weights = nullptr, const int32_t* weight_set = nullptr) {
   smpc::DevParams prm;
   int rc = make_dev_params(h->params, in->n_steps, &prm);
   if (rc != SMPC_OK) return rc;
   smpc::DevBatch bt;
   to_dev_batch(*in, &bt);
   bt.arrival = arrival;
+  bt.weights = weights;
+  bt.weight_set = weight_set;
   bt.cta_sync = (h->cta_sync < 0) ? 1 : h->cta_sync;
   smpc::DevResult rs;
   to_dev_result(*out, &rs);
@@ -580,13 +586,15 @@ static int launch_solve_on(smpc_handle* h, const smpc_batch* in, smpc_result* ou
   return SMPC_OK;
 }
 
-static int solve_device_locked(smpc_handle* h, const smpc_batch* in, smpc_result* out, cudaStream_t stream) {
+static int solve_device_locked(smpc_handle* h, const smpc_batch* in, smpc_result* out, cudaStream_t stream,
+                               const double* weights = nullptr, const int32_t* weight_set = nullptr) {
   int rc = check_batch(in);
   if (rc != SMPC_OK) return rc;
   if (!out) return fail(SMPC_ERR_ARGUMENT, "result is NULL");
   if (in->n_problems == 0) return SMPC_OK;
   SMPC_CUDA(cudaSetDevice(h->device));
-  return launch_solve_on(h, in, out, h->queue, static_cast<size_t>(in->n_problems), 0, true, stream);
+  return launch_solve_on(h, in, out, h->queue, static_cast<size_t>(in->n_problems), 0, true, stream, nullptr, weights,
+                         weight_set);
 }
 
 int smpc_solve_batch_device(smpc_handle* h, const smpc_batch* in, smpc_result* out, void* stream) {
@@ -594,6 +602,17 @@ int smpc_solve_batch_device(smpc_handle* h, const smpc_batch* in, smpc_result* o
   std::lock_guard<std::mutex> lk(h->mu);
   return solve_device_locked(h, in, out, stream ? static_cast<cudaStream_t>(stream) : h->stream);
 }
+
+}  // extern "C"
+
+int smpc_solve_batch_weighted(smpc_handle* h, const smpc_batch* in, smpc_result* out, const double* weights,
+                              const int32_t* weight_set, cudaStream_t stream) {
+  if (!h) return fail(SMPC_ERR_ARGUMENT, "handle is NULL");
+  std::lock_guard<std::mutex> lk(h->mu);
+  return solve_device_locked(h, in, out, stream, weights, weight_set);
+}
+
+extern "C" {
 
 // Chunk plan of the host-buffer pipeline (pure: no CUDA call, exported for the CPU test suite as
 // smpc_debug_plan_chunks). Chunking pays where the copies are a large share of the call: batches with people (28 kB

@@ -126,6 +126,9 @@ struct smpc_fleet_dev {
   double *init, *robot, *pose0, *u0, *path_xy, *goal_yaw, *agents, *cmds_new, *path_new, *cost0, *cost1;
   uint8_t *has_people, *usable, *optimized;
   int32_t *term, *iters, *n_out, *status;
+  // per-robot critic weights (NULL = the handle's): robot b's critics use row weight_set[b] of weights [P][9]
+  const double* weights;
+  const int32_t* weight_set;
 };
 
 // Carves the stage buffers and outputs of smpc_fleet_dev (init .. path_new, then usable .. status) from c.
@@ -171,8 +174,16 @@ smpc_memory* smpc_handle_memory(smpc_handle* h);
 int smpc_host_fail(int code, const std::string& msg);
 cudaStream_t smpc_handle_stream(smpc_handle* h);
 void smpc_handle_count_launch(smpc_handle* h);
-// the fleet tick on an explicit state (smpc_optimize_batch uses the handle's fleet state, smpc_optimize its own)
-int smpc_optimize_batch_on(smpc_handle* h, smpc_fleet_state* fs, smpc_fleet_io* io);
+// the fleet tick on an explicit state (smpc_optimize_batch uses the handle's fleet state, smpc_optimize its own);
+// w != NULL: per-robot critic weights (smpc_optimize_batch_weighted)
+int smpc_optimize_batch_on(smpc_handle* h, smpc_fleet_state* fs, smpc_fleet_io* io, const smpc_weight_sets* w = nullptr);
+// SMPC_ERR_ARGUMENT unless w is a valid weight table for n robots: n_sets >= 1, arrays given, every weight finite, every
+// index in 0..n_sets-1 (`name` prefixes the message)
+int smpc_check_weight_sets(const smpc_weight_sets* w, int n, const char* name);
+// smpc_solve_batch_device with per-problem critic weights (device pointers weights [P][9], weight_set [B]): the solve
+// of the fleet tick (people columns, unicycle blocks only)
+int smpc_solve_batch_weighted(smpc_handle* h, const smpc_batch* in, smpc_result* out, const double* weights,
+                              const int32_t* weight_set, cudaStream_t stream);
 
 #define SMPC_FLEET_CUDA(call)                                                                              \
   do {                                                                                                     \

@@ -810,7 +810,8 @@ int smpc_fleet_tick_enqueue(smpc_handle* h, const smpc_fleet_dev& d, cudaStream_
   smpc_result rs{};
   rs.cmds = d.cmds_new; rs.path = d.path_new; rs.usable = d.usable; rs.termination = d.term; rs.iterations = d.iters;
   rs.cost_initial = d.cost0; rs.cost_final = d.cost1;
-  const int rc = smpc_solve_batch_device(h, &bt, &rs, st);
+  const int rc = d.weights ? smpc_solve_batch_weighted(h, &bt, &rs, d.weights, d.weight_set, st)
+                           : smpc_solve_batch_device(h, &bt, &rs, st);
   if (rc != SMPC_OK) return rc;
 
   // ---- post-solve: outputs, memory update
@@ -822,7 +823,20 @@ int smpc_fleet_tick_enqueue(smpc_handle* h, const smpc_fleet_dev& d, cudaStream_
   return SMPC_OK;
 }
 
-int smpc_optimize_batch_on(smpc_handle* h, smpc_fleet_state* fs, smpc_fleet_io* io) {
+int smpc_check_weight_sets(const smpc_weight_sets* w, int n, const char* name) {
+  const std::string pre = std::string(name) + ": ";
+  if (!w) return smpc_host_fail(SMPC_ERR_ARGUMENT, pre + "NULL weight sets");
+  if (w->n_sets < 1) return smpc_host_fail(SMPC_ERR_ARGUMENT, pre + "n_sets < 1");
+  if (!w->weights || !w->set_index) return smpc_host_fail(SMPC_ERR_ARGUMENT, pre + "weights / set_index missing");
+  for (size_t i = 0; i < (size_t)w->n_sets * 9; ++i)
+    if (!std::isfinite(w->weights[i])) return smpc_host_fail(SMPC_ERR_ARGUMENT, pre + "a weight is not finite");
+  for (int b = 0; b < n; ++b)
+    if (w->set_index[b] < 0 || w->set_index[b] >= w->n_sets)
+      return smpc_host_fail(SMPC_ERR_ARGUMENT, pre + "set_index[b] outside 0..n_sets-1");
+  return SMPC_OK;
+}
+
+int smpc_optimize_batch_on(smpc_handle* h, smpc_fleet_state* fs, smpc_fleet_io* io, const smpc_weight_sets* w) {
   if (!h || !io || !fs) return smpc_host_fail(SMPC_ERR_ARGUMENT, "NULL argument");
   const int B = io->n_robots, stride = io->max_poses, A = io->n_agents;
   if (B < 0 || stride < 2 || A < 1 || A > kMaxAgents - 1)
@@ -836,6 +850,10 @@ int smpc_optimize_batch_on(smpc_handle* h, smpc_fleet_state* fs, smpc_fleet_io* 
   if (io->od_width == 0 || io->od_height == 0) return smpc_host_fail(SMPC_ERR_ARGUMENT, "ObstacleDistance grid has invalid size");
   if (!(io->od_resolution > 0.0f)) return smpc_host_fail(SMPC_ERR_ARGUMENT, "ObstacleDistance grid has invalid resolution");
   if (!io->n_out || !io->optimized) return smpc_host_fail(SMPC_ERR_ARGUMENT, "optimize_batch: n_out / optimized missing");
+  if (w) {
+    const int rc = smpc_check_weight_sets(w, B, "optimize_batch_weighted");
+    if (rc != SMPC_OK) return rc;
+  }
   const smpc_params* prm = smpc_handle_params(h);
   if (prm->omni_solve)  // the reference's Optimizer::optimize is unicycle-only (update_state.hpp:46-61)
     return smpc_host_fail(SMPC_ERR_UNSUPPORTED, "the level-2 entries mirror Optimizer::optimize, which has no omnidirectional solve");
@@ -926,6 +944,8 @@ int smpc_optimize_batch_on(smpc_handle* h, smpc_fleet_state* fs, smpc_fleet_io* 
     d.s_each = c.take<int32_t>(B);
     d.map_index = c.take<int32_t>(B);
     d.od_index = c.take<int32_t>(B);
+    d.weights = c.take<double>(w ? (size_t)w->n_sets * 9 : 0);  // unweighted: no bytes, the layout is unchanged
+    d.weight_set = c.take<int32_t>(w ? B : 0);
     smpc_fleet_carve_stages(c, &d);
   };
   size_t need = 0;
@@ -958,6 +978,8 @@ int smpc_optimize_batch_on(smpc_handle* h, smpc_fleet_state* fs, smpc_fleet_io* 
       {d.speed, io->speed, (size_t)B * 16},      {d.n_in, io->n_poses, (size_t)B * 4},
       {d.n_each, n_each.data(), (size_t)B * 4},  {d.s_each, s_each.data(), (size_t)B * 4},
       {d_map_index, io->costmap_index, (size_t)B * 4}, {d_od_index, io->od_index, (size_t)B * 4},
+      {d.weights, w ? w->weights : nullptr, w ? (size_t)w->n_sets * 72 : 0},
+      {d.weight_set, w ? w->set_index : nullptr, (size_t)B * 4},
   };
   if (packed) {
     FLEET_CUDA(fs->pin_in.reserve(in_span));
@@ -971,6 +993,10 @@ int smpc_optimize_batch_on(smpc_handle* h, smpc_fleet_state* fs, smpc_fleet_io* 
   }
   if (!io->costmap_index) d.map_index = nullptr;
   if (!io->od_index) d.od_index = nullptr;
+  if (!w) {
+    d.weights = nullptr;
+    d.weight_set = nullptr;
+  }
 
   rc = smpc_fleet_tick_enqueue(h, d, st);
   if (rc != SMPC_OK) return rc;
@@ -1010,6 +1036,13 @@ extern "C" {
 int smpc_optimize_batch(smpc_handle* h, smpc_fleet_io* io) {
   if (!h) return smpc_host_fail(SMPC_ERR_ARGUMENT, "handle is NULL");
   return smpc_optimize_batch_on(h, smpc_handle_fleet(h), io);
+}
+
+int smpc_optimize_batch_weighted(smpc_handle* h, smpc_fleet_io* io, const smpc_weight_sets* w) {
+  if (!h) return smpc_host_fail(SMPC_ERR_ARGUMENT, "handle is NULL");
+  const int rc = smpc_check_weight_sets(w, 0, "optimize_batch_weighted");  // the indices: once B is known
+  if (rc != SMPC_OK) return rc;
+  return smpc_optimize_batch_on(h, smpc_handle_fleet(h), io, w);
 }
 
 }  // extern "C"

@@ -14,6 +14,22 @@ from . import _lib, abi
 from .optimizer import Optimizer
 
 
+def weight_sets_arg(weights, n_robots: int):
+    """The smpc_weight_sets of the `weights=(table [P][9], set_index [B])` keyword, with the arrays it points to (keep
+    them alive for the call). Raises ValueError on a shape or an index the table does not have."""
+    table, set_index = weights
+    table = np.ascontiguousarray(table, dtype=np.float64)
+    set_index = np.asarray(set_index)
+    if table.ndim != 2 or table.shape[1] != len(abi.WEIGHT_NAMES) or table.shape[0] < 1:
+        raise ValueError(f"weights table must be [P][{len(abi.WEIGHT_NAMES)}] with P >= 1, got {table.shape}")
+    if set_index.shape != (n_robots,) or not np.issubdtype(set_index.dtype, np.integer):
+        raise ValueError(f"set_index must be {n_robots} integers, got {set_index.dtype} {set_index.shape}")
+    if n_robots and (set_index.min() < 0 or set_index.max() >= table.shape[0]):
+        raise ValueError(f"set_index outside 0..{table.shape[0] - 1}")
+    set_index = np.ascontiguousarray(set_index, dtype=np.int32)
+    return abi.SmpcWeightSets(table.shape[0], table.ctypes.data, set_index.ctypes.data), (table, set_index)
+
+
 class FleetOptimizer:
     def __init__(self, params, n_robots: int, n_agents: int = 3, device: int = 0):
         self.device = device
@@ -95,7 +111,7 @@ class FleetOptimizer:
 
     def optimize_batch(self, poses, cmds, people_raw, n_people, speed, costmaps, costmap_origin, costmap_resolution,
                        od: dict, costmap_index=None, od_index=None, n_poses=None, want_people_proj=True,
-                       inplace=False) -> dict:
+                       inplace=False, weights=None) -> dict:
         """One controller tick for the fleet (smpc_optimize_batch). poses [B][n][3], cmds [B][>= n-1][2] (trajectorizer
         seeds; n_poses [B] = valid poses per robot, default n for all), people_raw [B][A][5], n_people [B], speed [B][2],
         costmaps [M][sy][sx] u8, od = dict(width, height, resolution, origins [Mo][2], indexes u32 [Mo][h*w]).
@@ -103,7 +119,9 @@ class FleetOptimizer:
         up to n_out[b]), people_proj [B][A][6][n], termination, iterations, cost_initial, cost_final, project_status.
         Costmaps / obstacle grids are re-sent to the GPU only when the arrays passed here change identity.
         inplace = True: poses [B][n][3] and cmds [B][n][2] (C-contiguous float64) are the in/out buffers of the C call
-        themselves, like the reference's in-out path / cmds arguments — no copies on the Python side."""
+        themselves, like the reference's in-out path / cmds arguments — no copies on the Python side.
+        weights = (table [P][9], set_index [B]): robot b's critics use row set_index[b] (abi.WEIGHT_NAMES columns;
+        optimizer.weight_sets builds the table) instead of the handle's weights (smpc_optimize_batch_weighted)."""
         p = self.p
         poses = np.ascontiguousarray(poses, dtype=np.float64)
         B, n, _ = poses.shape
@@ -154,7 +172,11 @@ class FleetOptimizer:
         for k2, v in out.items():
             setattr(io, k2, v.ctypes.data)
         io.people_proj = None if proj is None else proj.ctypes.data
-        _lib.check(_lib.lib().smpc_optimize_batch(self.opt._h, C.byref(io)))
+        if weights is None:
+            _lib.check(_lib.lib().smpc_optimize_batch(self.opt._h, C.byref(io)))
+        else:
+            ws, keep = weight_sets_arg(weights, B)
+            _lib.check(_lib.lib().smpc_optimize_batch_weighted(self.opt._h, C.byref(io), C.byref(ws)))
         res = dict(out)
         res["optimized"] = out["optimized"].astype(bool)
         res["path"], res["cmds"], res["people_proj"] = pose_rows, cmd_rows, proj
@@ -166,18 +188,24 @@ class FleetOptimizer:
 
     def run_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
                      od: dict, ticks: int, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                     want_logs=False) -> dict:
+                     want_logs=False, weights=None) -> dict:
         """Closed-loop episodes on the GPU (smpc_run_episodes): each of the B robots runs its crowd scene for up to
         `ticks` controller ticks — trajectorizer seed, constant-velocity people, FOV filter, the fleet tick, a unicycle
         world step — with one upload and one download for the whole run. global_path [B][N][2], pose [B][3],
         speed [B][2], people [B][K][5] at t = 0 (x, y, vx, vy, vz), n_people [B] <= K, maps as in optimize_batch.
         Returns host numpy per episode: reached (bool), ticks, path_length, min_person_dist (inf without people),
         intimate_ticks, personal_ticks, collision_ticks, not_optimized_ticks, cmd_variation; with want_logs also
-        pose_log [B][T+1][3], cmd_log [B][T][2], optimized_log [B][T] (bool)."""
+        pose_log [B][T+1][3], cmd_log [B][T][2], optimized_log [B][T] (bool).
+        weights = (table [P][9], set_index [B]) as in optimize_batch: episode b runs with row set_index[b]
+        (smpc_run_weighted_episodes)."""
         io, out, logs, keep = self.episode_io(global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                                               costmap_resolution, od, ticks, control_period, goal_tolerance,
                                               costmap_index, od_index, want_logs)
-        _lib.check(_lib.lib().smpc_run_episodes(self.opt._h, C.byref(io)))
+        if weights is None:
+            _lib.check(_lib.lib().smpc_run_episodes(self.opt._h, C.byref(io)))
+        else:
+            ws, wkeep = weight_sets_arg(weights, self.B)
+            _lib.check(_lib.lib().smpc_run_weighted_episodes(self.opt._h, C.byref(io), None, None, C.byref(ws)))
         res = dict(out, **logs)
         res["reached"] = out["reached"].astype(bool)
         if want_logs:
@@ -187,34 +215,35 @@ class FleetOptimizer:
     def run_crowd_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                            costmap_resolution, od: dict, ticks: int, goals, desired_speed, substeps=1,
                            control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                           want_logs=False) -> dict:
+                           want_logs=False, weights=None) -> dict:
         """Closed-loop episodes with a reactive crowd (smpc_run_crowd_episodes): run_episodes, but the people walk to
         their goals [B][K][2] at their desired speeds [B][K] under the lightsfm social force model, `substeps` updates
         per control period, and give way to the robot; people [B][K][5] is their state at t = 0. Returns the dict of
         run_episodes plus people_disturbance [B] (sum of |F(robot -> person)| * dt_s over ticks, substeps and people);
-        with want_logs also people_log [B][T+1][K][5] (x, y, vx, vy, vz at every tick, row 0 = the input)."""
+        with want_logs also people_log [B][T+1][K][5] (x, y, vx, vy, vz at every tick, row 0 = the input).
+        weights: as in run_episodes."""
         return self._crowd_run(None, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                                costmap_resolution, od, ticks, goals, desired_speed, substeps, control_period,
-                               goal_tolerance, costmap_index, od_index, want_logs)
+                               goal_tolerance, costmap_index, od_index, want_logs, weights)
 
     def run_shared_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                             costmap_resolution, od: dict, ticks: int, goals, desired_speed, robots_per_scene,
                             substeps=1, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                            want_logs=False) -> dict:
+                            want_logs=False, weights=None) -> dict:
         """Closed-loop episodes in shared scenes (smpc_run_shared_episodes): run_crowd_episodes with the B robots
         grouped into S = B / R scenes of R = robots_per_scene consecutive robots that share one crowd, costmap and
         obstacle grid, and that see each other as people. Per robot: global_path [B][N][2], pose [B][3],
         speed [B][2], costmap_index / od_index [B] (equal within a scene). Per scene: people [S][K][5],
         n_people [S], goals [S][K][2], desired_speed [S][K]. Returns the dict of run_crowd_episodes plus
         robot_min_dist [B] (nearest other robot of the scene, inf for R = 1) and robot_intimate_ticks [B]; with
-        want_logs people_log is per scene, [S][T+1][K][5]."""
+        want_logs people_log is per scene, [S][T+1][K][5]. weights: as in run_episodes, set_index per robot."""
         return self._crowd_run(int(robots_per_scene), global_path, pose, speed, people, n_people, costmaps,
                                costmap_origin, costmap_resolution, od, ticks, goals, desired_speed, substeps,
-                               control_period, goal_tolerance, costmap_index, od_index, want_logs)
+                               control_period, goal_tolerance, costmap_index, od_index, want_logs, weights)
 
     def _crowd_run(self, R, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
                    od, ticks, goals, desired_speed, substeps, control_period, goal_tolerance, costmap_index, od_index,
-                   want_logs) -> dict:
+                   want_logs, weights=None) -> dict:
         """run_crowd_episodes (R None) or run_shared_episodes (R robots per scene)."""
         io, out, logs, keep = self.episode_io(global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                                               costmap_resolution, od, ticks, control_period, goal_tolerance,
@@ -232,11 +261,17 @@ class FleetOptimizer:
         people_log = np.zeros((S, T + 1, K, 5)) if want_logs else None
         crowd.people_log = None if people_log is None else people_log.ctypes.data
         res = dict(out, **logs)
-        if R is None:
-            _lib.check(_lib.lib().smpc_run_crowd_episodes(self.opt._h, C.byref(io), C.byref(crowd)))
-        else:
+        scene = None
+        if R is not None:
             res.update(robot_min_dist=np.zeros(B), robot_intimate_ticks=np.zeros(B, np.int32))
             scene = abi.SmpcSceneIo(R, res["robot_min_dist"].ctypes.data, res["robot_intimate_ticks"].ctypes.data)
+        if weights is not None:
+            ws, wkeep = weight_sets_arg(weights, B)
+            _lib.check(_lib.lib().smpc_run_weighted_episodes(self.opt._h, C.byref(io), C.byref(crowd),
+                                                             None if scene is None else C.byref(scene), C.byref(ws)))
+        elif R is None:
+            _lib.check(_lib.lib().smpc_run_crowd_episodes(self.opt._h, C.byref(io), C.byref(crowd)))
+        else:
             _lib.check(_lib.lib().smpc_run_shared_episodes(self.opt._h, C.byref(io), C.byref(crowd), C.byref(scene)))
         res["reached"] = out["reached"].astype(bool)
         res["people_disturbance"] = disturbance

@@ -52,6 +52,27 @@ class OptimizerParams:
         return self
 
 
+def weight_sets(params_list, base) -> np.ndarray:
+    """The [P][9] weight table (abi.WEIGHT_NAMES columns) of P params structs that may differ from `base`, the handle's
+    params, in their critic weights only: every other field is the handle's in a weighted call, so a params that
+    differs elsewhere would not be computed as written. Raises ValueError naming the first such field."""
+    def fields(p):
+        c = p.c if isinstance(p, OptimizerParams) else p
+        return {k: getattr(c, k) for k, _ in abi.SmpcParams._fields_}
+    ref = fields(base)
+    rows = []
+    for i, p in enumerate(params_list):
+        f = fields(p)
+        for k, v in f.items():
+            if k not in abi.WEIGHT_NAMES and v != ref[k]:
+                raise ValueError(f"weight_sets: params {i} differs from the handle's params in {k} "
+                                 f"({v!r} vs {ref[k]!r}); only the critic weights may differ")
+        rows.append(abi.weight_row(p))
+    if not rows:
+        raise ValueError("weight_sets: no params given")
+    return np.array(rows, dtype=np.float64)
+
+
 class Optimizer:
     """Batched drop-in for the solve inside nav2_social_mpc_controller::Optimizer. One instance per GPU."""
 

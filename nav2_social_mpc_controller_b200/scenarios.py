@@ -519,6 +519,20 @@ def crowd_episodes(B: int, K: int, seed: int = 6, ticks: int = 200, substeps: in
     return s
 
 
+EPISODE_ROWS = ("global_path", "pose", "speed", "people", "n_people", "costmap_index", "goals", "desired_speed")
+
+
+def tile_scenes(s: dict, P: int) -> dict:
+    """The one-robot scenes of episodes / crowd_episodes repeated P times: episode p * B0 + i is scene i. The maps stay
+    shared and costmap_index is tiled, so every copy keeps its scene's map. With per-episode critic weights
+    (weights=(table, np.repeat(np.arange(P), B0))) copy p runs under row p: P tunings on the same scenes in one call."""
+    t = dict(s)
+    for k in EPISODE_ROWS:
+        if k in s:
+            t[k] = np.concatenate([np.asarray(s[k])] * P)
+    return t
+
+
 def _place_crowd(s: dict, K: int, seed: int, robots: np.ndarray):
     """The people of crowd_episodes for the scenes of s (episodes(B, 0, ...)): starts keep CROWD_CLEARANCE from every
     robot start robots [B][R][2] and from lethal cells. Returns people [B][K][5], goals [B][K][2], desired speeds."""
