@@ -481,6 +481,53 @@ int smpc_optimize_batch_weighted(smpc_handle* h, smpc_fleet_io* io, const smpc_w
 int smpc_run_weighted_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd /* NULL: constant-velocity people */,
                                const smpc_scene_io* scene /* NULL: one robot per scene */, const smpc_weight_sets* w);
 
+/* ---- closed-loop episodes with an ORCA crowd: people who avoid the robot by a model the controller does not contain -----
+ * smpc_run_crowd_episodes (scene == NULL) or smpc_run_shared_episodes (scene given), optionally with per-robot weights
+ * (w != NULL, as in smpc_run_weighted_episodes), with the people moved by optimal reciprocal collision avoidance (ORCA;
+ * van den Berg et al., "Reciprocal n-body collision avoidance", RVO2's Agent::computeNewVelocity, linearProgram1/2/3
+ * and Agent::update) instead of the social force model the controller's projection uses. io, crowd, scene and w keep
+ * every meaning, layout, output and log; only the crowd step differs. With the lightsfm crowd the controller is graded
+ * on people who behave as it predicts them; ORCA people choose velocities, not forces, and may ignore the robot.
+ * Model, per tick and scene still running, `substeps` synchronous updates of dt_s = control_period / substeps in FP64
+ * (RVO_EPSILON = 1e-5); every line is built from the state at the start of the substep:
+ * - Agents: the scene's n_people_each people and, unless robot_responsibility == 0, robots 0 .. R-1. Robot r is at
+ *   x_k + (s dt_s) v_k (cos th_k, sin th_k) with that velocity; a finished robot stands still; the model never moves it.
+ * - Preferred velocity: desired_speed * unit(goal - p) while the person holds its goal, zero after; the maximum speed
+ *   is desired_speed. The goal is cleared for good the first time an updated position is within 0.25 m of it.
+ * - Neighbours: the other people in slot order, then the robots in order, with distSq < neighbor_dist^2, inserted into a
+ *   list sorted by distSq (strictly <: equal distances keep scan order) of at most max_neighbors; once the list is full
+ *   the range shrinks to its last entry's distSq.
+ * - Obstacle line first: the nearest obstacle cell of the episode's obstacle-distance grid at the person's position
+ *   (none outside the grid) is a static point if it lies within time_horizon_obst * max speed + person_radius: the
+ *   agent line with relative velocity v_i, combined radius person_radius, 1 / time_horizon_obst and full
+ *   responsibility (point = v_i + u). It is never relaxed.
+ * - Agent lines in neighbour order: RVO2's cut-off circle, left-leg and right-leg cases; overlapping agents take the
+ *   collision case with 1 / dt_s. Combined radius person_radius + the other's radius; point = v_i + resp u with
+ *   resp = 1/2 for a person and robot_responsibility for a robot. A collision with |w| == 0 (coincident, co-moving)
+ *   adds no line.
+ * - Solve: linearProgram2 toward the preferred velocity within the circle of the maximum speed; if it fails at line f,
+ *   linearProgram3 from f with the obstacle line hard. Update: v <- the new velocity, p <- p + v dt_s,
+ *   vz = wrap(atan2(vy, vx) - yaw of the previous substep) / dt_s.
+ * people_disturbance[b] here is the velocity change robot b demanded, in m: the sum over ticks robot b ran, substeps
+ * and people whose current velocity violates robot b's line (det(dir, point - v_i) > 0) of
+ * robot_responsibility |u| dt_s. It is not comparable with the lightsfm crowd's force-based value.
+ * Limits as in the lightsfm crowd (n_people + R <= 64, R <= 8, substeps 1..64, finite goals, desired speed > 0).
+ * Returns what the lightsfm entry returns, plus SMPC_ERR_ARGUMENT for orca == NULL, crowd == NULL, a distance, horizon
+ * or radius that is not finite and > 0, max_neighbors outside 1..16 or robot_responsibility outside [0, 1]; all before
+ * anything is launched and before the fleet state is touched. */
+typedef struct smpc_orca_params {
+  double neighbor_dist;        /* m, > 0: agents farther than this do not constrain a person (RVO2 neighborDist) */
+  int max_neighbors;           /* 1..16: the nearest agents within neighbor_dist that a person takes into account */
+  double time_horizon;         /* s, > 0: against other agents */
+  double time_horizon_obst;    /* s, > 0: against the nearest obstacle cell */
+  double person_radius;        /* m, > 0 */
+  double robot_radius;         /* m, > 0 */
+  double robot_responsibility; /* 0..1: share of avoiding a robot that people take; 0 = robots invisible to the crowd */
+} smpc_orca_params;
+int smpc_run_orca_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd,
+                           const smpc_scene_io* scene /* NULL: one robot per scene */,
+                           const smpc_weight_sets* w /* NULL: the handle's weights */, const smpc_orca_params* orca);
+
 /* ---- batched pre-solve stage on the GPU: project_people (src/optimizer.cpp:554-671 + sfm.hpp) -----------------
  * One warp per problem, lanes over agents, sequential over the horizon. Generalised from the reference's 3 people to
  * A columns. Inputs (device pointers): robot [B][S+1][6] = the robot AgentTrajectory of format_to_optimize

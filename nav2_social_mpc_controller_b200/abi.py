@@ -433,6 +433,32 @@ class SmpcWeightSets(C.Structure):
     ]
 
 
+class SmpcOrcaParams(C.Structure):
+    """struct smpc_orca_params — the ORCA crowd of smpc_run_orca_episodes."""
+    _fields_ = [
+        ("neighbor_dist", C.c_double),
+        ("max_neighbors", C.c_int),
+        ("time_horizon", C.c_double),
+        ("time_horizon_obst", C.c_double),
+        ("person_radius", C.c_double),
+        ("robot_radius", C.c_double),
+        ("robot_responsibility", C.c_double),
+    ]
+
+
+ORCA_DEFAULTS = dict(neighbor_dist=10.0, max_neighbors=10, time_horizon=5.0, time_horizon_obst=5.0, person_radius=0.3,
+                     robot_radius=0.3, robot_responsibility=0.5)
+
+
+def orca_params(**overrides) -> SmpcOrcaParams:
+    """SmpcOrcaParams with the defaults ORCA_DEFAULTS (RVO2's usual crowd settings, radii of 0.3 m, people taking half
+    of the avoidance of a robot), any field overridden by keyword."""
+    unknown = set(overrides) - set(ORCA_DEFAULTS)
+    if unknown:
+        raise TypeError(f"unknown ORCA parameters: {sorted(unknown)}")
+    return SmpcOrcaParams(**dict(ORCA_DEFAULTS, **overrides))
+
+
 # the nine critic weights of a row of smpc_weight_sets.weights, in smpc_params order
 WEIGHT_NAMES = ("distance_w", "socialwork_w", "velocity_w", "angle_w", "agent_angle_w", "proxemics_w",
                 "velocity_feasibility_w", "obstacle_w", "goal_align_w")

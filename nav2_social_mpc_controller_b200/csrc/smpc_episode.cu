@@ -1,9 +1,10 @@
-// smpc_episode.cu — closed-loop episodes (smpc_run_episodes, smpc_run_crowd_episodes, smpc_run_shared_episodes): B
+// smpc_episode.cu — closed-loop episodes (smpc_run_episodes, smpc_run_crowd_episodes, smpc_run_shared_episodes,
+// smpc_run_weighted_episodes, smpc_run_orca_episodes): B
 // robots through their crowd scenes for up to T controller ticks, every tick enqueued on the handle's stream without a
 // host round trip. One tick per episode is
 //   trajectorizer (seed) -> tick prep (constant-velocity people at k * dt_c, seed repack, max_time cut) -> [scene view]
-//   -> FOV filter -> fleet tick (smpc_fleet_tick_enqueue) -> [reactive crowd step, smpc_crowd.cu] -> world step (robot
-//   Euler step, metrics, goal check, logs) -> [robot-robot metrics].
+//   -> FOV filter -> fleet tick (smpc_fleet_tick_enqueue) -> [reactive crowd step, smpc_crowd.cu, or ORCA crowd step,
+//   smpc_orca.cu] -> world step (robot Euler step, metrics, goal check, logs) -> [robot-robot metrics].
 // All entries share one loop: with a crowd the prep leaves the people alone, the FOV filter and the world step read
 // the crowd's state, and the crowd step moves it from tick k to k + 1. Shared scenes (R robots per scene, one crowd per
 // scene) add the scene view, which puts the other robots of the scene in front of the people the FOV filter sees, and
@@ -285,9 +286,10 @@ __global__ void smpc_robot_metrics_kernel(RobotMetrics a) {
 
 // The loop of all entries; crowd == NULL: constant-velocity people (smpc_run_episodes); scene == NULL: one robot per
 // scene (smpc_run_episodes, smpc_run_crowd_episodes).
-// w != NULL: per-episode critic weights (smpc_run_weighted_episodes).
+// w != NULL: per-episode critic weights (smpc_run_weighted_episodes). orca != NULL (checked, crowd given): the crowd
+// moves by ORCA (smpc_run_orca_episodes) instead of the social force model.
 int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd, const smpc_scene_io* scene,
-                 const char* name, const smpc_weight_sets* w = nullptr) {
+                 const char* name, const smpc_weight_sets* w = nullptr, const smpc_orca_params* orca = nullptr) {
   auto fail_arg = [name](const char* msg) {
     return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string(name) + ": " + msg);
   };
@@ -566,7 +568,7 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
     if (rc != SMPC_OK) return rc;
     if (reactive) {
       ca.k = k;
-      rc = smpc_crowd_step_enqueue(h, ca, st);
+      rc = orca ? smpc_orca_step_enqueue(h, ca, *orca, st) : smpc_crowd_step_enqueue(h, ca, st);
       if (rc != SMPC_OK) return rc;
     }
     es.k = k;
@@ -648,4 +650,26 @@ extern "C" int smpc_run_weighted_episodes(smpc_handle* h, smpc_episode_io* io, c
   if (rc != SMPC_OK) return rc;
   if (scene && !crowd) return smpc_host_fail(SMPC_ERR_ARGUMENT, "run_weighted_episodes: a shared scene needs a crowd");
   return run_episodes(h, io, crowd, scene, "run_weighted_episodes", w);
+}
+
+extern "C" int smpc_run_orca_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd,
+                                      const smpc_scene_io* scene, const smpc_weight_sets* w,
+                                      const smpc_orca_params* orca) {
+  auto fail_arg = [](const char* msg) {
+    return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string("run_orca_episodes: ") + msg);
+  };
+  if (!orca) return fail_arg("NULL orca");
+  if (!crowd) return fail_arg("NULL crowd");
+  auto positive = [](double x) { return std::isfinite(x) && x > 0.0; };
+  if (!positive(orca->neighbor_dist) || !positive(orca->time_horizon) || !positive(orca->time_horizon_obst) ||
+      !positive(orca->person_radius) || !positive(orca->robot_radius))
+    return fail_arg("a distance, horizon or radius not finite and > 0");
+  if (orca->max_neighbors < 1 || orca->max_neighbors > 16) return fail_arg("max_neighbors outside 1..16");
+  if (!(orca->robot_responsibility >= 0.0 && orca->robot_responsibility <= 1.0))
+    return fail_arg("robot_responsibility outside [0, 1]");
+  if (w) {
+    const int rc = smpc_check_weight_sets(w, 0, "run_orca_episodes");  // the indices: once B is known
+    if (rc != SMPC_OK) return rc;
+  }
+  return run_episodes(h, io, crowd, scene, "run_orca_episodes", w, orca);
 }

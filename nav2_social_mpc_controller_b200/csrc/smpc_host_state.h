@@ -164,6 +164,9 @@ struct smpc_crowd_step_args {
 };
 // Enqueues smpc_crowd_step_kernel on st (one launch).
 int smpc_crowd_step_enqueue(smpc_handle* h, const smpc_crowd_step_args& a, cudaStream_t st);
+// Enqueues smpc_orca_step_kernel (smpc_orca.cu) on st (one launch): the same tick of the same crowd state, with the
+// people moved by ORCA under the checked parameters o instead of the social force model.
+int smpc_orca_step_enqueue(smpc_handle* h, const smpc_crowd_step_args& a, const smpc_orca_params& o, cudaStream_t st);
 
 const smpc_params* smpc_handle_params(smpc_handle* h);
 smpc_fleet_state* smpc_handle_fleet(smpc_handle* h);

@@ -215,36 +215,39 @@ class FleetOptimizer:
     def run_crowd_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                            costmap_resolution, od: dict, ticks: int, goals, desired_speed, substeps=1,
                            control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                           want_logs=False, weights=None) -> dict:
+                           want_logs=False, weights=None, orca=None) -> dict:
         """Closed-loop episodes with a reactive crowd (smpc_run_crowd_episodes): run_episodes, but the people walk to
         their goals [B][K][2] at their desired speeds [B][K] under the lightsfm social force model, `substeps` updates
         per control period, and give way to the robot; people [B][K][5] is their state at t = 0. Returns the dict of
         run_episodes plus people_disturbance [B] (sum of |F(robot -> person)| * dt_s over ticks, substeps and people);
         with want_logs also people_log [B][T+1][K][5] (x, y, vx, vy, vz at every tick, row 0 = the input).
-        weights: as in run_episodes."""
+        weights: as in run_episodes. orca: abi.orca_params(...) (or a dict of its overrides) moves the people by ORCA
+        instead (smpc_run_orca_episodes), a crowd model the controller does not predict with; people_disturbance is
+        then the velocity change the robot demanded, in m."""
         return self._crowd_run(None, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                                costmap_resolution, od, ticks, goals, desired_speed, substeps, control_period,
-                               goal_tolerance, costmap_index, od_index, want_logs, weights)
+                               goal_tolerance, costmap_index, od_index, want_logs, weights, orca)
 
     def run_shared_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                             costmap_resolution, od: dict, ticks: int, goals, desired_speed, robots_per_scene,
                             substeps=1, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                            want_logs=False, weights=None) -> dict:
+                            want_logs=False, weights=None, orca=None) -> dict:
         """Closed-loop episodes in shared scenes (smpc_run_shared_episodes): run_crowd_episodes with the B robots
         grouped into S = B / R scenes of R = robots_per_scene consecutive robots that share one crowd, costmap and
         obstacle grid, and that see each other as people. Per robot: global_path [B][N][2], pose [B][3],
         speed [B][2], costmap_index / od_index [B] (equal within a scene). Per scene: people [S][K][5],
         n_people [S], goals [S][K][2], desired_speed [S][K]. Returns the dict of run_crowd_episodes plus
         robot_min_dist [B] (nearest other robot of the scene, inf for R = 1) and robot_intimate_ticks [B]; with
-        want_logs people_log is per scene, [S][T+1][K][5]. weights: as in run_episodes, set_index per robot."""
+        want_logs people_log is per scene, [S][T+1][K][5]. weights: as in run_episodes, set_index per robot.
+        orca: as in run_crowd_episodes."""
         return self._crowd_run(int(robots_per_scene), global_path, pose, speed, people, n_people, costmaps,
                                costmap_origin, costmap_resolution, od, ticks, goals, desired_speed, substeps,
-                               control_period, goal_tolerance, costmap_index, od_index, want_logs, weights)
+                               control_period, goal_tolerance, costmap_index, od_index, want_logs, weights, orca)
 
     def _crowd_run(self, R, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
                    od, ticks, goals, desired_speed, substeps, control_period, goal_tolerance, costmap_index, od_index,
-                   want_logs, weights=None) -> dict:
-        """run_crowd_episodes (R None) or run_shared_episodes (R robots per scene)."""
+                   want_logs, weights=None, orca=None) -> dict:
+        """run_crowd_episodes (R None) or run_shared_episodes (R robots per scene); orca: the ORCA crowd."""
         io, out, logs, keep = self.episode_io(global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                                               costmap_resolution, od, ticks, control_period, goal_tolerance,
                                               costmap_index, od_index, want_logs, robots_per_scene=R or 1)
@@ -265,7 +268,13 @@ class FleetOptimizer:
         if R is not None:
             res.update(robot_min_dist=np.zeros(B), robot_intimate_ticks=np.zeros(B, np.int32))
             scene = abi.SmpcSceneIo(R, res["robot_min_dist"].ctypes.data, res["robot_intimate_ticks"].ctypes.data)
-        if weights is not None:
+        if orca is not None:
+            op = orca if isinstance(orca, abi.SmpcOrcaParams) else abi.orca_params(**orca)
+            ws, wkeep = weight_sets_arg(weights, B) if weights is not None else (None, None)
+            _lib.check(_lib.lib().smpc_run_orca_episodes(self.opt._h, C.byref(io), C.byref(crowd),
+                                                         None if scene is None else C.byref(scene),
+                                                         None if ws is None else C.byref(ws), C.byref(op)))
+        elif weights is not None:
             ws, wkeep = weight_sets_arg(weights, B)
             _lib.check(_lib.lib().smpc_run_weighted_episodes(self.opt._h, C.byref(io), C.byref(crowd),
                                                              None if scene is None else C.byref(scene), C.byref(ws)))
