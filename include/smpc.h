@@ -528,6 +528,58 @@ int smpc_run_orca_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd
                            const smpc_scene_io* scene /* NULL: one robot per scene */,
                            const smpc_weight_sets* w /* NULL: the handle's weights */, const smpc_orca_params* orca);
 
+/* ---- closed-loop episodes with sensor-limited perception: range, occlusion, missed detections, noisy tracks ----------
+ * Any episode kind above (crowd == NULL: constant-velocity people as smpc_run_episodes; crowd given: the lightsfm crowd,
+ * or the ORCA crowd with orca given; scene given: shared scenes; w given: per-robot weights) with one more stage per
+ * tick between the true scene state and the FOV filter. Its input is the list the FOV filter reads without it, L rows
+ * per robot: the scene's n_people_each people (L = K) or, in shared scenes, the scene view (the other R-1 robots, then
+ * the people; L = R-1+K). Its output is the rows the sensor reports, compacted in input order, which the FOV filter
+ * then reads unchanged. Each row has an agent id: people keep their scene slot 0..K-1, robot r of the scene is K + r.
+ * Row j of robot b at tick k is reported when all four hold:
+ * - range: its true distance from the robot is <= max_range;
+ * - walls (occluding_cost > 0): no costmap cell strictly between the robot's cell and the row's cell has
+ *   cost >= occluding_cost. Amanatides-Woo in grid units g = (p - origin) / resolution of the episode's costmap
+ *   (costmap_index, as the FOV filter), stepping x when tMaxX <= tMaxY and never past the end index on an axis, so the
+ *   walk takes |dix| + |diy| steps; cells outside the costmap do not block;
+ * - people and robots (occluder_radius > 0): no other row i, reported or not, with a strictly smaller squared distance
+ *   lies on the line of sight: e = p_j - r, f = p_i - r, t = (f.e) / (e.e), 0 < t < 1 and |f - t e|^2 <
+ *   occluder_radius^2;
+ * - detection: a uniform u in (0, 1] is <= detect_prob.
+ * A reported row gets N(0, pos_noise^2) on x and y and N(0, vel_noise^2) on vx and vy (vz unchanged; a zero std adds
+ * nothing). Visibility uses true positions. Random numbers: Philox4x32-10 with key (seed low, high 32 bits) and counter
+ * (k, stream, agent id, d), d = 0 for the position pair, 1 for the velocity pair, 2 for the detection draw,
+ * stream = stream_index[b] (NULL: b); u = ((a << 21) + (b >> 11) + 1) 2^-53 from two words (a, b), normals by Box-Muller
+ * r = sqrt(-2 ln u1), (r cos 2 pi u2, r sin 2 pi u2). Counter-based draws do not depend on the launch configuration,
+ * the early-stop poll or the batch: with stream_index[b] = b % B0, copies of B0 scenes (one per weight row) see the same
+ * noise and dropouts.
+ * unseen_personal_ticks[b] counts the ticks robot b ran in which perception did not report some person (not a robot)
+ * whose true distance at tick k is < 1.2 m. Neutral parameters (max_range INFINITY, occluder_radius 0,
+ * occluding_cost 0, detect_prob 1, both noises 0) compute what the entry without perception computes, bit for bit,
+ * with one more launch per tick (none with K = 0 and R = 1: no list, the metric is 0).
+ * Returns what the entry without perception returns, plus SMPC_ERR_ARGUMENT for perception == NULL, a parameter outside
+ * its range or NaN, L > 64, a scene or orca without a crowd, a negative stream_index, unseen_personal_ticks == NULL or
+ * only one of the two logs; all before anything is launched and before the fleet state is touched. */
+typedef struct smpc_perception {
+  double max_range;               /* m, > 0 (INFINITY: unlimited) */
+  double occluder_radius;         /* m, >= 0 and finite; 0 = people and robots do not occlude */
+  int occluding_cost;             /* 0 = walls transparent, else 1..255: a cell with cost >= this blocks sight */
+  double detect_prob;             /* [0, 1] */
+  double pos_noise;               /* m, >= 0, finite: std of each reported coordinate */
+  double vel_noise;               /* m/s, >= 0, finite */
+  uint64_t seed;
+  const int32_t* stream_index;    /* [B] >= 0, or NULL (= b) */
+  int32_t* unseen_personal_ticks; /* [B] out, not NULL */
+  double* seen_log;               /* [B][T][L][5] or NULL: what the FOV filter received at tick k (rows >= n zero;
+                                     rows after an episode is done zero) */
+  int32_t* n_seen_log;            /* [B][T] or NULL (given together with seen_log; 0 after an episode is done) */
+} smpc_perception;
+int smpc_run_perceived_episodes(smpc_handle* h, smpc_episode_io* io,
+                                const smpc_crowd_io* crowd /* NULL: constant-velocity people */,
+                                const smpc_scene_io* scene /* NULL: one robot per scene */,
+                                const smpc_weight_sets* w /* NULL: the handle's weights */,
+                                const smpc_orca_params* orca /* NULL: the lightsfm crowd if crowd is given */,
+                                const smpc_perception* perception);
+
 /* ---- batched pre-solve stage on the GPU: project_people (src/optimizer.cpp:554-671 + sfm.hpp) -----------------
  * One warp per problem, lanes over agents, sequential over the horizon. Generalised from the reference's 3 people to
  * A columns. Inputs (device pointers): robot [B][S+1][6] = the robot AgentTrajectory of format_to_optimize

@@ -459,6 +459,41 @@ def orca_params(**overrides) -> SmpcOrcaParams:
     return SmpcOrcaParams(**dict(ORCA_DEFAULTS, **overrides))
 
 
+class SmpcPerception(C.Structure):
+    """struct smpc_perception — the sensor-limited perception of smpc_run_perceived_episodes."""
+    _fields_ = [
+        ("max_range", C.c_double),
+        ("occluder_radius", C.c_double),
+        ("occluding_cost", C.c_int),
+        ("detect_prob", C.c_double),
+        ("pos_noise", C.c_double),
+        ("vel_noise", C.c_double),
+        ("seed", C.c_uint64),
+        ("stream_index", C.c_void_p),
+        ("unseen_personal_ticks", C.c_void_p),
+        ("seen_log", C.c_void_p),
+        ("n_seen_log", C.c_void_p),
+    ]
+
+
+# A plausible 2-D lidar people tracker (not measured from one): 8 m range, people and robots of 0.25 m radius and lethal
+# cells (254) block the line of sight, 95 % of the visible people detected per tick, 5 cm / 0.1 m/s track noise.
+PERCEPTION_DEFAULTS = dict(max_range=8.0, occluder_radius=0.25, occluding_cost=254, detect_prob=0.95, pos_noise=0.05,
+                           vel_noise=0.1, seed=0)
+# parameters under which the perceived entry computes what the entry without perception computes
+PERCEPTION_NEUTRAL = dict(max_range=float("inf"), occluder_radius=0.0, occluding_cost=0, detect_prob=1.0,
+                          pos_noise=0.0, vel_noise=0.0)
+
+
+def perception_params(**overrides) -> SmpcPerception:
+    """SmpcPerception with the defaults PERCEPTION_DEFAULTS, any field overridden by keyword; the output and stream
+    pointers stay NULL (FleetOptimizer fills them)."""
+    unknown = set(overrides) - set(PERCEPTION_DEFAULTS)
+    if unknown:
+        raise TypeError(f"unknown perception parameters: {sorted(unknown)}")
+    return SmpcPerception(**dict(PERCEPTION_DEFAULTS, **overrides))
+
+
 # the nine critic weights of a row of smpc_weight_sets.weights, in smpc_params order
 WEIGHT_NAMES = ("distance_w", "socialwork_w", "velocity_w", "angle_w", "agent_angle_w", "proxemics_w",
                 "velocity_feasibility_w", "obstacle_w", "goal_align_w")

@@ -1,10 +1,11 @@
 // smpc_episode.cu — closed-loop episodes (smpc_run_episodes, smpc_run_crowd_episodes, smpc_run_shared_episodes,
-// smpc_run_weighted_episodes, smpc_run_orca_episodes): B
+// smpc_run_weighted_episodes, smpc_run_orca_episodes, smpc_run_perceived_episodes): B
 // robots through their crowd scenes for up to T controller ticks, every tick enqueued on the handle's stream without a
 // host round trip. One tick per episode is
 //   trajectorizer (seed) -> tick prep (constant-velocity people at k * dt_c, seed repack, max_time cut) -> [scene view]
-//   -> FOV filter -> fleet tick (smpc_fleet_tick_enqueue) -> [reactive crowd step, smpc_crowd.cu, or ORCA crowd step,
-//   smpc_orca.cu] -> world step (robot Euler step, metrics, goal check, logs) -> [robot-robot metrics].
+//   -> [perception, smpc_perception.cu] -> FOV filter -> fleet tick (smpc_fleet_tick_enqueue) -> [reactive crowd
+//   step, smpc_crowd.cu, or ORCA crowd step, smpc_orca.cu] -> world step (robot Euler step, metrics, goal check, logs)
+//   -> [robot-robot metrics].
 // All entries share one loop: with a crowd the prep leaves the people alone, the FOV filter and the world step read
 // the crowd's state, and the crowd step moves it from tick k to k + 1. Shared scenes (R robots per scene, one crowd per
 // scene) add the scene view, which puts the other robots of the scene in front of the people the FOV filter sees, and
@@ -27,6 +28,7 @@ namespace {
 constexpr int kPollTicks = 16;  // ticks between two reads of the device count of active episodes
 constexpr int kCrowdMaxAgents = 64;  // people + robots in the agent slots of smpc_crowd_step_kernel
 constexpr int kMaxRobotsPerScene = 8;
+constexpr int kPerceptionMaxRows = 64;  // two rows per lane of smpc_perception_kernel's warp
 constexpr double kIntimate = 0.45;  // m, the intimate zone of the person metrics
 // The trajectorizer produces no step within this distance of the path end (smpc_trajectorize_kernel,
 // src/path_trajectorizer.cpp:152). A robot that close has no seed, so the fleet tick leaves it inactive and its
@@ -287,9 +289,11 @@ __global__ void smpc_robot_metrics_kernel(RobotMetrics a) {
 // The loop of all entries; crowd == NULL: constant-velocity people (smpc_run_episodes); scene == NULL: one robot per
 // scene (smpc_run_episodes, smpc_run_crowd_episodes).
 // w != NULL: per-episode critic weights (smpc_run_weighted_episodes). orca != NULL (checked, crowd given): the crowd
-// moves by ORCA (smpc_run_orca_episodes) instead of the social force model.
+// moves by ORCA (smpc_run_orca_episodes) instead of the social force model. pc != NULL (parameters checked): the
+// perception stage cuts the FOV filter's input to what the sensor reports (smpc_run_perceived_episodes).
 int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd, const smpc_scene_io* scene,
-                 const char* name, const smpc_weight_sets* w = nullptr, const smpc_orca_params* orca = nullptr) {
+                 const char* name, const smpc_weight_sets* w = nullptr, const smpc_orca_params* orca = nullptr,
+                 const smpc_perception* pc = nullptr) {
   auto fail_arg = [name](const char* msg) {
     return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string(name) + ": " + msg);
   };
@@ -356,6 +360,12 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
         if (!std::isfinite(vd) || !(vd > 0.0)) return fail_arg("desired_speed not finite and > 0");
       }
   }
+  const int n_list = scene ? R - 1 + K : K;  // rows of the FOV filter's input
+  if (pc) {
+    if (n_list > kPerceptionMaxRows) return fail_arg("the perceived list (R - 1 + n_people rows) above 64");
+    for (int b = 0; b < B && pc->stream_index; ++b)
+      if (pc->stream_index[b] < 0) return fail_arg("stream_index[b] < 0");
+  }
   // the trajectorizer integrates with the yaml DOUBLE time_step (SURVEY Q15), as FleetOptimizer.trajectorize_batch
   const double traj_dt = std::round((double)prm->time_step * 1e6) / 1e6;
   const int max_steps = (int)std::round((double)prm->max_time / traj_dt);
@@ -387,6 +397,11 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
   const bool fov = scene ? n_view > 0 : K > 0;
   const bool logs_pose = io->pose_log != nullptr, logs_cmd = io->cmd_log != nullptr, logs_opt = io->optimized_log != nullptr;
   const bool logs_people = reactive && crowd->people_log != nullptr;
+  const bool perceive = pc && fov;  // K = 0 and R = 1: no list to perceive
+  const bool logs_seen = perceive && pc->seen_log != nullptr;
+  const size_t Lz = n_list;
+  double* seen = nullptr, *seen_log = nullptr;
+  int32_t *seen_n = nullptr, *unseen = nullptr, *stream_idx = nullptr, *n_seen_log = nullptr;
   double *goals = nullptr, *vdes = nullptr, *disturbance = nullptr, *people_log = nullptr;
   double *view = nullptr, *robot_min = nullptr;
   int32_t *view_n = nullptr, *robot_intimate = nullptr;
@@ -454,6 +469,14 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       robot_min = c.take<double>(Bz);
       robot_intimate = c.take<int32_t>(Bz);
     }
+    if (perceive) {
+      seen = c.take<double>(Bz * Lz * 5);
+      seen_n = c.take<int32_t>(Bz);
+      unseen = c.take<int32_t>(Bz);
+      stream_idx = c.take<int32_t>(pc->stream_index ? Bz : 0);
+      seen_log = c.take<double>(logs_seen ? Bz * T * Lz * 5 : 0);
+      n_seen_log = c.take<int32_t>(logs_seen ? Bz * T : 0);
+    }
   };
   size_t need = 0;
   {
@@ -474,6 +497,7 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       {gp, io->global_path, Bz * N * 16}, {pose, io->pose, Bz * 24}, {speed, io->speed, Bz * 16},
       {people0, K > 0 ? io->people : nullptr, Sz * Kz * 40}, {n_people_dev, K > 0 ? io->n_people_each : nullptr, Sz * 4},
       {weights, w ? w->weights : nullptr, w ? (size_t)w->n_sets * 72 : 0}, {weight_set, w ? w->set_index : nullptr, Bz * 4},
+      {stream_idx, perceive ? pc->stream_index : nullptr, Bz * 4},
   };
   for (const Up& u : ups)
     if (u.host && u.bytes) SMPC_FLEET_CUDA(cudaMemcpyAsync(u.dev, u.host, u.bytes, cudaMemcpyHostToDevice, st));
@@ -489,6 +513,7 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
   SMPC_FLEET_CUDA(cudaMemsetAsync(active, 1, Bz, st));
   SMPC_FLEET_CUDA(cudaMemsetAsync(fov_people, 0, Bz * A * 40, st));
   SMPC_FLEET_CUDA(cudaMemsetAsync(fov_n, 0, Bz * 4, st));  // K == 0: nobody to filter, n_people stays 0
+  if (perceive) SMPC_FLEET_CUDA(cudaMemsetAsync(unseen, 0, Bz * 4, st));
   SMPC_FLEET_CUDA(fs->pin_out.reserve(sizeof(int)));
   int* host_active = static_cast<int*>(fs->pin_out.ptr);
   *host_active = B;
@@ -513,6 +538,21 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
   fa.people_in = scene ? view : people; fa.n_people_in = scene ? view_n : n_people_dev; fa.pose = pose;
   fa.costmap_origin = map_org;
   fa.costmap_index = d.map_index; fa.people_out = fov_people; fa.n_people_out = fov_n;
+
+  smpc_perception_args pa{};
+  if (perceive) {  // between the list and the FOV filter, which then reads what the sensor reports
+    pa.B = B; pa.R = R; pa.K = K; pa.L = n_list; pa.T = T;
+    pa.max_range = pc->max_range; pa.occluder_r2 = pc->occluder_radius * pc->occluder_radius;
+    pa.detect_prob = pc->detect_prob; pa.pos_noise = pc->pos_noise; pa.vel_noise = pc->vel_noise;
+    pa.occluding_cost = pc->occluding_cost; pa.seed = pc->seed;
+    pa.active = active; pa.pose = pose; pa.list = fa.people_in; pa.n_list = fa.n_people_in;
+    pa.stream_index = pc->stream_index ? stream_idx : nullptr;
+    pa.maps = maps; pa.map_org = map_org; pa.map_index = d.map_index;
+    pa.n_costmaps = io->n_costmaps; pa.size_x = io->size_x; pa.size_y = io->size_y; pa.resolution = io->resolution;
+    pa.seen = seen; pa.n_seen = seen_n; pa.unseen = unseen;
+    pa.seen_log = logs_seen ? seen_log : nullptr; pa.n_seen_log = logs_seen ? n_seen_log : nullptr;
+    fa.people_in = seen; fa.n_people_in = seen_n;
+  }
 
   // with a crowd the prep moves nobody (K = 0 there): the crowd step does
   EpisodePrep pp{B, reactive ? 0 : K, stride, max_steps, maxsize, 0.0, n_steps, seed_cmds, active, people0, people, d.poses, d.cmds,
@@ -560,6 +600,11 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       SMPC_FLEET_CUDA(cudaGetLastError());
       smpc_handle_count_launch(h);
     }
+    if (perceive) {
+      pa.k = k;
+      rc = smpc_perception_enqueue(h, pa, st);
+      if (rc != SMPC_OK) return rc;
+    }
     if (fov) {
       rc = smpc_fov_filter_batch_device(h, &fa, st);
       if (rc != SMPC_OK) return rc;
@@ -602,6 +647,9 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       {logs_people ? crowd->people_log : nullptr, people_log, Sz * (T + 1) * Kz * 40},
       {scene ? scene->robot_min_dist : nullptr, robot_min, Bz * 8},
       {scene ? scene->robot_intimate_ticks : nullptr, robot_intimate, Bz * 4},
+      {perceive ? pc->unseen_personal_ticks : nullptr, unseen, Bz * 4},
+      {logs_seen ? pc->seen_log : nullptr, seen_log, Bz * T * Lz * 40},
+      {logs_seen ? pc->n_seen_log : nullptr, n_seen_log, Bz * T * 4},
   };
   for (const Down& c : downs)
     if (c.host) SMPC_FLEET_CUDA(cudaMemcpyAsync(c.host, c.dev, c.bytes, cudaMemcpyDeviceToHost, st));
@@ -615,6 +663,14 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
         std::memcpy(io->pose_log + ((size_t)b * (T + 1) + k) * 3, io->pose_log + ((size_t)b * (T + 1) + tb) * 3, 24);
     if (logs_cmd) std::memset(io->cmd_log + ((size_t)b * T + tb) * 2, 0, (size_t)(T - tb) * 16);
     if (logs_opt) std::memset(io->optimized_log + (size_t)b * T + tb, 0, (size_t)(T - tb));
+    if (logs_seen) {
+      std::memset(pc->seen_log + ((size_t)b * T + tb) * Lz * 5, 0, (size_t)(T - tb) * Lz * 40);
+      std::memset(pc->n_seen_log + (size_t)b * T + tb, 0, (size_t)(T - tb) * 4);
+    }
+  }
+  if (pc && !perceive) {  // no list: nothing reported, nobody missed
+    std::memset(pc->unseen_personal_ticks, 0, Bz * 4);
+    if (pc->n_seen_log) std::memset(pc->n_seen_log, 0, Bz * T * 4);
   }
   for (int c = 0; c < S && logs_people; ++c) {  // the people of a finished scene stand where they were at its last tick
     int tc = 0;
@@ -652,6 +708,43 @@ extern "C" int smpc_run_weighted_episodes(smpc_handle* h, smpc_episode_io* io, c
   return run_episodes(h, io, crowd, scene, "run_weighted_episodes", w);
 }
 
+namespace {
+
+// SMPC_ERR_ARGUMENT unless the ORCA parameters are in range (`name` prefixes the message)
+int check_orca_params(const smpc_orca_params* orca, const char* name) {
+  auto fail_arg = [name](const char* msg) {
+    return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string(name) + ": " + msg);
+  };
+  auto positive = [](double x) { return std::isfinite(x) && x > 0.0; };
+  if (!positive(orca->neighbor_dist) || !positive(orca->time_horizon) || !positive(orca->time_horizon_obst) ||
+      !positive(orca->person_radius) || !positive(orca->robot_radius))
+    return fail_arg("a distance, horizon or radius not finite and > 0");
+  if (orca->max_neighbors < 1 || orca->max_neighbors > 16) return fail_arg("max_neighbors outside 1..16");
+  if (!(orca->robot_responsibility >= 0.0 && orca->robot_responsibility <= 1.0))
+    return fail_arg("robot_responsibility outside [0, 1]");
+  return SMPC_OK;
+}
+
+// SMPC_ERR_ARGUMENT unless the perception parameters are in range and the outputs given (the stream indices: once B is
+// known)
+int check_perception(const smpc_perception* pc, const char* name) {
+  auto fail_arg = [name](const char* msg) {
+    return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string(name) + ": " + msg);
+  };
+  if (!(pc->max_range > 0.0)) return fail_arg("max_range not > 0");
+  if (!(std::isfinite(pc->occluder_radius) && pc->occluder_radius >= 0.0))
+    return fail_arg("occluder_radius not finite and >= 0");
+  if (pc->occluding_cost < 0 || pc->occluding_cost > 255) return fail_arg("occluding_cost outside 0..255");
+  if (!(pc->detect_prob >= 0.0 && pc->detect_prob <= 1.0)) return fail_arg("detect_prob outside [0, 1]");
+  if (!(std::isfinite(pc->pos_noise) && pc->pos_noise >= 0.0) || !(std::isfinite(pc->vel_noise) && pc->vel_noise >= 0.0))
+    return fail_arg("pos_noise or vel_noise not finite and >= 0");
+  if (!pc->unseen_personal_ticks) return fail_arg("missing output");
+  if ((pc->seen_log == nullptr) != (pc->n_seen_log == nullptr)) return fail_arg("seen_log and n_seen_log not given together");
+  return SMPC_OK;
+}
+
+}  // namespace
+
 extern "C" int smpc_run_orca_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd,
                                       const smpc_scene_io* scene, const smpc_weight_sets* w,
                                       const smpc_orca_params* orca) {
@@ -660,16 +753,34 @@ extern "C" int smpc_run_orca_episodes(smpc_handle* h, smpc_episode_io* io, const
   };
   if (!orca) return fail_arg("NULL orca");
   if (!crowd) return fail_arg("NULL crowd");
-  auto positive = [](double x) { return std::isfinite(x) && x > 0.0; };
-  if (!positive(orca->neighbor_dist) || !positive(orca->time_horizon) || !positive(orca->time_horizon_obst) ||
-      !positive(orca->person_radius) || !positive(orca->robot_radius))
-    return fail_arg("a distance, horizon or radius not finite and > 0");
-  if (orca->max_neighbors < 1 || orca->max_neighbors > 16) return fail_arg("max_neighbors outside 1..16");
-  if (!(orca->robot_responsibility >= 0.0 && orca->robot_responsibility <= 1.0))
-    return fail_arg("robot_responsibility outside [0, 1]");
+  const int orc = check_orca_params(orca, "run_orca_episodes");
+  if (orc != SMPC_OK) return orc;
   if (w) {
     const int rc = smpc_check_weight_sets(w, 0, "run_orca_episodes");  // the indices: once B is known
     if (rc != SMPC_OK) return rc;
   }
   return run_episodes(h, io, crowd, scene, "run_orca_episodes", w, orca);
+}
+
+extern "C" int smpc_run_perceived_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd,
+                                           const smpc_scene_io* scene, const smpc_weight_sets* w,
+                                           const smpc_orca_params* orca, const smpc_perception* perception) {
+  const char* name = "run_perceived_episodes";
+  auto fail_arg = [name](const char* msg) {
+    return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string(name) + ": " + msg);
+  };
+  if (!perception) return fail_arg("NULL perception");
+  int rc = check_perception(perception, name);
+  if (rc != SMPC_OK) return rc;
+  if (scene && !crowd) return fail_arg("a shared scene needs a crowd");
+  if (orca && !crowd) return fail_arg("an ORCA crowd needs a crowd");
+  if (orca) {
+    rc = check_orca_params(orca, name);
+    if (rc != SMPC_OK) return rc;
+  }
+  if (w) {
+    rc = smpc_check_weight_sets(w, 0, name);  // the indices: once B is known
+    if (rc != SMPC_OK) return rc;
+  }
+  return run_episodes(h, io, crowd, scene, name, w, orca, perception);
 }

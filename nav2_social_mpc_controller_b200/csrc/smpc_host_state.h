@@ -168,6 +168,32 @@ int smpc_crowd_step_enqueue(smpc_handle* h, const smpc_crowd_step_args& a, cudaS
 // people moved by ORCA under the checked parameters o instead of the social force model.
 int smpc_orca_step_enqueue(smpc_handle* h, const smpc_crowd_step_args& a, const smpc_orca_params& o, cudaStream_t st);
 
+// One controller tick of the perception stage of smpc_run_perceived_episodes (smpc_perception.cu), all device pointers:
+// robot b's list (L rows, n_list[b] of them valid) cut to the rows its sensor reports, compacted in input order.
+struct smpc_perception_args {
+  int B, R, K, L, T, k;           // R robots per scene (1: the list holds people only)
+  double max_range, occluder_r2, detect_prob, pos_noise, vel_noise;
+  int occluding_cost;
+  unsigned long long seed;
+  const uint8_t* active;          // [B] robots running tick k; the others report nothing (n_seen = 0)
+  const double* pose;             // [B][3] robot pose of tick k
+  const double* list;             // [B][L][5] the FOV filter's input without perception
+  const int32_t* n_list;          // [B]
+  const int32_t* stream_index;    // [B] or NULL (= b)
+  const uint8_t* maps;
+  const double* map_org;
+  const int32_t* map_index;       // may be NULL (map b % n_costmaps)
+  int n_costmaps, size_x, size_y;
+  double resolution;
+  double* seen;                   // [B][L][5] out: the reported rows
+  int32_t* n_seen;                // [B] out
+  int32_t* unseen;                // [B] += 1 when a person within 1.2 m went unreported
+  double* seen_log;               // [B][T][L][5] or NULL: row k of the robots running tick k
+  int32_t* n_seen_log;            // [B][T] or NULL
+};
+// Enqueues smpc_perception_kernel on st (one launch).
+int smpc_perception_enqueue(smpc_handle* h, const smpc_perception_args& a, cudaStream_t st);
+
 const smpc_params* smpc_handle_params(smpc_handle* h);
 smpc_fleet_state* smpc_handle_fleet(smpc_handle* h);
 smpc_fleet_state* smpc_handle_single(smpc_handle* h);

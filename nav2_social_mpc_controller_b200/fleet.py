@@ -30,6 +30,32 @@ def weight_sets_arg(weights, n_robots: int):
     return abi.SmpcWeightSets(table.shape[0], table.ctypes.data, set_index.ctypes.data), (table, set_index)
 
 
+def perception_arg(perception, n_robots: int, ticks: int, n_rows: int, want_logs: bool):
+    """The smpc_perception of the `perception=` keyword (an abi.SmpcPerception, or a dict of abi.perception_params
+    overrides that may also hold `stream_index` [B]) with its outputs pointed at new arrays: (struct, outputs dict,
+    arrays to keep alive for the call). n_rows = L, the rows of the perceived list."""
+    if isinstance(perception, abi.SmpcPerception):
+        pc = abi.SmpcPerception.from_buffer_copy(perception)
+        stream_index = None
+    else:
+        over = dict(perception)
+        stream_index = over.pop("stream_index", None)
+        pc = abi.perception_params(**over)
+    keep = []
+    if stream_index is not None:
+        stream_index = np.ascontiguousarray(stream_index, dtype=np.int32)
+        if stream_index.shape != (n_robots,):
+            raise ValueError(f"stream_index must be {n_robots} integers, got {stream_index.shape}")
+        pc.stream_index = stream_index.ctypes.data
+        keep.append(stream_index)
+    out = dict(unseen_personal_ticks=np.zeros(n_robots, np.int32))
+    if want_logs:
+        out.update(seen_log=np.zeros((n_robots, ticks, n_rows, 5)), n_seen_log=np.zeros((n_robots, ticks), np.int32))
+    for k, v in out.items():
+        setattr(pc, k, v.ctypes.data)
+    return pc, out, keep
+
+
 class FleetOptimizer:
     def __init__(self, params, n_robots: int, n_agents: int = 3, device: int = 0):
         self.device = device
@@ -188,7 +214,7 @@ class FleetOptimizer:
 
     def run_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
                      od: dict, ticks: int, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                     want_logs=False, weights=None) -> dict:
+                     want_logs=False, weights=None, perception=None) -> dict:
         """Closed-loop episodes on the GPU (smpc_run_episodes): each of the B robots runs its crowd scene for up to
         `ticks` controller ticks — trajectorizer seed, constant-velocity people, FOV filter, the fleet tick, a unicycle
         world step — with one upload and one download for the whole run. global_path [B][N][2], pose [B][3],
@@ -197,11 +223,22 @@ class FleetOptimizer:
         intimate_ticks, personal_ticks, collision_ticks, not_optimized_ticks, cmd_variation; with want_logs also
         pose_log [B][T+1][3], cmd_log [B][T][2], optimized_log [B][T] (bool).
         weights = (table [P][9], set_index [B]) as in optimize_batch: episode b runs with row set_index[b]
-        (smpc_run_weighted_episodes)."""
+        (smpc_run_weighted_episodes).
+        perception: abi.perception_params(...), or a dict of its overrides plus an optional stream_index [B], puts a
+        sensor between the people and the FOV filter (smpc_run_perceived_episodes): range, occlusion by walls and people,
+        missed detections and noisy tracks. The dict then also holds unseen_personal_ticks [B] (ticks with a person
+        within 1.2 m that went unreported) and, with want_logs, seen_log [B][T][K][5] and n_seen_log [B][T] (what the
+        FOV filter received at each tick)."""
         io, out, logs, keep = self.episode_io(global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                                               costmap_resolution, od, ticks, control_period, goal_tolerance,
                                               costmap_index, od_index, want_logs)
-        if weights is None:
+        if perception is not None:
+            pc, pout, pkeep = perception_arg(perception, self.B, int(ticks), io.n_people, want_logs)
+            ws, wkeep = weight_sets_arg(weights, self.B) if weights is not None else (None, None)
+            _lib.check(_lib.lib().smpc_run_perceived_episodes(self.opt._h, C.byref(io), None, None,
+                                                              None if ws is None else C.byref(ws), None, C.byref(pc)))
+            out.update(pout)
+        elif weights is None:
             _lib.check(_lib.lib().smpc_run_episodes(self.opt._h, C.byref(io)))
         else:
             ws, wkeep = weight_sets_arg(weights, self.B)
@@ -215,7 +252,7 @@ class FleetOptimizer:
     def run_crowd_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                            costmap_resolution, od: dict, ticks: int, goals, desired_speed, substeps=1,
                            control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                           want_logs=False, weights=None, orca=None) -> dict:
+                           want_logs=False, weights=None, orca=None, perception=None) -> dict:
         """Closed-loop episodes with a reactive crowd (smpc_run_crowd_episodes): run_episodes, but the people walk to
         their goals [B][K][2] at their desired speeds [B][K] under the lightsfm social force model, `substeps` updates
         per control period, and give way to the robot; people [B][K][5] is their state at t = 0. Returns the dict of
@@ -223,15 +260,15 @@ class FleetOptimizer:
         with want_logs also people_log [B][T+1][K][5] (x, y, vx, vy, vz at every tick, row 0 = the input).
         weights: as in run_episodes. orca: abi.orca_params(...) (or a dict of its overrides) moves the people by ORCA
         instead (smpc_run_orca_episodes), a crowd model the controller does not predict with; people_disturbance is
-        then the velocity change the robot demanded, in m."""
+        then the velocity change the robot demanded, in m. perception: as in run_episodes."""
         return self._crowd_run(None, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                                costmap_resolution, od, ticks, goals, desired_speed, substeps, control_period,
-                               goal_tolerance, costmap_index, od_index, want_logs, weights, orca)
+                               goal_tolerance, costmap_index, od_index, want_logs, weights, orca, perception)
 
     def run_shared_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                             costmap_resolution, od: dict, ticks: int, goals, desired_speed, robots_per_scene,
                             substeps=1, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                            want_logs=False, weights=None, orca=None) -> dict:
+                            want_logs=False, weights=None, orca=None, perception=None) -> dict:
         """Closed-loop episodes in shared scenes (smpc_run_shared_episodes): run_crowd_episodes with the B robots
         grouped into S = B / R scenes of R = robots_per_scene consecutive robots that share one crowd, costmap and
         obstacle grid, and that see each other as people. Per robot: global_path [B][N][2], pose [B][3],
@@ -239,15 +276,18 @@ class FleetOptimizer:
         n_people [S], goals [S][K][2], desired_speed [S][K]. Returns the dict of run_crowd_episodes plus
         robot_min_dist [B] (nearest other robot of the scene, inf for R = 1) and robot_intimate_ticks [B]; with
         want_logs people_log is per scene, [S][T+1][K][5]. weights: as in run_episodes, set_index per robot.
-        orca: as in run_crowd_episodes."""
+        orca: as in run_crowd_episodes. perception: as in run_episodes; a robot's list is its scene view, the other
+        R - 1 robots then the people, so seen_log is [B][T][R-1+K][5]."""
         return self._crowd_run(int(robots_per_scene), global_path, pose, speed, people, n_people, costmaps,
                                costmap_origin, costmap_resolution, od, ticks, goals, desired_speed, substeps,
-                               control_period, goal_tolerance, costmap_index, od_index, want_logs, weights, orca)
+                               control_period, goal_tolerance, costmap_index, od_index, want_logs, weights, orca,
+                               perception)
 
     def _crowd_run(self, R, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
                    od, ticks, goals, desired_speed, substeps, control_period, goal_tolerance, costmap_index, od_index,
-                   want_logs, weights=None, orca=None) -> dict:
-        """run_crowd_episodes (R None) or run_shared_episodes (R robots per scene); orca: the ORCA crowd."""
+                   want_logs, weights=None, orca=None, perception=None) -> dict:
+        """run_crowd_episodes (R None) or run_shared_episodes (R robots per scene); orca: the ORCA crowd; perception:
+        the sensor between the scene and the FOV filter."""
         io, out, logs, keep = self.episode_io(global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                                               costmap_resolution, od, ticks, control_period, goal_tolerance,
                                               costmap_index, od_index, want_logs, robots_per_scene=R or 1)
@@ -268,7 +308,16 @@ class FleetOptimizer:
         if R is not None:
             res.update(robot_min_dist=np.zeros(B), robot_intimate_ticks=np.zeros(B, np.int32))
             scene = abi.SmpcSceneIo(R, res["robot_min_dist"].ctypes.data, res["robot_intimate_ticks"].ctypes.data)
-        if orca is not None:
+        if perception is not None:
+            op = None if orca is None else orca if isinstance(orca, abi.SmpcOrcaParams) else abi.orca_params(**orca)
+            pc, pout, pkeep = perception_arg(perception, B, T, (R or 1) - 1 + K, want_logs)
+            ws, wkeep = weight_sets_arg(weights, B) if weights is not None else (None, None)
+            _lib.check(_lib.lib().smpc_run_perceived_episodes(self.opt._h, C.byref(io), C.byref(crowd),
+                                                              None if scene is None else C.byref(scene),
+                                                              None if ws is None else C.byref(ws),
+                                                              None if op is None else C.byref(op), C.byref(pc)))
+            res.update(pout)
+        elif orca is not None:
             op = orca if isinstance(orca, abi.SmpcOrcaParams) else abi.orca_params(**orca)
             ws, wkeep = weight_sets_arg(weights, B) if weights is not None else (None, None)
             _lib.check(_lib.lib().smpc_run_orca_episodes(self.opt._h, C.byref(io), C.byref(crowd),
