@@ -580,6 +580,56 @@ int smpc_run_perceived_episodes(smpc_handle* h, smpc_episode_io* io,
                                 const smpc_orca_params* orca /* NULL: the lightsfm crowd if crowd is given */,
                                 const smpc_perception* perception);
 
+/* ---- closed-loop episodes with tracked perception: a per-robot Kalman people tracker with confirmation, coasting and
+ * latency ---------------------------------------------------------------------------------------------------------------
+ * smpc_run_perceived_episodes with a people tracker between the sensor and the FOV filter. The detections are those of
+ * the perception stage (same seed, stream, tests and draws); the measurement is the detected position z with its
+ * pos_noise, so perception->vel_noise must be 0. Association is by agent id (people: scene slot 0..K-1, robot r of a
+ * shared scene: K + r), with no gating and no id switches. Each id of each robot has one constant-velocity Kalman track
+ * with state (x, y, vx, vy) and one per-axis covariance (p_pp, p_pv, p_vv) that both axes share; every tick the robot
+ * runs, with dt = control_period, a2 = accel_noise^2, r2 = meas_noise^2:
+ * - a detection of an id without a track starts one: p = z, v = 0, (p_pp, p_pv, p_vv) = (r2, 0, init_vel_std^2),
+ *   hits = 1;
+ * - a detection of a tracked id predicts (p += dt v; p_pp += 2 dt p_pv + dt^2 p_vv + a2 dt^4 / 4;
+ *   p_pv += dt p_vv + a2 dt^3 / 2; p_vv += a2 dt^2) and updates (S = p_pp + r2, k0 = p_pp / S, k1 = p_pv / S;
+ *   p += k0 (z - p), v += k1 (z - p), p_vv -= k1 p_pv, p_pv -= k0 p_pv, p_pp -= k0 p_pp from the predicted values);
+ *   hits += 1 (saturating at 16), misses = 0;
+ * - a missed tracked id predicts only; misses += 1, and the track ends when misses > max_coast_ticks.
+ * A track is published while it lives with hits >= confirm_hits, coasting ones at their prediction, as the row
+ * (x, y, vx, vy, 0) (a position tracker estimates no turn rate), in the order of the perceived list. The FOV filter at
+ * tick k reads the list published at tick k - latency_ticks (nobody before latency_ticks). A finished robot publishes
+ * nothing and its tracks freeze. perception->seen_log / n_seen_log record that delayed list, track_id_log the ids of
+ * its rows (-1 past n and after an episode is done).
+ * Per robot, over the ticks it ran and for people only: untracked_personal_ticks counts the ticks in which a person
+ * truly within 1.2 m at tick k is not in the list the FOV filter received; track_rows counts the people rows it
+ * received, track_pos_err / track_vel_err sum |p_hat - p(k)| and |v_hat - v(k)| against their true rows of tick k.
+ * confirm_hits 1, max_coast_ticks 0 and latency_ticks 0 publish exactly what was detected; on people standing still
+ * with pos_noise 0 that is the list of smpc_run_perceived_episodes, bit for bit. The launches per tick are those of
+ * smpc_run_perceived_episodes. Device memory beyond it: 64 B per track (B M, M = K, or K + R in shared scenes) and
+ * 44 B per row of each of the latency_ticks + 1 ring slots (B L).
+ * Returns what smpc_run_perceived_episodes returns, plus SMPC_ERR_ARGUMENT for tracker == NULL, a parameter outside its
+ * range or NaN, perception->vel_noise != 0, a missing output, or track_id_log given without seen_log or the other way
+ * round; all before anything is launched and before the fleet state is touched. */
+typedef struct smpc_tracker {
+  double accel_noise;               /* m/s^2, >= 0, finite: std of the white acceleration of the motion model */
+  double meas_noise;                /* m, > 0, finite: std of a detected coordinate */
+  double init_vel_std;              /* m/s, > 0, finite: std of the velocity of a new track */
+  int confirm_hits;                 /* 1..16: detections before a track is published */
+  int max_coast_ticks;              /* 0..64: misses a track survives */
+  int latency_ticks;                /* 0..16: ticks from publication to the FOV filter */
+  int32_t* untracked_personal_ticks; /* [B] out, not NULL */
+  int32_t* track_rows;              /* [B] out, not NULL */
+  double* track_pos_err;            /* [B] out, not NULL: m, summed over track_rows */
+  double* track_vel_err;            /* [B] out, not NULL: m/s, summed over track_rows */
+  int32_t* track_id_log;            /* [B][T][L] or NULL (given exactly when perception->seen_log is) */
+} smpc_tracker;
+int smpc_run_tracked_episodes(smpc_handle* h, smpc_episode_io* io,
+                              const smpc_crowd_io* crowd /* NULL: constant-velocity people */,
+                              const smpc_scene_io* scene /* NULL: one robot per scene */,
+                              const smpc_weight_sets* w /* NULL: the handle's weights */,
+                              const smpc_orca_params* orca /* NULL: the lightsfm crowd if crowd is given */,
+                              const smpc_perception* perception, const smpc_tracker* tracker);
+
 /* ---- batched pre-solve stage on the GPU: project_people (src/optimizer.cpp:554-671 + sfm.hpp) -----------------
  * One warp per problem, lanes over agents, sequential over the horizon. Generalised from the reference's 3 people to
  * A columns. Inputs (device pointers): robot [B][S+1][6] = the robot AgentTrajectory of format_to_optimize

@@ -494,6 +494,41 @@ def perception_params(**overrides) -> SmpcPerception:
     return SmpcPerception(**dict(PERCEPTION_DEFAULTS, **overrides))
 
 
+class SmpcTracker(C.Structure):
+    """struct smpc_tracker — the people tracker of smpc_run_tracked_episodes."""
+    _fields_ = [
+        ("accel_noise", C.c_double),
+        ("meas_noise", C.c_double),
+        ("init_vel_std", C.c_double),
+        ("confirm_hits", C.c_int),
+        ("max_coast_ticks", C.c_int),
+        ("latency_ticks", C.c_int),
+        ("untracked_personal_ticks", C.c_void_p),
+        ("track_rows", C.c_void_p),
+        ("track_pos_err", C.c_void_p),
+        ("track_vel_err", C.c_void_p),
+        ("track_id_log", C.c_void_p),
+    ]
+
+
+# A plausible 2-D people tracker (not measured from one): a constant-velocity Kalman filter with 0.5 m/s^2 white
+# acceleration and 5 cm measurement noise, new tracks at 1 m/s velocity uncertainty, published after 3 detections,
+# coasted through 10 missed ticks (0.5 s at 20 Hz) and delivered 2 ticks (100 ms) late.
+TRACKER_DEFAULTS = dict(accel_noise=0.5, meas_noise=0.05, init_vel_std=1.0, confirm_hits=3, max_coast_ticks=10,
+                        latency_ticks=2)
+# parameters under which the tracker publishes exactly what was detected, at once
+TRACKER_PASS_THROUGH = dict(confirm_hits=1, max_coast_ticks=0, latency_ticks=0)
+
+
+def tracker_params(**overrides) -> SmpcTracker:
+    """SmpcTracker with the defaults TRACKER_DEFAULTS, any field overridden by keyword; the output pointers stay NULL
+    (FleetOptimizer fills them)."""
+    unknown = set(overrides) - set(TRACKER_DEFAULTS)
+    if unknown:
+        raise TypeError(f"unknown tracker parameters: {sorted(unknown)}")
+    return SmpcTracker(**dict(TRACKER_DEFAULTS, **overrides))
+
+
 # the nine critic weights of a row of smpc_weight_sets.weights, in smpc_params order
 WEIGHT_NAMES = ("distance_w", "socialwork_w", "velocity_w", "angle_w", "agent_angle_w", "proxemics_w",
                 "velocity_feasibility_w", "obstacle_w", "goal_align_w")

@@ -1,11 +1,11 @@
 // smpc_episode.cu — closed-loop episodes (smpc_run_episodes, smpc_run_crowd_episodes, smpc_run_shared_episodes,
-// smpc_run_weighted_episodes, smpc_run_orca_episodes, smpc_run_perceived_episodes): B
+// smpc_run_weighted_episodes, smpc_run_orca_episodes, smpc_run_perceived_episodes, smpc_run_tracked_episodes): B
 // robots through their crowd scenes for up to T controller ticks, every tick enqueued on the handle's stream without a
 // host round trip. One tick per episode is
 //   trajectorizer (seed) -> tick prep (constant-velocity people at k * dt_c, seed repack, max_time cut) -> [scene view]
-//   -> [perception, smpc_perception.cu] -> FOV filter -> fleet tick (smpc_fleet_tick_enqueue) -> [reactive crowd
-//   step, smpc_crowd.cu, or ORCA crowd step, smpc_orca.cu] -> world step (robot Euler step, metrics, goal check, logs)
-//   -> [robot-robot metrics].
+//   -> [perception, smpc_perception.cu, or tracked perception, smpc_tracker.cu] -> FOV filter -> fleet tick
+//   (smpc_fleet_tick_enqueue) -> [reactive crowd step, smpc_crowd.cu, or ORCA crowd step, smpc_orca.cu] -> world step
+//   (robot Euler step, metrics, goal check, logs) -> [robot-robot metrics].
 // All entries share one loop: with a crowd the prep leaves the people alone, the FOV filter and the world step read
 // the crowd's state, and the crowd step moves it from tick k to k + 1. Shared scenes (R robots per scene, one crowd per
 // scene) add the scene view, which puts the other robots of the scene in front of the people the FOV filter sees, and
@@ -290,10 +290,12 @@ __global__ void smpc_robot_metrics_kernel(RobotMetrics a) {
 // scene (smpc_run_episodes, smpc_run_crowd_episodes).
 // w != NULL: per-episode critic weights (smpc_run_weighted_episodes). orca != NULL (checked, crowd given): the crowd
 // moves by ORCA (smpc_run_orca_episodes) instead of the social force model. pc != NULL (parameters checked): the
-// perception stage cuts the FOV filter's input to what the sensor reports (smpc_run_perceived_episodes).
+// perception stage cuts the FOV filter's input to what the sensor reports (smpc_run_perceived_episodes). tk != NULL
+// (checked, pc given): a people tracker follows the sensor and the FOV filter reads its delayed published list
+// (smpc_run_tracked_episodes).
 int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd, const smpc_scene_io* scene,
                  const char* name, const smpc_weight_sets* w = nullptr, const smpc_orca_params* orca = nullptr,
-                 const smpc_perception* pc = nullptr) {
+                 const smpc_perception* pc = nullptr, const smpc_tracker* tk = nullptr) {
   auto fail_arg = [name](const char* msg) {
     return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string(name) + ": " + msg);
   };
@@ -402,6 +404,12 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
   const size_t Lz = n_list;
   double* seen = nullptr, *seen_log = nullptr;
   int32_t *seen_n = nullptr, *unseen = nullptr, *stream_idx = nullptr, *n_seen_log = nullptr;
+  const bool tracked = perceive && tk != nullptr;
+  const size_t Mz = scene ? K + R : K, Dz = tracked ? tk->latency_ticks + 1 : 0;  // track slots, ring slots
+  double *trk_x = nullptr, *trk_y = nullptr, *trk_vx = nullptr, *trk_vy = nullptr;
+  double *trk_pp = nullptr, *trk_pv = nullptr, *trk_vv = nullptr, *ring = nullptr, *pos_err = nullptr, *vel_err = nullptr;
+  int32_t *trk_hits = nullptr, *trk_misses = nullptr, *ring_n = nullptr, *ring_id = nullptr, *untracked = nullptr;
+  int32_t *track_rows = nullptr, *id_log = nullptr;
   double *goals = nullptr, *vdes = nullptr, *disturbance = nullptr, *people_log = nullptr;
   double *view = nullptr, *robot_min = nullptr;
   int32_t *view_n = nullptr, *robot_intimate = nullptr;
@@ -470,12 +478,31 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       robot_intimate = c.take<int32_t>(Bz);
     }
     if (perceive) {
-      seen = c.take<double>(Bz * Lz * 5);
-      seen_n = c.take<int32_t>(Bz);
+      seen = c.take<double>(tracked ? 0 : Bz * Lz * 5);
+      seen_n = c.take<int32_t>(tracked ? 0 : Bz);
       unseen = c.take<int32_t>(Bz);
       stream_idx = c.take<int32_t>(pc->stream_index ? Bz : 0);
       seen_log = c.take<double>(logs_seen ? Bz * T * Lz * 5 : 0);
       n_seen_log = c.take<int32_t>(logs_seen ? Bz * T : 0);
+    }
+    if (tracked) {
+      trk_x = c.take<double>(Bz * Mz);
+      trk_y = c.take<double>(Bz * Mz);
+      trk_vx = c.take<double>(Bz * Mz);
+      trk_vy = c.take<double>(Bz * Mz);
+      trk_pp = c.take<double>(Bz * Mz);
+      trk_pv = c.take<double>(Bz * Mz);
+      trk_vv = c.take<double>(Bz * Mz);
+      trk_hits = c.take<int32_t>(Bz * Mz);
+      trk_misses = c.take<int32_t>(Bz * Mz);
+      ring = c.take<double>(Dz * Bz * Lz * 5);
+      ring_n = c.take<int32_t>(Dz * Bz);
+      ring_id = c.take<int32_t>(Dz * Bz * Lz);
+      untracked = c.take<int32_t>(Bz);
+      track_rows = c.take<int32_t>(Bz);
+      pos_err = c.take<double>(Bz);
+      vel_err = c.take<double>(Bz);
+      id_log = c.take<int32_t>(logs_seen ? Bz * T * Lz : 0);
     }
   };
   size_t need = 0;
@@ -514,6 +541,17 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
   SMPC_FLEET_CUDA(cudaMemsetAsync(fov_people, 0, Bz * A * 40, st));
   SMPC_FLEET_CUDA(cudaMemsetAsync(fov_n, 0, Bz * 4, st));  // K == 0: nobody to filter, n_people stays 0
   if (perceive) SMPC_FLEET_CUDA(cudaMemsetAsync(unseen, 0, Bz * 4, st));
+  if (tracked) {  // no tracks, and nothing published before tick 0
+    SMPC_FLEET_CUDA(cudaMemsetAsync(trk_hits, 0, Bz * Mz * 4, st));
+    SMPC_FLEET_CUDA(cudaMemsetAsync(trk_misses, 0, Bz * Mz * 4, st));
+    for (double* p : {trk_x, trk_y, trk_vx, trk_vy, trk_pp, trk_pv, trk_vv})
+      SMPC_FLEET_CUDA(cudaMemsetAsync(p, 0, Bz * Mz * 8, st));
+    SMPC_FLEET_CUDA(cudaMemsetAsync(ring_n, 0, Dz * Bz * 4, st));
+    SMPC_FLEET_CUDA(cudaMemsetAsync(untracked, 0, Bz * 4, st));
+    SMPC_FLEET_CUDA(cudaMemsetAsync(track_rows, 0, Bz * 4, st));
+    SMPC_FLEET_CUDA(cudaMemsetAsync(pos_err, 0, Bz * 8, st));
+    SMPC_FLEET_CUDA(cudaMemsetAsync(vel_err, 0, Bz * 8, st));
+  }
   SMPC_FLEET_CUDA(fs->pin_out.reserve(sizeof(int)));
   int* host_active = static_cast<int*>(fs->pin_out.ptr);
   *host_active = B;
@@ -552,6 +590,18 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
     pa.seen = seen; pa.n_seen = seen_n; pa.unseen = unseen;
     pa.seen_log = logs_seen ? seen_log : nullptr; pa.n_seen_log = logs_seen ? n_seen_log : nullptr;
     fa.people_in = seen; fa.n_people_in = seen_n;
+  }
+  smpc_tracker_args tka{};
+  if (tracked) {  // the FOV filter reads a ring slot instead, switched every tick
+    tka.p = pa;
+    tka.p.seen = nullptr; tka.p.n_seen = nullptr;
+    tka.M = (int)Mz; tka.confirm_hits = tk->confirm_hits; tka.max_coast = tk->max_coast_ticks;
+    tka.dt = io->control_period; tka.accel_noise = tk->accel_noise; tka.meas_noise = tk->meas_noise;
+    tka.init_vel_std = tk->init_vel_std;
+    tka.px = trk_x; tka.py = trk_y; tka.vx = trk_vx; tka.vy = trk_vy;
+    tka.p_pp = trk_pp; tka.p_pv = trk_pv; tka.p_vv = trk_vv; tka.hits = trk_hits; tka.misses = trk_misses;
+    tka.untracked = untracked; tka.track_rows = track_rows; tka.pos_err = pos_err; tka.vel_err = vel_err;
+    tka.id_log = logs_seen ? id_log : nullptr;
   }
 
   // with a crowd the prep moves nobody (K = 0 there): the crowd step does
@@ -600,7 +650,15 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       SMPC_FLEET_CUDA(cudaGetLastError());
       smpc_handle_count_launch(h);
     }
-    if (perceive) {
+    if (tracked) {  // publish into slot k mod D; the FOV filter reads slot (k - latency) mod D
+      const size_t sp = (size_t)k % Dz, sd = (size_t)(k + 1) % Dz;
+      tka.p.k = k;
+      tka.pub = ring + sp * Bz * Lz * 5; tka.pub_n = ring_n + sp * Bz; tka.pub_id = ring_id + sp * Bz * Lz;
+      tka.del = ring + sd * Bz * Lz * 5; tka.del_n = ring_n + sd * Bz; tka.del_id = ring_id + sd * Bz * Lz;
+      fa.people_in = tka.del; fa.n_people_in = tka.del_n;
+      rc = smpc_tracked_perception_enqueue(h, tka, st);
+      if (rc != SMPC_OK) return rc;
+    } else if (perceive) {
       pa.k = k;
       rc = smpc_perception_enqueue(h, pa, st);
       if (rc != SMPC_OK) return rc;
@@ -650,6 +708,11 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       {perceive ? pc->unseen_personal_ticks : nullptr, unseen, Bz * 4},
       {logs_seen ? pc->seen_log : nullptr, seen_log, Bz * T * Lz * 40},
       {logs_seen ? pc->n_seen_log : nullptr, n_seen_log, Bz * T * 4},
+      {tracked ? tk->untracked_personal_ticks : nullptr, untracked, Bz * 4},
+      {tracked ? tk->track_rows : nullptr, track_rows, Bz * 4},
+      {tracked ? tk->track_pos_err : nullptr, pos_err, Bz * 8},
+      {tracked ? tk->track_vel_err : nullptr, vel_err, Bz * 8},
+      {tracked && logs_seen ? tk->track_id_log : nullptr, id_log, Bz * T * Lz * 4},
   };
   for (const Down& c : downs)
     if (c.host) SMPC_FLEET_CUDA(cudaMemcpyAsync(c.host, c.dev, c.bytes, cudaMemcpyDeviceToHost, st));
@@ -667,10 +730,17 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       std::memset(pc->seen_log + ((size_t)b * T + tb) * Lz * 5, 0, (size_t)(T - tb) * Lz * 40);
       std::memset(pc->n_seen_log + (size_t)b * T + tb, 0, (size_t)(T - tb) * 4);
     }
+    if (tracked && logs_seen) std::fill_n(tk->track_id_log + ((size_t)b * T + tb) * Lz, (size_t)(T - tb) * Lz, -1);
   }
   if (pc && !perceive) {  // no list: nothing reported, nobody missed
     std::memset(pc->unseen_personal_ticks, 0, Bz * 4);
     if (pc->n_seen_log) std::memset(pc->n_seen_log, 0, Bz * T * 4);
+  }
+  if (tk && !perceive) {  // no list: nothing tracked, nobody missed
+    std::memset(tk->untracked_personal_ticks, 0, Bz * 4);
+    std::memset(tk->track_rows, 0, Bz * 4);
+    std::memset(tk->track_pos_err, 0, Bz * 8);
+    std::memset(tk->track_vel_err, 0, Bz * 8);
   }
   for (int c = 0; c < S && logs_people; ++c) {  // the people of a finished scene stand where they were at its last tick
     int tc = 0;
@@ -743,6 +813,27 @@ int check_perception(const smpc_perception* pc, const char* name) {
   return SMPC_OK;
 }
 
+// SMPC_ERR_ARGUMENT unless the tracker parameters are in range, the perception gives positions only and the outputs
+// are given
+int check_tracker(const smpc_tracker* tk, const smpc_perception* pc, const char* name) {
+  auto fail_arg = [name](const char* msg) {
+    return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string(name) + ": " + msg);
+  };
+  if (!(std::isfinite(tk->accel_noise) && tk->accel_noise >= 0.0)) return fail_arg("accel_noise not finite and >= 0");
+  if (!(std::isfinite(tk->meas_noise) && tk->meas_noise > 0.0) ||
+      !(std::isfinite(tk->init_vel_std) && tk->init_vel_std > 0.0))
+    return fail_arg("meas_noise or init_vel_std not finite and > 0");
+  if (tk->confirm_hits < 1 || tk->confirm_hits > 16) return fail_arg("confirm_hits outside 1..16");
+  if (tk->max_coast_ticks < 0 || tk->max_coast_ticks > 64) return fail_arg("max_coast_ticks outside 0..64");
+  if (tk->latency_ticks < 0 || tk->latency_ticks > 16) return fail_arg("latency_ticks outside 0..16");
+  if (pc->vel_noise != 0.0) return fail_arg("perception vel_noise not 0 (the tracker estimates velocities itself)");
+  if (!tk->untracked_personal_ticks || !tk->track_rows || !tk->track_pos_err || !tk->track_vel_err)
+    return fail_arg("missing output");
+  if ((tk->track_id_log == nullptr) != (pc->seen_log == nullptr))
+    return fail_arg("track_id_log and seen_log not given together");
+  return SMPC_OK;
+}
+
 }  // namespace
 
 extern "C" int smpc_run_orca_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd,
@@ -762,16 +853,22 @@ extern "C" int smpc_run_orca_episodes(smpc_handle* h, smpc_episode_io* io, const
   return run_episodes(h, io, crowd, scene, "run_orca_episodes", w, orca);
 }
 
-extern "C" int smpc_run_perceived_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd,
-                                           const smpc_scene_io* scene, const smpc_weight_sets* w,
-                                           const smpc_orca_params* orca, const smpc_perception* perception) {
-  const char* name = "run_perceived_episodes";
+namespace {
+
+// smpc_run_perceived_episodes (tk == NULL) and smpc_run_tracked_episodes: the argument checks that need no B
+int run_perceived(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd, const smpc_scene_io* scene,
+                  const smpc_weight_sets* w, const smpc_orca_params* orca, const smpc_perception* perception,
+                  const smpc_tracker* tk, const char* name) {
   auto fail_arg = [name](const char* msg) {
     return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string(name) + ": " + msg);
   };
   if (!perception) return fail_arg("NULL perception");
   int rc = check_perception(perception, name);
   if (rc != SMPC_OK) return rc;
+  if (tk) {
+    rc = check_tracker(tk, perception, name);
+    if (rc != SMPC_OK) return rc;
+  }
   if (scene && !crowd) return fail_arg("a shared scene needs a crowd");
   if (orca && !crowd) return fail_arg("an ORCA crowd needs a crowd");
   if (orca) {
@@ -782,5 +879,21 @@ extern "C" int smpc_run_perceived_episodes(smpc_handle* h, smpc_episode_io* io, 
     rc = smpc_check_weight_sets(w, 0, name);  // the indices: once B is known
     if (rc != SMPC_OK) return rc;
   }
-  return run_episodes(h, io, crowd, scene, name, w, orca, perception);
+  return run_episodes(h, io, crowd, scene, name, w, orca, perception, tk);
+}
+
+}  // namespace
+
+extern "C" int smpc_run_perceived_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd,
+                                           const smpc_scene_io* scene, const smpc_weight_sets* w,
+                                           const smpc_orca_params* orca, const smpc_perception* perception) {
+  return run_perceived(h, io, crowd, scene, w, orca, perception, nullptr, "run_perceived_episodes");
+}
+
+extern "C" int smpc_run_tracked_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd,
+                                         const smpc_scene_io* scene, const smpc_weight_sets* w,
+                                         const smpc_orca_params* orca, const smpc_perception* perception,
+                                         const smpc_tracker* tracker) {
+  if (!tracker) return smpc_host_fail(SMPC_ERR_ARGUMENT, "run_tracked_episodes: NULL tracker");
+  return run_perceived(h, io, crowd, scene, w, orca, perception, tracker, "run_tracked_episodes");
 }

@@ -194,6 +194,30 @@ struct smpc_perception_args {
 // Enqueues smpc_perception_kernel on st (one launch).
 int smpc_perception_enqueue(smpc_handle* h, const smpc_perception_args& a, cudaStream_t st);
 
+// One controller tick of the tracked perception of smpc_run_tracked_episodes (smpc_tracker.cu), all device pointers:
+// the detections of the perception stage (p; its seen / n_seen are unused) update one constant-velocity Kalman track
+// per agent id, the confirmed tracks are published into the ring slot of tick k, and the FOV filter reads the slot of
+// tick k - latency, which p.seen_log / p.n_seen_log and id_log record.
+struct smpc_tracker_args {
+  smpc_perception_args p;
+  int M;                          // track slots per robot: K + R in shared scenes, else K
+  int confirm_hits, max_coast;
+  double dt, accel_noise, meas_noise, init_vel_std;
+  double *px, *py, *vx, *vy;      // [B][M] track state, zero at the start of a call
+  double *p_pp, *p_pv, *p_vv;     // [B][M] the per-axis covariance both axes share
+  int32_t *hits, *misses;         // [B][M]; hits == 0: no track
+  double* pub;                    // [B][L][5] the ring slot of tick k: the published rows
+  int32_t *pub_n, *pub_id;        // [B], [B][L]
+  const double* del;              // [B][L][5] the ring slot of tick k - latency (= pub when latency is 0)
+  const int32_t* del_id;          // [B][L]
+  int32_t* del_n;                 // [B] (zeroed for a finished robot: the FOV filter then reads nobody)
+  int32_t *untracked, *track_rows;  // [B] accumulated over the ticks a robot runs
+  double *pos_err, *vel_err;      // [B]
+  int32_t* id_log;                // [B][T][L] or NULL: the ids of the rows of p.seen_log
+};
+// Enqueues smpc_tracked_perception_kernel on st (one launch).
+int smpc_tracked_perception_enqueue(smpc_handle* h, const smpc_tracker_args& a, cudaStream_t st);
+
 const smpc_params* smpc_handle_params(smpc_handle* h);
 smpc_fleet_state* smpc_handle_fleet(smpc_handle* h);
 smpc_fleet_state* smpc_handle_single(smpc_handle* h);

@@ -56,6 +56,38 @@ def perception_arg(perception, n_robots: int, ticks: int, n_rows: int, want_logs
     return pc, out, keep
 
 
+def tracker_arg(tracker, pc, n_robots: int, ticks: int, n_rows: int, want_logs: bool):
+    """The smpc_tracker of the `tracker=` keyword (an abi.SmpcTracker, or a dict of abi.tracker_params overrides) with
+    its outputs pointed at new arrays: (struct, raw outputs dict). pc: the smpc_perception it follows, which must report
+    positions only (vel_noise 0); n_rows = L, the rows of the perceived list."""
+    if pc.vel_noise != 0.0:
+        raise ValueError("tracker= estimates velocities from detected positions: the perception needs vel_noise=0, "
+                         f"got {pc.vel_noise}")
+    if isinstance(tracker, abi.SmpcTracker):
+        tk = abi.SmpcTracker.from_buffer_copy(tracker)
+    else:
+        tk = abi.tracker_params(**dict(tracker))
+    raw = dict(untracked_personal_ticks=np.zeros(n_robots, np.int32), track_rows=np.zeros(n_robots, np.int32),
+               track_pos_err=np.zeros(n_robots), track_vel_err=np.zeros(n_robots))
+    if want_logs:
+        raw["track_id_log"] = np.full((n_robots, ticks, n_rows), -1, np.int32)
+    for k, v in raw.items():
+        setattr(tk, k, v.ctypes.data)
+    return tk, raw
+
+
+def tracker_results(raw) -> dict:
+    """The result entries of a tracked run from tracker_arg's raw outputs: the summed errors become means over the
+    people rows the FOV filter received (NaN for a robot that received none)."""
+    rows = raw["track_rows"]
+    out = dict(untracked_personal_ticks=raw["untracked_personal_ticks"], track_rows=rows)
+    for name, key in (("mean_track_pos_error", "track_pos_err"), ("mean_track_vel_error", "track_vel_err")):
+        out[name] = np.divide(raw[key], rows, out=np.full(rows.shape, np.nan), where=rows > 0)
+    if "track_id_log" in raw:
+        out["track_id_log"] = raw["track_id_log"]
+    return out
+
+
 class FleetOptimizer:
     def __init__(self, params, n_robots: int, n_agents: int = 3, device: int = 0):
         self.device = device
@@ -214,7 +246,7 @@ class FleetOptimizer:
 
     def run_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
                      od: dict, ticks: int, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                     want_logs=False, weights=None, perception=None) -> dict:
+                     want_logs=False, weights=None, perception=None, tracker=None) -> dict:
         """Closed-loop episodes on the GPU (smpc_run_episodes): each of the B robots runs its crowd scene for up to
         `ticks` controller ticks — trajectorizer seed, constant-velocity people, FOV filter, the fleet tick, a unicycle
         world step — with one upload and one download for the whole run. global_path [B][N][2], pose [B][3],
@@ -228,16 +260,23 @@ class FleetOptimizer:
         sensor between the people and the FOV filter (smpc_run_perceived_episodes): range, occlusion by walls and people,
         missed detections and noisy tracks. The dict then also holds unseen_personal_ticks [B] (ticks with a person
         within 1.2 m that went unreported) and, with want_logs, seen_log [B][T][K][5] and n_seen_log [B][T] (what the
-        FOV filter received at each tick)."""
+        FOV filter received at each tick).
+        tracker: abi.tracker_params(...), or a dict of its overrides, puts a people tracker after the sensor
+        (smpc_run_tracked_episodes): a constant-velocity Kalman track per person, published after confirm_hits
+        detections, coasted through max_coast_ticks misses and delivered latency_ticks late. It needs perception=, with
+        vel_noise=0. The dict then also holds untracked_personal_ticks [B] (ticks with a person within 1.2 m missing
+        from what the FOV filter received), track_rows [B] (people rows it received), mean_track_pos_error and
+        mean_track_vel_error [B] (their mean distance from the true position and velocity of the same tick, NaN
+        without rows) and, with want_logs, track_id_log [B][T][K] (the agent ids of the seen_log rows, -1 past
+        n_seen_log); seen_log and n_seen_log then hold the tracker's delayed list."""
+        if tracker is not None and perception is None:
+            raise ValueError("tracker= needs perception=: the tracker follows the sensor")
         io, out, logs, keep = self.episode_io(global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                                               costmap_resolution, od, ticks, control_period, goal_tolerance,
                                               costmap_index, od_index, want_logs)
         if perception is not None:
-            pc, pout, pkeep = perception_arg(perception, self.B, int(ticks), io.n_people, want_logs)
             ws, wkeep = weight_sets_arg(weights, self.B) if weights is not None else (None, None)
-            _lib.check(_lib.lib().smpc_run_perceived_episodes(self.opt._h, C.byref(io), None, None,
-                                                              None if ws is None else C.byref(ws), None, C.byref(pc)))
-            out.update(pout)
+            out.update(self._perceived(io, None, None, ws, None, perception, tracker, io.n_people, want_logs))
         elif weights is None:
             _lib.check(_lib.lib().smpc_run_episodes(self.opt._h, C.byref(io)))
         else:
@@ -252,7 +291,7 @@ class FleetOptimizer:
     def run_crowd_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                            costmap_resolution, od: dict, ticks: int, goals, desired_speed, substeps=1,
                            control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                           want_logs=False, weights=None, orca=None, perception=None) -> dict:
+                           want_logs=False, weights=None, orca=None, perception=None, tracker=None) -> dict:
         """Closed-loop episodes with a reactive crowd (smpc_run_crowd_episodes): run_episodes, but the people walk to
         their goals [B][K][2] at their desired speeds [B][K] under the lightsfm social force model, `substeps` updates
         per control period, and give way to the robot; people [B][K][5] is their state at t = 0. Returns the dict of
@@ -260,15 +299,15 @@ class FleetOptimizer:
         with want_logs also people_log [B][T+1][K][5] (x, y, vx, vy, vz at every tick, row 0 = the input).
         weights: as in run_episodes. orca: abi.orca_params(...) (or a dict of its overrides) moves the people by ORCA
         instead (smpc_run_orca_episodes), a crowd model the controller does not predict with; people_disturbance is
-        then the velocity change the robot demanded, in m. perception: as in run_episodes."""
+        then the velocity change the robot demanded, in m. perception, tracker: as in run_episodes."""
         return self._crowd_run(None, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                                costmap_resolution, od, ticks, goals, desired_speed, substeps, control_period,
-                               goal_tolerance, costmap_index, od_index, want_logs, weights, orca, perception)
+                               goal_tolerance, costmap_index, od_index, want_logs, weights, orca, perception, tracker)
 
     def run_shared_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                             costmap_resolution, od: dict, ticks: int, goals, desired_speed, robots_per_scene,
                             substeps=1, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                            want_logs=False, weights=None, orca=None, perception=None) -> dict:
+                            want_logs=False, weights=None, orca=None, perception=None, tracker=None) -> dict:
         """Closed-loop episodes in shared scenes (smpc_run_shared_episodes): run_crowd_episodes with the B robots
         grouped into S = B / R scenes of R = robots_per_scene consecutive robots that share one crowd, costmap and
         obstacle grid, and that see each other as people. Per robot: global_path [B][N][2], pose [B][3],
@@ -277,17 +316,20 @@ class FleetOptimizer:
         robot_min_dist [B] (nearest other robot of the scene, inf for R = 1) and robot_intimate_ticks [B]; with
         want_logs people_log is per scene, [S][T+1][K][5]. weights: as in run_episodes, set_index per robot.
         orca: as in run_crowd_episodes. perception: as in run_episodes; a robot's list is its scene view, the other
-        R - 1 robots then the people, so seen_log is [B][T][R-1+K][5]."""
+        R - 1 robots then the people, so seen_log is [B][T][R-1+K][5]. tracker: as in run_episodes; the other robots
+        are tracked too (ids K + r) but count in none of its metrics."""
         return self._crowd_run(int(robots_per_scene), global_path, pose, speed, people, n_people, costmaps,
                                costmap_origin, costmap_resolution, od, ticks, goals, desired_speed, substeps,
                                control_period, goal_tolerance, costmap_index, od_index, want_logs, weights, orca,
-                               perception)
+                               perception, tracker)
 
     def _crowd_run(self, R, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
                    od, ticks, goals, desired_speed, substeps, control_period, goal_tolerance, costmap_index, od_index,
-                   want_logs, weights=None, orca=None, perception=None) -> dict:
+                   want_logs, weights=None, orca=None, perception=None, tracker=None) -> dict:
         """run_crowd_episodes (R None) or run_shared_episodes (R robots per scene); orca: the ORCA crowd; perception:
-        the sensor between the scene and the FOV filter."""
+        the sensor between the scene and the FOV filter; tracker: the people tracker after it."""
+        if tracker is not None and perception is None:
+            raise ValueError("tracker= needs perception=: the tracker follows the sensor")
         io, out, logs, keep = self.episode_io(global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                                               costmap_resolution, od, ticks, control_period, goal_tolerance,
                                               costmap_index, od_index, want_logs, robots_per_scene=R or 1)
@@ -310,13 +352,8 @@ class FleetOptimizer:
             scene = abi.SmpcSceneIo(R, res["robot_min_dist"].ctypes.data, res["robot_intimate_ticks"].ctypes.data)
         if perception is not None:
             op = None if orca is None else orca if isinstance(orca, abi.SmpcOrcaParams) else abi.orca_params(**orca)
-            pc, pout, pkeep = perception_arg(perception, B, T, (R or 1) - 1 + K, want_logs)
             ws, wkeep = weight_sets_arg(weights, B) if weights is not None else (None, None)
-            _lib.check(_lib.lib().smpc_run_perceived_episodes(self.opt._h, C.byref(io), C.byref(crowd),
-                                                              None if scene is None else C.byref(scene),
-                                                              None if ws is None else C.byref(ws),
-                                                              None if op is None else C.byref(op), C.byref(pc)))
-            res.update(pout)
+            res.update(self._perceived(io, crowd, scene, ws, op, perception, tracker, (R or 1) - 1 + K, want_logs))
         elif orca is not None:
             op = orca if isinstance(orca, abi.SmpcOrcaParams) else abi.orca_params(**orca)
             ws, wkeep = weight_sets_arg(weights, B) if weights is not None else (None, None)
@@ -337,6 +374,20 @@ class FleetOptimizer:
             res["optimized_log"] = logs["optimized_log"].astype(bool)
             res["people_log"] = people_log
         return res
+
+    def _perceived(self, io, crowd, scene, ws, op, perception, tracker, n_rows, want_logs) -> dict:
+        """smpc_run_perceived_episodes (tracker None) or smpc_run_tracked_episodes on the built arguments: the
+        perception's results, and the tracker's. n_rows = L, the rows of the perceived list."""
+        pc, out, keep = perception_arg(perception, self.B, io.n_ticks, n_rows, want_logs)
+        args = [self.opt._h, C.byref(io), None if crowd is None else C.byref(crowd),
+                None if scene is None else C.byref(scene), None if ws is None else C.byref(ws),
+                None if op is None else C.byref(op), C.byref(pc)]
+        if tracker is None:
+            _lib.check(_lib.lib().smpc_run_perceived_episodes(*args))
+            return out
+        tk, raw = tracker_arg(tracker, pc, self.B, io.n_ticks, n_rows, want_logs)
+        _lib.check(_lib.lib().smpc_run_tracked_episodes(*args, C.byref(tk)))
+        return dict(out, **tracker_results(raw))
 
     def episode_io(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
                    od: dict, ticks: int, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
