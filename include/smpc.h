@@ -630,6 +630,65 @@ int smpc_run_tracked_episodes(smpc_handle* h, smpc_episode_io* io,
                               const smpc_orca_params* orca /* NULL: the lightsfm crowd if crowd is given */,
                               const smpc_perception* perception, const smpc_tracker* tracker);
 
+/* ---- closed-loop episodes with a rolling local costmap: a robot-centred window with the people in it marked -----------
+ * Any episode kind above (crowd, scene, w, orca, perception and tracker keep their meaning, checks and outputs;
+ * perception may be NULL: no sensor stage; a tracker needs perception) with the controller reading a per-robot window
+ * instead of the static costmap, as Nav2's controller reads its local costmap. Write (ox, oy), res and (W, H) for the
+ * origin, resolution and size of robot b's static costmap (costmap_index). At every tick k with
+ * k % update_period_ticks == 0 that robot b runs, its window of size_x x size_y cells at res is rebuilt:
+ * - placement: c = floor((x_k - o) / res) per axis is the robot's static cell; the window starts at static cell
+ *   c0 = (cx - size_x / 2, cy - size_y / 2) (C integer division: the robot's cell is the centre cell) and its origin is
+ *   (ox + c0x res, oy + c0y res), one IEEE multiply then add. Nav2's rolling window snaps to whole cells relative to its
+ *   previous origin with truncation toward zero, so its origin can differ from this one by up to one cell;
+ * - static layer: window cell (i, j) holds static cell (c0x + i, c0y + j), or 0 outside the static map (Nav2's local
+ *   costmap with track_unknown_space false); the static maps are taken as already inflated;
+ * - people layer (mark_people 1): every row of the list the perception stage reads (the scene's people, or in shared
+ *   scenes the other R - 1 robots then the people) at its true position of tick k (a laser obstacle layer has no
+ *   tracker latency and no detection draw) whose static cell, by the same floor rule, lies inside the window is
+ *   marked, and a cell's cost is max(static, max over marked rows of S[dy][dx]) for the fixed stencil S centred on the
+ *   row's cell;
+ * - stencil (smpc_local_costmap_stencil), in double: cell (dx, dy) is 254 when dx^2 + dy^2 <= rho^2,
+ *   rho = agent_radius / res + 1e-9; otherwise, with d the distance in cells between cell centres to the nearest such
+ *   cell, 253 when d res <= inscribed_radius + 1e-9, floor(252 exp(-cost_scaling_factor (d res - inscribed_radius)))
+ *   when d <= inflation_radius / res + 1e-9, else 0 (Nav2's InflationLayer::computeCost on a disc of lethal cells, so
+ *   the max over rows is the inflation of their union). Its half-width is the smallest holding every non-zero entry.
+ * The FOV filter's worldToMap test and the fleet tick's obstacle critic read robot b's latest window and origin
+ * (between builds: the last build). The perception and tracker wall walk, the world step's collision check and
+ * metrics, and the crowd models and people projection (through the obstacle-distance grid) keep reading the static
+ * map. A finished robot rebuilds nothing. The launches per tick are those of the entry without the window, plus one
+ * on build ticks. Device memory beyond it: B size_x size_y bytes of windows, 16 B of origin per robot, and the logs'
+ * sizes when given.
+ * Returns what the entry without the window returns, plus SMPC_ERR_ARGUMENT for local == NULL, a field outside its
+ * range or NaN, a stencil half-width above 32, marked_rows == NULL, only one of the two logs, or a tracker without
+ * perception; all before anything is launched and before the fleet state is touched. */
+typedef struct smpc_local_costmap {
+  int size_x, size_y;          /* cells, 8..256 each (the benchmark yaml's 4 m x 4 m at 0.05 m: 80 x 80) */
+  int update_period_ticks;     /* 1..20: rebuilt at ticks k % n == 0 (Nav2's default 5 Hz at 20 Hz: 4) */
+  int mark_people;             /* 0: static layer only, 1: people layer too */
+  double agent_radius;         /* m, >= 0, finite */
+  double inscribed_radius;     /* m, >= 0, finite */
+  double cost_scaling_factor;  /* 1/m, > 0, finite */
+  double inflation_radius;     /* m, >= inscribed_radius, finite */
+  int32_t* marked_rows;        /* [B] out, not NULL: rows marked, summed over the builds robot b ran */
+  uint8_t* costmap_log;        /* [B][n_builds][size_y][size_x] or NULL, n_builds = ceil(T / update_period_ticks);
+                                  builds after an episode is done are zero */
+  double* origin_log;          /* [B][n_builds][2] or NULL (given together with costmap_log); NaN after it is done */
+} smpc_local_costmap;
+int smpc_run_local_costmap_episodes(smpc_handle* h, smpc_episode_io* io,
+                                    const smpc_crowd_io* crowd /* NULL: constant-velocity people */,
+                                    const smpc_scene_io* scene /* NULL: one robot per scene */,
+                                    const smpc_weight_sets* w /* NULL: the handle's weights */,
+                                    const smpc_orca_params* orca /* NULL: the lightsfm crowd if crowd is given */,
+                                    const smpc_perception* perception /* NULL: no sensor stage */,
+                                    const smpc_tracker* tracker /* NULL; needs perception */,
+                                    const smpc_local_costmap* local);
+/* Diagnostics, no GPU: the stencil smpc_run_local_costmap_episodes would splat at this resolution, row-major
+ * [2 hw + 1][2 hw + 1] (row = dy + hw, column = dx + hw) into out when it has the capacity, and its half-width hw.
+ * SMPC_ERR_ARGUMENT for what the episode entry rejects in local (the outputs aside), resolution not > 0, a half-width
+ * above 32 (*half_width is then 33) or capacity too small; out may be NULL to query the half-width. */
+int smpc_local_costmap_stencil(const smpc_local_costmap* local, double resolution, uint8_t* out, int capacity,
+                               int* half_width);
+
 /* ---- batched pre-solve stage on the GPU: project_people (src/optimizer.cpp:554-671 + sfm.hpp) -----------------
  * One warp per problem, lanes over agents, sequential over the horizon. Generalised from the reference's 3 people to
  * A columns. Inputs (device pointers): robot [B][S+1][6] = the robot AgentTrajectory of format_to_optimize

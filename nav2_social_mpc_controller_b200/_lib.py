@@ -85,6 +85,13 @@ def lib():
                                             P(abi.SmpcWeightSets), P(abi.SmpcOrcaParams), P(abi.SmpcPerception),
                                             P(abi.SmpcTracker)]
     L.smpc_run_tracked_episodes.restype = C.c_int
+    L.smpc_run_local_costmap_episodes.argtypes = [C.c_void_p, P(abi.SmpcEpisodeIo), P(abi.SmpcCrowdIo),
+                                                  P(abi.SmpcSceneIo), P(abi.SmpcWeightSets), P(abi.SmpcOrcaParams),
+                                                  P(abi.SmpcPerception), P(abi.SmpcTracker), P(abi.SmpcLocalCostmap)]
+    L.smpc_run_local_costmap_episodes.restype = C.c_int
+    L.smpc_local_costmap_stencil.argtypes = [P(abi.SmpcLocalCostmap), C.c_double, C.c_void_p, C.c_int,
+                                             P(C.c_int)]
+    L.smpc_local_costmap_stencil.restype = C.c_int
     L.smpc_reset_memory.argtypes = [C.c_void_p]
     L.smpc_reset_memory.restype = C.c_int
     L.smpc_project_people_batch.argtypes = [C.c_void_p, P(abi.SmpcProjectArgs)]
@@ -138,6 +145,7 @@ EXPORTED_SYMBOLS = (
     "smpc_optimize", "smpc_optimize_batch", "smpc_run_episodes", "smpc_run_crowd_episodes",
     "smpc_run_shared_episodes", "smpc_optimize_batch_weighted", "smpc_run_weighted_episodes",
     "smpc_run_orca_episodes", "smpc_run_perceived_episodes", "smpc_run_tracked_episodes",
+    "smpc_run_local_costmap_episodes", "smpc_local_costmap_stencil",
     "smpc_reset_memory", "smpc_project_people_batch", "smpc_project_people_batch_device",
     "smpc_format_batch_device", "smpc_people_to_status_device", "smpc_memory_update_device",
     "smpc_trajectorize_batch_device", "smpc_fov_filter_batch_device", "smpc_multi_create", "smpc_multi_destroy",

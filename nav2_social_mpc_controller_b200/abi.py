@@ -529,6 +529,39 @@ def tracker_params(**overrides) -> SmpcTracker:
     return SmpcTracker(**dict(TRACKER_DEFAULTS, **overrides))
 
 
+class SmpcLocalCostmap(C.Structure):
+    """struct smpc_local_costmap — the rolling local costmap of smpc_run_local_costmap_episodes."""
+    _fields_ = [
+        ("size_x", C.c_int),
+        ("size_y", C.c_int),
+        ("update_period_ticks", C.c_int),
+        ("mark_people", C.c_int),
+        ("agent_radius", C.c_double),
+        ("inscribed_radius", C.c_double),
+        ("cost_scaling_factor", C.c_double),
+        ("inflation_radius", C.c_double),
+        ("marked_rows", C.c_void_p),
+        ("costmap_log", C.c_void_p),
+        ("origin_log", C.c_void_p),
+    ]
+
+
+# A plausible local costmap (not measured from one): the reference benchmark yaml's 4 m x 4 m window at 0.05 m, rebuilt
+# at Nav2's default 5 Hz under a 20 Hz controller, people marked as discs of the perception stage's 0.25 m occluder
+# radius, no inscribed band, the decay of scenarios.wall_costmap and Nav2's default 0.55 m inflation radius.
+LOCAL_COSTMAP_DEFAULTS = dict(size_x=80, size_y=80, update_period_ticks=4, mark_people=1, agent_radius=0.25,
+                              inscribed_radius=0.0, cost_scaling_factor=3.0, inflation_radius=0.55)
+
+
+def local_costmap_params(**overrides) -> SmpcLocalCostmap:
+    """SmpcLocalCostmap with the defaults LOCAL_COSTMAP_DEFAULTS, any field overridden by keyword; the output pointers
+    stay NULL (FleetOptimizer fills them). Raises ValueError for an unknown field."""
+    unknown = set(overrides) - set(LOCAL_COSTMAP_DEFAULTS)
+    if unknown:
+        raise ValueError(f"unknown local costmap parameters: {sorted(unknown)}")
+    return SmpcLocalCostmap(**dict(LOCAL_COSTMAP_DEFAULTS, **overrides))
+
+
 # the nine critic weights of a row of smpc_weight_sets.weights, in smpc_params order
 WEIGHT_NAMES = ("distance_w", "socialwork_w", "velocity_w", "angle_w", "agent_angle_w", "proxemics_w",
                 "velocity_feasibility_w", "obstacle_w", "goal_align_w")

@@ -1,9 +1,10 @@
 // smpc_episode.cu — closed-loop episodes (smpc_run_episodes, smpc_run_crowd_episodes, smpc_run_shared_episodes,
-// smpc_run_weighted_episodes, smpc_run_orca_episodes, smpc_run_perceived_episodes, smpc_run_tracked_episodes): B
-// robots through their crowd scenes for up to T controller ticks, every tick enqueued on the handle's stream without a
-// host round trip. One tick per episode is
+// smpc_run_weighted_episodes, smpc_run_orca_episodes, smpc_run_perceived_episodes, smpc_run_tracked_episodes,
+// smpc_run_local_costmap_episodes): B robots through their crowd scenes for up to T controller ticks, every tick
+// enqueued on the handle's stream without a host round trip. One tick per episode is
 //   trajectorizer (seed) -> tick prep (constant-velocity people at k * dt_c, seed repack, max_time cut) -> [scene view]
-//   -> [perception, smpc_perception.cu, or tracked perception, smpc_tracker.cu] -> FOV filter -> fleet tick
+//   -> [perception, smpc_perception.cu, or tracked perception, smpc_tracker.cu] -> [local costmap build on build
+//   ticks, smpc_local_costmap.cu] -> FOV filter -> fleet tick
 //   (smpc_fleet_tick_enqueue) -> [reactive crowd step, smpc_crowd.cu, or ORCA crowd step, smpc_orca.cu] -> world step
 //   (robot Euler step, metrics, goal check, logs) -> [robot-robot metrics].
 // All entries share one loop: with a crowd the prep leaves the people alone, the FOV filter and the world step read
@@ -292,10 +293,12 @@ __global__ void smpc_robot_metrics_kernel(RobotMetrics a) {
 // moves by ORCA (smpc_run_orca_episodes) instead of the social force model. pc != NULL (parameters checked): the
 // perception stage cuts the FOV filter's input to what the sensor reports (smpc_run_perceived_episodes). tk != NULL
 // (checked, pc given): a people tracker follows the sensor and the FOV filter reads its delayed published list
-// (smpc_run_tracked_episodes).
+// (smpc_run_tracked_episodes). local != NULL (outputs checked): the FOV filter and the fleet tick read per-robot rolling
+// windows that smpc_local_costmap_kernel rebuilds every update_period_ticks (smpc_run_local_costmap_episodes).
 int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd, const smpc_scene_io* scene,
                  const char* name, const smpc_weight_sets* w = nullptr, const smpc_orca_params* orca = nullptr,
-                 const smpc_perception* pc = nullptr, const smpc_tracker* tk = nullptr) {
+                 const smpc_perception* pc = nullptr, const smpc_tracker* tk = nullptr,
+                 const smpc_local_costmap* local = nullptr) {
   auto fail_arg = [name](const char* msg) {
     return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string(name) + ": " + msg);
   };
@@ -368,6 +371,12 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
     for (int b = 0; b < B && pc->stream_index; ++b)
       if (pc->stream_index[b] < 0) return fail_arg("stream_index[b] < 0");
   }
+  std::vector<uint8_t> stencil;
+  int half = 0;
+  if (local) {
+    const int lrc = smpc_local_costmap_build_stencil(local, io->resolution, &stencil, &half, name);
+    if (lrc != SMPC_OK) return lrc;
+  }
   // the trajectorizer integrates with the yaml DOUBLE time_step (SURVEY Q15), as FleetOptimizer.trajectorize_batch
   const double traj_dt = std::round((double)prm->time_step * 1e6) / 1e6;
   const int max_steps = (int)std::round((double)prm->max_time / traj_dt);
@@ -423,6 +432,12 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
   int* n_active;
   double* weights = nullptr;
   int32_t* weight_set = nullptr;
+  const int n_period = local ? local->update_period_ticks : 1, n_builds = (T + n_period - 1) / n_period;
+  const size_t cells = local ? (size_t)local->size_x * local->size_y : 0;
+  const bool logs_local = local && local->costmap_log != nullptr;
+  uint8_t *windows = nullptr, *stencil_dev = nullptr, *window_log = nullptr;
+  double *window_org = nullptr, *window_org_log = nullptr;
+  int32_t* marked = nullptr;
   auto carve = [&](smpc_carve& c) {
     maps = c.take<uint8_t>(map_bytes);
     od = c.take<uint32_t>(od_bytes / 4);
@@ -504,6 +519,14 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       vel_err = c.take<double>(Bz);
       id_log = c.take<int32_t>(logs_seen ? Bz * T * Lz : 0);
     }
+    if (local) {
+      windows = c.take<uint8_t>(Bz * cells);
+      window_org = c.take<double>(Bz * 2);
+      stencil_dev = c.take<uint8_t>(stencil.size());
+      marked = c.take<int32_t>(Bz);
+      window_log = c.take<uint8_t>(logs_local ? Bz * n_builds * cells : 0);
+      window_org_log = c.take<double>(logs_local ? Bz * n_builds * 2 : 0);
+    }
   };
   size_t need = 0;
   {
@@ -525,6 +548,7 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       {people0, K > 0 ? io->people : nullptr, Sz * Kz * 40}, {n_people_dev, K > 0 ? io->n_people_each : nullptr, Sz * 4},
       {weights, w ? w->weights : nullptr, w ? (size_t)w->n_sets * 72 : 0}, {weight_set, w ? w->set_index : nullptr, Bz * 4},
       {stream_idx, perceive ? pc->stream_index : nullptr, Bz * 4},
+      {stencil_dev, local ? stencil.data() : nullptr, stencil.size()},
   };
   for (const Up& u : ups)
     if (u.host && u.bytes) SMPC_FLEET_CUDA(cudaMemcpyAsync(u.dev, u.host, u.bytes, cudaMemcpyHostToDevice, st));
@@ -541,6 +565,7 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
   SMPC_FLEET_CUDA(cudaMemsetAsync(fov_people, 0, Bz * A * 40, st));
   SMPC_FLEET_CUDA(cudaMemsetAsync(fov_n, 0, Bz * 4, st));  // K == 0: nobody to filter, n_people stays 0
   if (perceive) SMPC_FLEET_CUDA(cudaMemsetAsync(unseen, 0, Bz * 4, st));
+  if (local) SMPC_FLEET_CUDA(cudaMemsetAsync(marked, 0, Bz * 4, st));
   if (tracked) {  // no tracks, and nothing published before tick 0
     SMPC_FLEET_CUDA(cudaMemsetAsync(trk_hits, 0, Bz * Mz * 4, st));
     SMPC_FLEET_CUDA(cudaMemsetAsync(trk_misses, 0, Bz * Mz * 4, st));
@@ -632,6 +657,21 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
     ca.od_resolution = io->od_resolution; ca.od = od; ca.od_org = od_org; ca.od_index = d.od_index;
   }
 
+  smpc_local_costmap_args la{};
+  if (local) {  // built from the true list, before perception; the FOV filter and the fleet tick read the windows
+    la.B = B; la.sx = local->size_x; la.sy = local->size_y; la.half = half; la.L = n_list; la.n_builds = n_builds;
+    la.active = active; la.pose = pose; la.list = scene ? view : people;
+    la.n_list = local->mark_people && fov ? (scene ? view_n : n_people_dev) : nullptr;
+    la.stencil = stencil_dev; la.maps = maps; la.map_org = map_org; la.map_index = d.map_index;
+    la.n_costmaps = io->n_costmaps; la.size_x = io->size_x; la.size_y = io->size_y; la.resolution = io->resolution;
+    la.window = windows; la.origin = window_org; la.marked = marked;
+    la.window_log = logs_local ? window_log : nullptr; la.origin_log = logs_local ? window_org_log : nullptr;
+    d.maps = windows; d.map_org = window_org; d.map_index = nullptr;
+    d.n_costmaps = B; d.size_x = local->size_x; d.size_y = local->size_y;
+    fa.costmap_origin = window_org; fa.costmap_index = nullptr;
+    fa.n_costmaps = B; fa.size_x = local->size_x; fa.size_y = local->size_y;
+  }
+
   const SceneView sv{B, R, K, n_view, active, pose, speed, people, K > 0 ? n_people_dev : nullptr, view, view_n};
   RobotMetrics rm{B, R, 0, pose, ticks, robot_min, robot_intimate};
 
@@ -661,6 +701,11 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
     } else if (perceive) {
       pa.k = k;
       rc = smpc_perception_enqueue(h, pa, st);
+      if (rc != SMPC_OK) return rc;
+    }
+    if (local && k % n_period == 0) {
+      la.build = k / n_period;
+      rc = smpc_local_costmap_enqueue(h, la, st);
       if (rc != SMPC_OK) return rc;
     }
     if (fov) {
@@ -713,6 +758,9 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       {tracked ? tk->track_pos_err : nullptr, pos_err, Bz * 8},
       {tracked ? tk->track_vel_err : nullptr, vel_err, Bz * 8},
       {tracked && logs_seen ? tk->track_id_log : nullptr, id_log, Bz * T * Lz * 4},
+      {local ? local->marked_rows : nullptr, marked, Bz * 4},
+      {logs_local ? local->costmap_log : nullptr, window_log, Bz * n_builds * cells},
+      {logs_local ? local->origin_log : nullptr, window_org_log, Bz * n_builds * 16},
   };
   for (const Down& c : downs)
     if (c.host) SMPC_FLEET_CUDA(cudaMemcpyAsync(c.host, c.dev, c.bytes, cudaMemcpyDeviceToHost, st));
@@ -731,6 +779,11 @@ int run_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd
       std::memset(pc->n_seen_log + (size_t)b * T + tb, 0, (size_t)(T - tb) * 4);
     }
     if (tracked && logs_seen) std::fill_n(tk->track_id_log + ((size_t)b * T + tb) * Lz, (size_t)(T - tb) * Lz, -1);
+    if (logs_local) {  // builds at ticks j * n_period >= tb never ran
+      const int jb = (tb + n_period - 1) / n_period;
+      std::memset(local->costmap_log + ((size_t)b * n_builds + jb) * cells, 0, (size_t)(n_builds - jb) * cells);
+      std::fill_n(local->origin_log + ((size_t)b * n_builds + jb) * 2, (size_t)(n_builds - jb) * 2, (double)NAN);
+    }
   }
   if (pc && !perceive) {  // no list: nothing reported, nobody missed
     std::memset(pc->unseen_personal_ticks, 0, Bz * 4);
@@ -855,19 +908,30 @@ extern "C" int smpc_run_orca_episodes(smpc_handle* h, smpc_episode_io* io, const
 
 namespace {
 
-// smpc_run_perceived_episodes (tk == NULL) and smpc_run_tracked_episodes: the argument checks that need no B
+// smpc_run_perceived_episodes (tk == NULL), smpc_run_tracked_episodes and smpc_run_local_costmap_episodes: the argument
+// checks that need no B (perception may be NULL only with local given; the local costmap's fields: once the
+// resolution is checked)
 int run_perceived(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd, const smpc_scene_io* scene,
                   const smpc_weight_sets* w, const smpc_orca_params* orca, const smpc_perception* perception,
-                  const smpc_tracker* tk, const char* name) {
+                  const smpc_tracker* tk, const char* name, const smpc_local_costmap* local = nullptr) {
   auto fail_arg = [name](const char* msg) {
     return smpc_host_fail(SMPC_ERR_ARGUMENT, std::string(name) + ": " + msg);
   };
-  if (!perception) return fail_arg("NULL perception");
-  int rc = check_perception(perception, name);
-  if (rc != SMPC_OK) return rc;
+  if (!perception && !local) return fail_arg("NULL perception");
+  int rc = SMPC_OK;
+  if (perception) {
+    rc = check_perception(perception, name);
+    if (rc != SMPC_OK) return rc;
+  }
   if (tk) {
+    if (!perception) return fail_arg("a tracker needs perception");
     rc = check_tracker(tk, perception, name);
     if (rc != SMPC_OK) return rc;
+  }
+  if (local) {
+    if (!local->marked_rows) return fail_arg("missing output");
+    if ((local->costmap_log == nullptr) != (local->origin_log == nullptr))
+      return fail_arg("costmap_log and origin_log not given together");
   }
   if (scene && !crowd) return fail_arg("a shared scene needs a crowd");
   if (orca && !crowd) return fail_arg("an ORCA crowd needs a crowd");
@@ -879,7 +943,7 @@ int run_perceived(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crow
     rc = smpc_check_weight_sets(w, 0, name);  // the indices: once B is known
     if (rc != SMPC_OK) return rc;
   }
-  return run_episodes(h, io, crowd, scene, name, w, orca, perception, tk);
+  return run_episodes(h, io, crowd, scene, name, w, orca, perception, tk, local);
 }
 
 }  // namespace
@@ -896,4 +960,12 @@ extern "C" int smpc_run_tracked_episodes(smpc_handle* h, smpc_episode_io* io, co
                                          const smpc_tracker* tracker) {
   if (!tracker) return smpc_host_fail(SMPC_ERR_ARGUMENT, "run_tracked_episodes: NULL tracker");
   return run_perceived(h, io, crowd, scene, w, orca, perception, tracker, "run_tracked_episodes");
+}
+
+extern "C" int smpc_run_local_costmap_episodes(smpc_handle* h, smpc_episode_io* io, const smpc_crowd_io* crowd,
+                                               const smpc_scene_io* scene, const smpc_weight_sets* w,
+                                               const smpc_orca_params* orca, const smpc_perception* perception,
+                                               const smpc_tracker* tracker, const smpc_local_costmap* local) {
+  if (!local) return smpc_host_fail(SMPC_ERR_ARGUMENT, "run_local_costmap_episodes: NULL local costmap");
+  return run_perceived(h, io, crowd, scene, w, orca, perception, tracker, "run_local_costmap_episodes", local);
 }

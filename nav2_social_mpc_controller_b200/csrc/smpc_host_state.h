@@ -218,6 +218,35 @@ struct smpc_tracker_args {
 // Enqueues smpc_tracked_perception_kernel on st (one launch).
 int smpc_tracked_perception_enqueue(smpc_handle* h, const smpc_tracker_args& a, cudaStream_t st);
 
+// One build of the rolling local costmaps of smpc_run_local_costmap_episodes (smpc_local_costmap.cu), all device
+// pointers: robot b's window of sx x sy cells around its pose of tick k, the static layer cropped from its static costmap
+// and, with n_list given, the stencil splatted on the cell of every row of its true list that lies inside the window.
+struct smpc_local_costmap_args {
+  int B, sx, sy, half;            // window size, stencil half-width (<= 32)
+  int L, build, n_builds;         // list rows; this build's index k / update_period_ticks, of n_builds
+  const uint8_t* active;          // [B] robots running tick k; the others build nothing
+  const double* pose;             // [B][3] robot pose of tick k
+  const double* list;             // [B][L][5] true positions of the people (shared scenes: the scene view)
+  const int32_t* n_list;          // [B], or NULL: no people layer
+  const uint8_t* stencil;         // [2 half + 1][2 half + 1]
+  const uint8_t* maps;            // the static costmaps
+  const double* map_org;
+  const int32_t* map_index;       // may be NULL (map b % n_costmaps)
+  int n_costmaps, size_x, size_y;
+  double resolution;
+  uint8_t* window;                // [B][sy][sx] out
+  double* origin;                 // [B][2] out
+  int32_t* marked;                // [B] += rows marked
+  uint8_t* window_log;            // [B][n_builds][sy][sx] or NULL
+  double* origin_log;             // [B][n_builds][2] or NULL
+};
+// Enqueues smpc_local_costmap_kernel on st (one launch).
+int smpc_local_costmap_enqueue(smpc_handle* h, const smpc_local_costmap_args& a, cudaStream_t st);
+// SMPC_ERR_ARGUMENT unless every field of the smpc_local_costmap l that the build reads is in range and the stencil at
+// resolution res has a half-width <= 32; then the stencil, row-major [2 half + 1]^2, and its half-width
+int smpc_local_costmap_build_stencil(const smpc_local_costmap* l, double res, std::vector<uint8_t>* stencil, int* half,
+                                     const char* name);
+
 const smpc_params* smpc_handle_params(smpc_handle* h);
 smpc_fleet_state* smpc_handle_fleet(smpc_handle* h);
 smpc_fleet_state* smpc_handle_single(smpc_handle* h);

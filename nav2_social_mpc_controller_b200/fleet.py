@@ -88,6 +88,38 @@ def tracker_results(raw) -> dict:
     return out
 
 
+def local_costmap_arg(local_costmap, n_robots: int, ticks: int, want_logs: bool):
+    """The smpc_local_costmap of the `local_costmap=` keyword (an abi.SmpcLocalCostmap, or a dict of
+    abi.local_costmap_params overrides) with its outputs pointed at new arrays: (struct, outputs dict). The logs hold
+    one row per build, n_builds = ceil(ticks / update_period_ticks)."""
+    if isinstance(local_costmap, abi.SmpcLocalCostmap):
+        lc = abi.SmpcLocalCostmap.from_buffer_copy(local_costmap)
+    else:
+        lc = abi.local_costmap_params(**dict(local_costmap))
+    out = dict(marked_rows=np.zeros(n_robots, np.int32))
+    fields = dict(marked_rows="marked_rows")
+    if want_logs:
+        n_builds = -(-ticks // max(int(lc.update_period_ticks), 1))
+        out.update(local_costmap_log=np.zeros((n_robots, n_builds, lc.size_y, lc.size_x), np.uint8),
+                   local_origin_log=np.zeros((n_robots, n_builds, 2)))
+        fields.update(local_costmap_log="costmap_log", local_origin_log="origin_log")
+    for k, f in fields.items():
+        setattr(lc, f, out[k].ctypes.data)
+    return lc, out
+
+
+def local_costmap_stencil(resolution: float, local_costmap=None) -> np.ndarray:
+    """The inflation stencil smpc_run_local_costmap_episodes splats on a marked row at this resolution
+    (smpc_local_costmap_stencil, no GPU): uint8 [2 hw + 1][2 hw + 1], row dy + hw, column dx + hw. local_costmap: as the
+    keyword of run_episodes (None: the defaults). Raises SmpcError for what the episode entry rejects."""
+    lc = local_costmap_arg({} if local_costmap is None else local_costmap, 0, 0, False)[0]
+    L, hw = _lib.lib(), C.c_int(0)
+    _lib.check(L.smpc_local_costmap_stencil(C.byref(lc), float(resolution), None, 0, C.byref(hw)))
+    out = np.zeros((2 * hw.value + 1, 2 * hw.value + 1), np.uint8)
+    _lib.check(L.smpc_local_costmap_stencil(C.byref(lc), float(resolution), out.ctypes.data, out.size, C.byref(hw)))
+    return out
+
+
 class FleetOptimizer:
     def __init__(self, params, n_robots: int, n_agents: int = 3, device: int = 0):
         self.device = device
@@ -246,7 +278,7 @@ class FleetOptimizer:
 
     def run_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
                      od: dict, ticks: int, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                     want_logs=False, weights=None, perception=None, tracker=None) -> dict:
+                     want_logs=False, weights=None, perception=None, tracker=None, local_costmap=None) -> dict:
         """Closed-loop episodes on the GPU (smpc_run_episodes): each of the B robots runs its crowd scene for up to
         `ticks` controller ticks — trajectorizer seed, constant-velocity people, FOV filter, the fleet tick, a unicycle
         world step — with one upload and one download for the whole run. global_path [B][N][2], pose [B][3],
@@ -268,15 +300,22 @@ class FleetOptimizer:
         from what the FOV filter received), track_rows [B] (people rows it received), mean_track_pos_error and
         mean_track_vel_error [B] (their mean distance from the true position and velocity of the same tick, NaN
         without rows) and, with want_logs, track_id_log [B][T][K] (the agent ids of the seen_log rows, -1 past
-        n_seen_log); seen_log and n_seen_log then hold the tracker's delayed list."""
+        n_seen_log); seen_log and n_seen_log then hold the tracker's delayed list.
+        local_costmap: abi.local_costmap_params(...), or a dict of its overrides, makes the FOV filter and the fleet
+        tick read a rolling robot-centred window of each robot's costmap with the people in it marked and inflated
+        (smpc_run_local_costmap_episodes), rebuilt every update_period_ticks; it works with every keyword above. The dict
+        then also holds marked_rows [B] (people rows marked, summed over the builds) and, with want_logs,
+        local_costmap_log [B][n_builds][size_y][size_x] and local_origin_log [B][n_builds][2] (each build's window and
+        origin; zero and NaN for builds after the episode was done)."""
         if tracker is not None and perception is None:
             raise ValueError("tracker= needs perception=: the tracker follows the sensor")
         io, out, logs, keep = self.episode_io(global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                                               costmap_resolution, od, ticks, control_period, goal_tolerance,
                                               costmap_index, od_index, want_logs)
-        if perception is not None:
+        if perception is not None or local_costmap is not None:
             ws, wkeep = weight_sets_arg(weights, self.B) if weights is not None else (None, None)
-            out.update(self._perceived(io, None, None, ws, None, perception, tracker, io.n_people, want_logs))
+            out.update(self._perceived(io, None, None, ws, None, perception, tracker, io.n_people, want_logs,
+                                       local_costmap))
         elif weights is None:
             _lib.check(_lib.lib().smpc_run_episodes(self.opt._h, C.byref(io)))
         else:
@@ -291,7 +330,8 @@ class FleetOptimizer:
     def run_crowd_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                            costmap_resolution, od: dict, ticks: int, goals, desired_speed, substeps=1,
                            control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                           want_logs=False, weights=None, orca=None, perception=None, tracker=None) -> dict:
+                           want_logs=False, weights=None, orca=None, perception=None, tracker=None,
+                           local_costmap=None) -> dict:
         """Closed-loop episodes with a reactive crowd (smpc_run_crowd_episodes): run_episodes, but the people walk to
         their goals [B][K][2] at their desired speeds [B][K] under the lightsfm social force model, `substeps` updates
         per control period, and give way to the robot; people [B][K][5] is their state at t = 0. Returns the dict of
@@ -299,15 +339,17 @@ class FleetOptimizer:
         with want_logs also people_log [B][T+1][K][5] (x, y, vx, vy, vz at every tick, row 0 = the input).
         weights: as in run_episodes. orca: abi.orca_params(...) (or a dict of its overrides) moves the people by ORCA
         instead (smpc_run_orca_episodes), a crowd model the controller does not predict with; people_disturbance is
-        then the velocity change the robot demanded, in m. perception, tracker: as in run_episodes."""
+        then the velocity change the robot demanded, in m. perception, tracker, local_costmap: as in run_episodes."""
         return self._crowd_run(None, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                                costmap_resolution, od, ticks, goals, desired_speed, substeps, control_period,
-                               goal_tolerance, costmap_index, od_index, want_logs, weights, orca, perception, tracker)
+                               goal_tolerance, costmap_index, od_index, want_logs, weights, orca, perception, tracker,
+                               local_costmap)
 
     def run_shared_episodes(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin,
                             costmap_resolution, od: dict, ticks: int, goals, desired_speed, robots_per_scene,
                             substeps=1, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
-                            want_logs=False, weights=None, orca=None, perception=None, tracker=None) -> dict:
+                            want_logs=False, weights=None, orca=None, perception=None, tracker=None,
+                            local_costmap=None) -> dict:
         """Closed-loop episodes in shared scenes (smpc_run_shared_episodes): run_crowd_episodes with the B robots
         grouped into S = B / R scenes of R = robots_per_scene consecutive robots that share one crowd, costmap and
         obstacle grid, and that see each other as people. Per robot: global_path [B][N][2], pose [B][3],
@@ -317,17 +359,19 @@ class FleetOptimizer:
         want_logs people_log is per scene, [S][T+1][K][5]. weights: as in run_episodes, set_index per robot.
         orca: as in run_crowd_episodes. perception: as in run_episodes; a robot's list is its scene view, the other
         R - 1 robots then the people, so seen_log is [B][T][R-1+K][5]. tracker: as in run_episodes; the other robots
-        are tracked too (ids K + r) but count in none of its metrics."""
+        are tracked too (ids K + r) but count in none of its metrics. local_costmap: as in run_episodes; the other
+        robots of the scene are marked like people."""
         return self._crowd_run(int(robots_per_scene), global_path, pose, speed, people, n_people, costmaps,
                                costmap_origin, costmap_resolution, od, ticks, goals, desired_speed, substeps,
                                control_period, goal_tolerance, costmap_index, od_index, want_logs, weights, orca,
-                               perception, tracker)
+                               perception, tracker, local_costmap)
 
     def _crowd_run(self, R, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
                    od, ticks, goals, desired_speed, substeps, control_period, goal_tolerance, costmap_index, od_index,
-                   want_logs, weights=None, orca=None, perception=None, tracker=None) -> dict:
+                   want_logs, weights=None, orca=None, perception=None, tracker=None, local_costmap=None) -> dict:
         """run_crowd_episodes (R None) or run_shared_episodes (R robots per scene); orca: the ORCA crowd; perception:
-        the sensor between the scene and the FOV filter; tracker: the people tracker after it."""
+        the sensor between the scene and the FOV filter; tracker: the people tracker after it; local_costmap: the
+        rolling windows the FOV filter and the fleet tick read."""
         if tracker is not None and perception is None:
             raise ValueError("tracker= needs perception=: the tracker follows the sensor")
         io, out, logs, keep = self.episode_io(global_path, pose, speed, people, n_people, costmaps, costmap_origin,
@@ -350,10 +394,11 @@ class FleetOptimizer:
         if R is not None:
             res.update(robot_min_dist=np.zeros(B), robot_intimate_ticks=np.zeros(B, np.int32))
             scene = abi.SmpcSceneIo(R, res["robot_min_dist"].ctypes.data, res["robot_intimate_ticks"].ctypes.data)
-        if perception is not None:
+        if perception is not None or local_costmap is not None:
             op = None if orca is None else orca if isinstance(orca, abi.SmpcOrcaParams) else abi.orca_params(**orca)
             ws, wkeep = weight_sets_arg(weights, B) if weights is not None else (None, None)
-            res.update(self._perceived(io, crowd, scene, ws, op, perception, tracker, (R or 1) - 1 + K, want_logs))
+            res.update(self._perceived(io, crowd, scene, ws, op, perception, tracker, (R or 1) - 1 + K, want_logs,
+                                       local_costmap))
         elif orca is not None:
             op = orca if isinstance(orca, abi.SmpcOrcaParams) else abi.orca_params(**orca)
             ws, wkeep = weight_sets_arg(weights, B) if weights is not None else (None, None)
@@ -375,19 +420,28 @@ class FleetOptimizer:
             res["people_log"] = people_log
         return res
 
-    def _perceived(self, io, crowd, scene, ws, op, perception, tracker, n_rows, want_logs) -> dict:
-        """smpc_run_perceived_episodes (tracker None) or smpc_run_tracked_episodes on the built arguments: the
-        perception's results, and the tracker's. n_rows = L, the rows of the perceived list."""
-        pc, out, keep = perception_arg(perception, self.B, io.n_ticks, n_rows, want_logs)
+    def _perceived(self, io, crowd, scene, ws, op, perception, tracker, n_rows, want_logs, local_costmap=None) -> dict:
+        """smpc_run_perceived_episodes (tracker None), smpc_run_tracked_episodes or, with local_costmap,
+        smpc_run_local_costmap_episodes (perception may then be None) on the built arguments: the results of the
+        perception, the tracker and the local costmap. n_rows = L, the rows of the perceived list."""
+        out, pc, tk = {}, None, None
+        if perception is not None:
+            pc, out, keep = perception_arg(perception, self.B, io.n_ticks, n_rows, want_logs)
         args = [self.opt._h, C.byref(io), None if crowd is None else C.byref(crowd),
                 None if scene is None else C.byref(scene), None if ws is None else C.byref(ws),
-                None if op is None else C.byref(op), C.byref(pc)]
-        if tracker is None:
+                None if op is None else C.byref(op), None if pc is None else C.byref(pc)]
+        if tracker is not None:
+            tk, raw = tracker_arg(tracker, pc, self.B, io.n_ticks, n_rows, want_logs)
+        if local_costmap is not None:
+            lc, lout = local_costmap_arg(local_costmap, self.B, io.n_ticks, want_logs)
+            _lib.check(_lib.lib().smpc_run_local_costmap_episodes(*args, None if tk is None else C.byref(tk),
+                                                                  C.byref(lc)))
+            out = dict(out, **lout)
+        elif tk is None:
             _lib.check(_lib.lib().smpc_run_perceived_episodes(*args))
-            return out
-        tk, raw = tracker_arg(tracker, pc, self.B, io.n_ticks, n_rows, want_logs)
-        _lib.check(_lib.lib().smpc_run_tracked_episodes(*args, C.byref(tk)))
-        return dict(out, **tracker_results(raw))
+        else:
+            _lib.check(_lib.lib().smpc_run_tracked_episodes(*args, C.byref(tk)))
+        return out if tk is None else dict(out, **tracker_results(raw))
 
     def episode_io(self, global_path, pose, speed, people, n_people, costmaps, costmap_origin, costmap_resolution,
                    od: dict, ticks: int, control_period=0.05, goal_tolerance=0.25, costmap_index=None, od_index=None,
